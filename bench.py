@@ -25,6 +25,8 @@ A "step" is one pass of the hot path over the rank's shard.
   verified : every rank compares the first 20 000 queries of its shard's timed output with the oracle (outside the timed
           region); a mismatch fails the run
 `--impl reference` times that CPU port alone (the reference is Rust + polars and cannot be built in this image).
+`--dump-outputs DIR` writes the result of the last timed step (the headline arm: device-resident, or C5's streamed run) to
+DIR/*.npy in a canonical, sampled form (dump_outputs); the inputs are seeded, so two builds can be compared file by file.
 """
 from __future__ import annotations
 
@@ -46,6 +48,11 @@ BASE_SEED = 20261018
 CUSTOM = {"domain": 50, "kingdom": 60, "phylum": 75, "class": 80, "order": 85, "family": 92, "genus": 97, "species": 99}
 CPU_SAMPLE_Q = 100_000
 VERIFY_Q = 20_000
+# --dump-outputs: queries sampled from the result, and at most this many of their beans / accession references
+# (float64 columns: 16 x 64 Ki + 4 x 512 Ki + 3 x 1 Mi values = 48 MiB at most)
+DUMP_QUERIES = 1 << 16
+DUMP_BEANS = 1 << 19
+DUMP_ACCESSIONS = 1 << 20
 
 CONFIGS = {
     "c2": dict(cid=2, queries=1_000_000, hits=50, zipf=False, taxa=30_000, taxon="custom", strategy="relaxed", scaling="weak",
@@ -186,6 +193,61 @@ def generate_shard(w, cfg, q_begin, n_queries, pinned, cap, dbuf, host_keep_byte
     return total, rows, host_bytes, host_q, host_rows
 
 
+def _ranges(starts, counts):
+    """Concatenation of arange(s, s + n) over (starts, counts)."""
+    import numpy as np
+
+    counts = counts.astype(np.int64)
+    ends = np.cumsum(counts)
+    return np.repeat(starts.astype(np.int64) - (ends - counts), counts) + np.arange(int(ends[-1]) if len(ends) else 0, dtype=np.int64)
+
+
+def dump_outputs(out, directory):
+    """Writes a result as float64 .npy files: its sizes and checksum, and a seeded sample of its queries with their records,
+    beans and accession references.  The kernels place records, beans and strings in an order that differs from run to run,
+    so the dump is canonical: queries sorted by id, beans and accessions in the order their query lists them, strings as
+    (CRC-32, length).  Two builds given the same arguments write the same files."""
+    import zlib
+
+    import numpy as np
+
+    from blutils_b200 import _ffi
+
+    out.download()
+    lib, h = _ffi.lib(), out._h
+    nq, nb, na = len(out), lib.blu_result_num_beans(h), lib.blu_result_num_accessions(h)
+    plen = C.c_uint64()
+    pptr = lib.blu_result_pool(h, C.byref(plen))
+    pool = np.ctypeslib.as_array(C.cast(pptr, C.POINTER(C.c_uint8)), shape=(plen.value,)) if plen.value else np.zeros(0, np.uint8)
+    recs = np.ctypeslib.as_array(lib.blu_result_records(h), shape=(nq,)) if nq else np.zeros(0, np.dtype(_ffi.blu_record))
+    beans = np.ctypeslib.as_array(C.cast(lib.blu_result_beans(h), C.POINTER(_ffi.blu_bean)), shape=(nb,)) if nb else np.zeros(0, np.dtype(_ffi.blu_bean))
+    accs = np.ctypeslib.as_array(C.cast(lib.blu_result_accessions(h), C.POINTER(C.c_uint64)), shape=(na,)) if na else np.zeros(0, np.uint64)
+
+    ids = [pool[o:o + n].tobytes() for o, n in zip(recs["query_off"].tolist(), recs["query_len"].tolist())]
+    by_id = np.array(sorted(range(nq), key=ids.__getitem__), dtype=np.int64)
+    rank = np.sort(np.random.default_rng(BASE_SEED).choice(nq, size=min(nq, DUMP_QUERIES), replace=False))
+    r = recs[by_id[rank]]
+    cols = {"query_rank": rank, "query_crc32": [zlib.crc32(ids[i]) for i in by_id[rank].tolist()], "keep_mask_lo": r["keep_mask"] & 0xFFFFFFFF,
+            "keep_mask_hi": r["keep_mask"] >> 32}
+    for f in ("query_len", "n_rows", "status", "single_match", "mutated", "perc_identity", "bit_score", "ref_lineage", "reached_pos",
+              "allowed_pos", "bean_level", "n_beans"):
+        cols[f] = r[f]
+    # beans of the sampled queries, query by query (bean_query: index into the sample)
+    bean_query = np.repeat(np.arange(len(r)), r["n_beans"].astype(np.int64))[:DUMP_BEANS]
+    b = beans[_ranges(r["bean_base"], r["n_beans"])[:DUMP_BEANS]]
+    cols.update(bean_query=bean_query, bean_first_lineage=b["first_lineage"], bean_occurrences=b["occurrences"], bean_n_acc=b["n_acc"])
+    # their accession references (acc_begin is relative to the query's acc_base), bean by bean
+    acc_bean = np.repeat(np.arange(len(b)), b["n_acc"].astype(np.int64))[:DUMP_ACCESSIONS]
+    a = accs[_ranges(r["acc_base"][bean_query].astype(np.int64) + b["acc_begin"], b["n_acc"])[:DUMP_ACCESSIONS]]
+    a_off, a_len = (a >> 16).tolist(), (a & 0xFFFF).tolist()
+    cols.update(accession_bean=acc_bean, accession_crc32=[zlib.crc32(pool[o:o + n].tobytes()) for o, n in zip(a_off, a_len)], accession_len=a_len)
+    ck = out.checksum()
+    cols.update(result_counts=[nq, out.n_rows, nb, na], result_checksum=[ck & 0xFFFFFFFF, ck >> 32])
+    os.makedirs(directory, exist_ok=True)
+    for name, v in cols.items():
+        np.save(os.path.join(directory, name + ".npy"), np.asarray(v, dtype=np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -201,7 +263,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-verify", action="store_true")
     ap.add_argument("--no-file-arm", action="store_true", help="skip the blu_consensus_run_file timing (the call the CLI makes)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path computed in its last step to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the results of the CUDA path (--impl b200)")
 
     cfg = dict(CONFIGS[args.config])
     if args.hits:
@@ -216,6 +284,9 @@ def main():
     rank = env_int("RANK", 0)
     world = env_int("WORLD_SIZE", 1)
     local_rank = env_int("LOCAL_RANK", 0)
+    dump_dir = args.dump_outputs
+    if dump_dir and world > 1:
+        dump_dir = os.path.join(dump_dir, f"rank{rank}")
     if scaling == "weak":
         q_rank, q_begin, q_table = cfg["queries"], rank * cfg["queries"], world * cfg["queries"]
     else:
@@ -387,6 +458,8 @@ def main():
                 if rank == 0:
                     print(json.dumps({"error": "timed output differs from the oracle", "verified": verified}))
                 sys.exit(3)
+        if dump_dir:
+            dump_outputs(last, dump_dir)
         last.close()
 
         # ---------------- the same step with the result downloaded to pinned host memory ----------------------------------
@@ -441,19 +514,26 @@ def main():
     for _ in range(max(1, args.warmup // 2)):
         eng.run_host(pinned, host_bytes).close()
     barrier()
-    e2e_steps = args.steps if not streamed_only else max(1, min(args.steps, 2))
+    e2e_steps = args.steps
     t0 = time.perf_counter()
     d2h = 0
     e2e_launches = 0
-    for _ in range(e2e_steps):
+    last = None
+    for i in range(e2e_steps):
         for _p in range(passes):
             out = eng.run_host(pinned, host_bytes)
             tm = eng.timings()
             d2h = int(tm["d2h_bytes"])
             e2e_launches += int(tm["n_kernel_launches"])
-            out.close()
+            if streamed_only and dump_dir and i + 1 == e2e_steps and _p + 1 == passes:
+                last = out  # C5's timed output
+            else:
+                out.close()
     torch.cuda.synchronize()
     e2e_own = time.perf_counter() - t0
+    if last is not None:
+        dump_outputs(last, dump_dir)
+        last.close()
     e2e_s = max_over_ranks(e2e_own) / e2e_steps
     e2e_per_rank = every_rank(e2e_own / e2e_steps * 1e3)
     barrier()

@@ -66,6 +66,8 @@ SYMBOLS = [
     ("blu_consensus_run_file", C.c_int, [C.c_void_p, C.c_char_p, C.POINTER(C.c_void_p)]),
     ("blu_result_add_headers", C.c_int, [C.c_void_p, C.c_char_p, C.c_uint64]),
     ("blu_result_num_queries", C.c_uint64, [C.c_void_p]),
+    ("blu_result_num_records", C.c_uint64, [C.c_void_p]),
+    ("blu_result_sort_by_query", C.c_int, [C.c_void_p, C.c_void_p]),
     ("blu_result_num_rows", C.c_uint64, [C.c_void_p]),
     ("blu_result_records", C.POINTER(blu_record), [C.c_void_p]),
     ("blu_result_beans", C.c_void_p, [C.c_void_p]),

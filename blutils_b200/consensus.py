@@ -226,6 +226,12 @@ class ConsensusOutput:
             raise RuntimeError("blu_result_download failed")
         return self
 
+    def sort_by_query(self) -> "ConsensusOutput":
+        """Orders the records by query id on the GPU of the engine that produced the result (blu_result_sort_by_query): a
+        stable, bytewise sort, the writer's order.  Works on device-resident results before `.download()` too."""
+        self._engine._check(_ffi.lib().blu_result_sort_by_query(self._engine._h, self._h))
+        return self
+
     def device_arrays(self):
         """(records_ptr, beans_ptr, n_beans, accessions_ptr, n_accessions) of a device-resident result."""
         nb, na = C.c_uint64(), C.c_uint64()
@@ -240,8 +246,8 @@ class ConsensusOutput:
         return _ffi.lib().blu_result_device_text(self._h, C.byref(n)), n.value
 
     def records(self):
-        """The binary records as a ctypes array (host results)."""
-        n = _ffi.lib().blu_result_num_queries(self._h)
+        """The binary records as a ctypes array (host results); hit-less headers are not records."""
+        n = _ffi.lib().blu_result_num_records(self._h)
         p = _ffi.lib().blu_result_records(self._h)
         return C.cast(p, C.POINTER(_ffi.blu_record * n)).contents if p else None
 

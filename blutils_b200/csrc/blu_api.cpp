@@ -32,6 +32,7 @@
 #include "blu_decode.h"
 #include "blu_json.h"
 #include "blu_kernels.h"
+#include "blu_sort.h"
 #include "blu_tabular.h"
 #include "blu_taxonomy.h"
 
@@ -258,6 +259,7 @@ struct blu_result {
     std::vector<ResultPartOwned> parts;
     uint64_t n_rows = 0;
     std::vector<std::string> hitless;  // NoConsensusFound (mod.rs:84-102)
+    bool sorted = false;               // the records are in query-id order (blu_result_sort_by_query)
     // concatenation of a multi-part result for the array accessors (built on first use)
     mutable std::mutex merge_mu;
     mutable bool merged = false;
@@ -295,6 +297,7 @@ ResultView make_view(const blu_result* r) {
         v.parts.push_back(q);
     }
     v.hitless_ = &r->hitless;
+    v.sorted = r->sorted;
     return v;
 }
 
@@ -1545,6 +1548,197 @@ void merge_parts(const blu_result* r) {
     r->merged = true;
 }
 
+// --- records in query-id order (blu_result_sort_by_query) ----------------------------------------------------------------
+// BLU_SORT_TRACE=1: wall time of every stage on stderr (the stream is synchronised at each mark: measurement only)
+struct SortTrace {
+    bool on;
+    cudaStream_t s;
+    std::chrono::steady_clock::time_point t0;
+    std::string line;
+    explicit SortTrace(cudaStream_t st) : on(getenv("BLU_SORT_TRACE") != nullptr), s(st), t0(std::chrono::steady_clock::now()) {}
+    void mark(const char* what) {
+        if (!on) return;
+        cudaStreamSynchronize(s);
+        const auto t1 = std::chrono::steady_clock::now();
+        char b[96];
+        snprintf(b, sizeof b, "%s%s %.3f", line.empty() ? "" : ", ", what, std::chrono::duration<double, std::milli>(t1 - t0).count());
+        line += b;
+        t0 = t1;
+    }
+    ~SortTrace() {
+        if (on) fprintf(stderr, "[blu sort] ms: %s\n", line.c_str());
+    }
+};
+
+// device scratch of one sort call
+struct CudaMem {
+    void* p = nullptr;
+    CudaMem() = default;
+    CudaMem(const CudaMem&) = delete;
+    CudaMem& operator=(const CudaMem&) = delete;
+    ~CudaMem() {
+        if (p) cudaFree(p);
+    }
+    template <class T>
+    T* alloc(uint64_t count) {
+        if (cudaMalloc(&p, std::max<uint64_t>(count, 1) * sizeof(T)) != cudaSuccess) {
+            cudaGetLastError();
+            throw UnsupportedErr("the query ids and the sort's scratch do not fit the device");
+        }
+        return (T*)p;
+    }
+};
+
+// the ids (id_bytes), their references, the permutation, `extra` bytes and the sort's scratch must fit the free device memory
+void require_sort_fits(uint64_t n, uint64_t id_bytes, uint64_t extra) {
+    size_t free_b = 0, total_b = 0;
+    CK(cudaMemGetInfo(&free_b, &total_b));
+    const uint64_t need = id_bytes + n * (sizeof(uint64_t) + 2 * sizeof(uint32_t)) + extra + sort_ids_device_bytes(n) + (64ull << 20);
+    if (need > (uint64_t)free_b)
+        throw UnsupportedErr("the query ids and the sort's scratch (" + std::to_string(need >> 20) + " MiB) do not fit the device (" +
+                             std::to_string(free_b >> 20) + " MiB free)");
+}
+
+void sort_ids_checked(const uint8_t* base, const uint64_t* off, const uint32_t* len, uint32_t n, uint32_t* perm, cudaStream_t s) {
+    const int rc = sort_ids_device(base, off, len, n, perm, s);
+    if (rc == 1) throw UnsupportedErr("the sort's scratch does not fit the device");
+    if (rc < 0) throw CudaErr(std::string("sort_ids_device: ") + cudaGetErrorString((cudaError_t)(-rc)));
+}
+
+// a device-resident part: the records are gathered in HBM into a record buffer of the context's DevicePool
+void sort_part_device(blu_ctx* c, ResultPartOwned& p) {
+    CK(cudaSetDevice(c->device));
+    cudaStream_t s = c->stream;
+    const uint32_t n = (uint32_t)p.n_rec;
+    SortTrace tr(s);
+    require_sort_fits(n, 0, (uint64_t)n * sizeof(blu_record));
+    CudaMem m_off, m_len, m_perm;
+    uint64_t* off = m_off.alloc<uint64_t>(n);
+    uint32_t* len = m_len.alloc<uint32_t>(n);
+    uint32_t* perm = m_perm.alloc<uint32_t>(n);
+    CK(launch_record_ids(p.dev->rec.p, n, off, len, s));
+    sort_ids_checked(p.dtext, off, len, n, perm, s);
+    tr.mark("sort");
+    std::unique_ptr<DeviceSet> set = p.dev_pool->acquire();
+    try {
+        set->rec.ensure(n);
+        CK(launch_gather_records(p.dev->rec.p, perm, n, set->rec.p, s));
+        CK(cudaStreamSynchronize(s));
+    } catch (...) {
+        cudaStreamSynchronize(s);
+        p.dev_pool->release(std::move(set));
+        throw;
+    }
+    std::swap(p.dev->rec, set->rec);
+    p.dev_pool->release(std::move(set));
+    tr.mark("permute");
+}
+
+// the parts of a multi-device host result become one part (the concatenation merge_parts builds)
+void concat_parts(blu_ctx* g, blu_result* r) {
+    merge_parts(r);
+    ResultPartOwned one;
+    one.pinned = g->pool;
+    try {
+        auto put = [&](PinnedBuf& b, const void* src, uint64_t bytes) {
+            b = g->acquire(std::max<uint64_t>(bytes, 64));
+            if (bytes) memcpy(b.p, src, bytes);
+        };
+        put(one.b_rec, r->m_rec.data(), r->m_rec.size() * sizeof(blu_record));
+        put(one.b_beans, r->m_beans.data(), r->m_beans.size() * sizeof(blu_bean));
+        put(one.b_accs, r->m_accs.data(), r->m_accs.size() * sizeof(blu_acc));
+        if (r->m_ext) {
+            one.ext_strings = r->m_ext, one.ext_len = r->m_ext_len;
+        } else {
+            put(one.b_pool, r->m_pool.data(), r->m_pool.size());
+            one.pool_len = r->m_pool.size();
+        }
+    } catch (...) {
+        one.free_buffers();
+        throw;
+    }
+    one.n_rec = r->m_rec.size(), one.n_beans = r->m_beans.size(), one.n_accs = r->m_accs.size();
+    for (auto& p : r->parts) p.free_buffers();
+    r->parts.clear();
+    r->parts.push_back(std::move(one));
+    std::lock_guard<std::mutex> lk(r->merge_mu);
+    r->merged = false;
+    std::vector<blu_record>().swap(r->m_rec);
+    std::vector<blu_bean>().swap(r->m_beans);
+    std::vector<blu_acc>().swap(r->m_accs);
+    std::string().swap(r->m_pool);
+    r->m_ext = nullptr, r->m_ext_len = 0;
+}
+
+// a host part: its ids are packed into pinned memory and sorted on g's GPU; the permutation comes back and the records are
+// gathered on all host threads
+void sort_part_host(blu_ctx* g, ResultPartOwned& p) {
+    const uint64_t n = p.n_rec;
+    const blu_record* rec = (const blu_record*)p.b_rec.p;
+    const char* str = p.strings();
+    cudaStream_t s = g->stream;
+    struct Pinned {
+        std::shared_ptr<PinnedPool> pool;
+        PinnedBuf b;
+        ~Pinned() { pool->release(b); }
+    };
+    SortTrace tr(s);
+    Pinned h_off{g->pool, g->acquire(n * sizeof(uint64_t))}, h_len{g->pool, g->acquire(n * sizeof(uint32_t))};
+    uint64_t* off = (uint64_t*)h_off.b.p;
+    uint32_t* len = (uint32_t*)h_len.b.p;
+    std::vector<uint64_t> sums(host_threads() + 1, 0);
+    parallel_ranges(n, [&](unsigned t, size_t a, size_t b) {
+        uint64_t x = 0;
+        for (size_t i = a; i < b; i++) x += rec[i].query_len;
+        sums[t + 1] = x;
+    });
+    for (size_t t = 1; t < sums.size(); t++) sums[t] += sums[t - 1];
+    const uint64_t id_bytes = sums.back();
+    Pinned h_ids{g->pool, g->acquire(std::max<uint64_t>(id_bytes, 64))};
+    char* ids = (char*)h_ids.b.p;
+    parallel_ranges(n, [&](unsigned t, size_t a, size_t b) {
+        uint64_t o = sums[t];
+        for (size_t i = a; i < b; i++) {
+            off[i] = o, len[i] = rec[i].query_len;
+            memcpy(ids + o, str + rec[i].query_off, rec[i].query_len);
+            o += rec[i].query_len;
+        }
+    });
+    tr.mark("pack");
+    require_sort_fits(n, id_bytes, 0);
+    Pinned h_perm{g->pool, g->acquire(n * sizeof(uint32_t))};
+    {
+        CudaMem m_ids, m_off, m_len, m_perm;
+        uint8_t* d_ids = m_ids.alloc<uint8_t>(id_bytes);
+        uint64_t* d_off = m_off.alloc<uint64_t>(n);
+        uint32_t* d_len = m_len.alloc<uint32_t>(n);
+        uint32_t* d_perm = m_perm.alloc<uint32_t>(n);
+        try {
+            if (id_bytes) CK(cudaMemcpyAsync(d_ids, ids, id_bytes, cudaMemcpyHostToDevice, s));
+            CK(cudaMemcpyAsync(d_off, off, n * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+            CK(cudaMemcpyAsync(d_len, len, n * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
+            tr.mark("h2d");
+            sort_ids_checked(d_ids, d_off, d_len, (uint32_t)n, d_perm, s);
+            tr.mark("sort");
+            CK(cudaMemcpyAsync(h_perm.b.p, d_perm, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+            CK(cudaStreamSynchronize(s));
+            tr.mark("d2h");
+        } catch (...) {  // nothing may still be copying when the buffers go back to their pools
+            cudaStreamSynchronize(s);
+            throw;
+        }
+    }
+    const uint32_t* perm = (const uint32_t*)h_perm.b.p;
+    PinnedBuf out = p.pinned->acquire(n * sizeof(blu_record));
+    blu_record* dst = (blu_record*)out.p;
+    parallel_ranges(n, [&](unsigned, size_t a, size_t b) {
+        for (size_t i = a; i < b; i++) dst[i] = rec[perm[i]];
+    });
+    p.pinned->release(p.b_rec);
+    p.b_rec = out;
+    tr.mark("permute");
+}
+
 }  // namespace
 
 // =================================================================================================================
@@ -1955,6 +2149,26 @@ int blu_result_download(blu_result* r) {
     }
 }
 
+int blu_result_sort_by_query(blu_ctx* c, blu_result* r) {
+    if (!c || !r) return fail(c, BLU_ERR_ARG, "null argument");
+    if (!r->on_host() && (r->parts.size() != 1 || r->parts[0].ctx != c))
+        return fail(c, BLU_ERR_ARG, "a device-resident result is sorted with the context that produced it");
+    return guarded(c, [&] {
+        const uint64_t n = r->n_rec();
+        if (n == 0) return;
+        if (n > 0xFFFFFFFFull) throw UnsupportedErr("more than 2^32 - 1 records");
+        if (!r->on_host()) {
+            sort_part_device(c, r->parts[0]);
+        } else {
+            blu_ctx* g = c->is_multi() ? c->shards[0].get() : c;
+            CK(cudaSetDevice(g->device));
+            if (r->parts.size() > 1) concat_parts(g, r);
+            sort_part_host(g, r->parts[0]);
+        }
+        r->sorted = true;
+    });
+}
+
 int blu_consensus_run_host(blu_ctx* c, const char* text, uint64_t n, blu_result** out) {
     if (!c || !out || (!text && n)) return fail(c, BLU_ERR_ARG, "null argument");
     *out = nullptr;
@@ -2050,6 +2264,7 @@ int blu_result_add_headers(blu_result* r, const char* headers_nl, uint64_t len) 
 }
 
 uint64_t blu_result_num_queries(const blu_result* r) { return r ? r->n_rec() + r->hitless.size() : 0; }
+uint64_t blu_result_num_records(const blu_result* r) { return r ? r->n_rec() : 0; }
 uint64_t blu_result_num_rows(const blu_result* r) { return r ? r->n_rows : 0; }
 uint64_t blu_result_num_beans(const blu_result* r) {
     uint64_t n = 0;

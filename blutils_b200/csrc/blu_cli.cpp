@@ -200,6 +200,14 @@ int main(int argc, char** argv) {
         die(blu_last_error(ctx));
     blu_result* res = nullptr;
     if (blu_consensus_run_file(ctx, blast_out.c_str(), &res) != BLU_OK) die(std::string("Unexpected error on parse blast results: ") + blu_last_error(ctx));
+    // The writer's sort by query id, on the GPU from 10^7 records on (the writer then only merges the hit-less headers in).
+    // A host result's ids are packed, sorted on the GPU and its records permuted on the host: on a B200 (1000 W) sort + JSONL /
+    // JSON write against the writer's own host sort, q%09d ids: 1.52 / 2.31 vs 1.00 / 1.14 ms at 10^3, 139 / 226 vs 123 / 176 ms
+    // at 10^6, 1360 / 1957 vs 1518 / 1807 ms at 10^7; 40-byte read names: 205 / 229 vs 188 / 214 ms at 10^6, 2081 / 2010 vs
+    // 2046 / 2154 ms at 10^7 (tools/sort_scale.py, DESIGN section 9).  Below 10^7 the host sort wins; at 10^7 they are even.
+    constexpr uint64_t kGpuSortMinRecords = 10000000;
+    if (blu_result_num_records(res) >= kGpuSortMinRecords && blu_result_sort_by_query(ctx, res) != BLU_OK)
+        die(std::string("Unexpected error on sort results: ") + blu_last_error(ctx));
     if (blu_result_write(res, have_out ? out_file.c_str() : nullptr, format, nullptr) != BLU_OK) die("Error on persist output results");
     blu_result_free(res);
     blu_ctx_destroy(ctx);

@@ -39,6 +39,7 @@ struct ResultView {
     Cutoffs cut;
     std::vector<ResultPart> parts;
     const std::vector<std::string>* hitless_ = nullptr;
+    bool sorted = false;  // the records of the parts, in part order, are in query-id order already
     uint64_t n_rec() const {
         uint64_t n = 0;
         for (auto& p : parts) n += p.n_rec;
@@ -248,15 +249,26 @@ void parallel_ranges(size_t n, F&& f) {
 
 // write_blutils_output.rs:87-111: flatten + sort by query (bytewise).  At 10^6 - 10^8 queries the sort of the ids is what the
 // writer waits for first (SURVEY 8f-1): the entries are sorted in per-thread chunks and merged pairwise in parallel (stable:
-// equal ids keep their file order, like the reference's sort_by).
+// equal ids keep their file order, like the reference's sort_by).  Records sorted on the GPU already (ResultView::sorted) are
+// only merged with the sorted hit-less headers, records first among equal ids: the same order.
 inline std::vector<Entry> sorted_entries(const ResultView* r) {
     std::vector<Entry> v;
     v.reserve(r->n_rec() + (r->hitless_ ? r->hitless_->size() : 0));
     for (auto& p : r->parts)
         for (uint64_t i = 0; i < p.n_rec; i++) v.push_back({rec_query(p, p.rec[i]), &p.rec[i], &p});
+    auto less = [](const Entry& a, const Entry& b) { return a.query < b.query; };
+    if (r->sorted) {
+        std::vector<Entry> h;
+        if (r->hitless_)
+            for (auto& x : *r->hitless_) h.push_back({std::string_view(x), nullptr, nullptr});
+        if (h.empty()) return v;
+        std::stable_sort(h.begin(), h.end(), less);
+        std::vector<Entry> out(v.size() + h.size());
+        std::merge(v.begin(), v.end(), h.begin(), h.end(), out.begin(), less);
+        return out;
+    }
     if (r->hitless_)
         for (auto& h : *r->hitless_) v.push_back({std::string_view(h), nullptr, nullptr});
-    auto less = [](const Entry& a, const Entry& b) { return a.query < b.query; };
     const size_t n = v.size();
     unsigned nt = (unsigned)std::min<size_t>(host_threads(), std::max<size_t>(1, n / 65536));
     if (nt <= 1) {
@@ -629,7 +641,7 @@ inline std::string view_to_jsonl(const ResultView* r, uint64_t max_entries = ~0u
     Decoder d(r);
     std::vector<Entry> ent;
     const uint64_t total = r->n_rec() + (r->hitless_ ? r->hitless_->size() : 0);
-    if (max_entries < total) {
+    if (max_entries < total && !r->sorted) {
         ent.reserve(total);
         for (auto& p : r->parts)
             for (uint64_t i = 0; i < p.n_rec; i++) ent.push_back({rec_query(p, p.rec[i]), &p.rec[i], &p});
@@ -646,8 +658,10 @@ inline std::string view_to_jsonl(const ResultView* r, uint64_t max_entries = ~0u
         head.reserve(max_entries);
         for (uint64_t i = 0; i < max_entries; i++) head.push_back(ent[idx[i]]);
         ent.swap(head);
-    } else
+    } else {
         ent = sorted_entries(r);
+        if (ent.size() > max_entries) ent.resize(max_entries);
+    }
     std::vector<std::string> parts(host_threads());
     parallel_ranges(ent.size(), [&](unsigned t, size_t a, size_t b) {
         std::string& o = parts[t];

@@ -11,8 +11,7 @@
 //   first row       open-addressing table keyed by the hash: slot.min_row = the first row with that id (atomicMin); every
 //                   row then compares its id BYTES with that row's, so a hash collision is detected (the host path takes
 //                   over), never silently merged
-//   order           stable radix sort of the rows by "first row of my query" (cub::DeviceRadixSort: library code on a
-//                   rare fallback path, not on the hot path)
+//   order           stable radix sort of the rows by "first row of my query" (blu_sort.cu)
 //   copy            exclusive scan of the row lengths in the new order, one warp per row copies it to its place
 //
 // Everything stays in HBM; the regrouped text is handed to the normal device-resident pipeline.
@@ -23,8 +22,9 @@
 
 #include <chrono>
 
-#include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
+
+#include "blu_sort.h"
 
 // (declared in blu_kernels.h; that header pulls in the device core, which this file does not need)
 
@@ -309,11 +309,11 @@ int regroup_device(const uint8_t* d_text, uint64_t n, cudaStream_t s, uint8_t** 
     // stable sort of the rows by the first row of their query
     int bits = 1;
     while (bits < 32 && (1ull << bits) < (uint64_t)n_rows) bits++;
-    size_t sort_bytes = 0;
-    RG_CK(cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, first, first_sorted, iota, order, (int)n_rows, 0, bits, s));
     uint8_t* sort_tmp;
-    if (!sc.alloc(&sort_tmp, sort_bytes)) return 1;
-    RG_CK(cub::DeviceRadixSort::SortPairs(sort_tmp, sort_bytes, first, first_sorted, iota, order, (int)n_rows, 0, bits, s));
+    if (!sc.alloc(&sort_tmp, radix_sort_scratch_bytes(n_rows))) return 1;
+    bool in_alt = false;
+    RG_CK(radix_sort_pairs_u32(first, first_sorted, iota, order, n_rows, bits, sort_tmp, s, &in_alt));
+    if (!in_alt) order = iota;
     tr.mark("sort");
     // where every row goes
     if (!sc.alloc(&slen, n_rows) || !sc.alloc(&dst, n_rows)) return 1;

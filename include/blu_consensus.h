@@ -181,6 +181,21 @@ int blu_result_add_headers(blu_result* res, const char* headers_nl, uint64_t len
 
 /* ---- results -------------------------------------------------------------------------------------------- */
 uint64_t blu_result_num_queries(const blu_result* res);
+/* Records with hits only (blu_result_num_queries also counts hit-less headers). */
+uint64_t blu_result_num_records(const blu_result* res);
+/* Orders the records of `res` by query id, bytewise -- the order write_blutils_output writes them in
+ * (write_blutils_output.rs:111) -- on the GPU of `ctx` (its first device for a multi-device context).
+ * Device-resident result (not yet downloaded): sorted in device memory; `ctx` must be the context that produced it
+ * (else BLU_ERR_ARG); blu_result_device_records() may return a new pointer afterwards.
+ * Host result: its query ids are copied to the device and sorted there, and its records are permuted on the host.  The
+ * parts of a multi-device result are concatenated first; the result is one part afterwards.
+ * Only records move: beans and accession references stay where they are, and each record still points at its own.
+ * Hit-less headers (blu_result_add_headers) are not records and are not touched, before or after this call.
+ * Order afterwards = std::stable_sort of the records by their id bytes (unsigned), applied to the order before the call.
+ * The checksum, every count and every writer's output are the same before and after; the writers then only merge the
+ * hit-less headers in instead of sorting every entry.  0 records: nothing to do.  Ids plus the sort's scratch that do not
+ * fit the device: BLU_ERR_UNSUPPORTED. */
+int blu_result_sort_by_query(blu_ctx* ctx, blu_result* res);
 uint64_t blu_result_num_rows(const blu_result* res);
 /* Host arrays of the result (the parts of a multi-device result are concatenated on the first call; the string
  * references of such a result are relative to blu_result_pool of that same concatenation). */

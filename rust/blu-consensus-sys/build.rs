@@ -8,7 +8,7 @@ fn main() {
     assert!(status.success(), "building libblu_consensus.so failed (needs nvcc with sm_100a support)");
     println!("cargo:rustc-link-search=native={}", root.join("blutils_b200").display());
     println!("cargo:rustc-link-lib=dylib=blu_consensus");
-    for f in ["blu_kernels.cu", "blu_api.cpp", "blu_taxonomy.cpp", "blu_core.cuh", "blu_decode.h"] {
+    for f in ["blu_kernels.cu", "blu_regroup.cu", "blu_sort.cu", "blu_sort.h", "blu_api.cpp", "blu_taxonomy.cpp", "blu_core.cuh", "blu_decode.h"] {
         println!("cargo:rerun-if-changed={}", csrc.join(f).display());
     }
     println!("cargo:rerun-if-changed={}", root.join("include/blu_consensus.h").display());

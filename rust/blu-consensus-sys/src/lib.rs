@@ -39,6 +39,8 @@ extern "C" {
     pub fn blu_consensus_run_host(ctx: *mut blu_ctx, text: *const c_char, n: u64, out: *mut *mut blu_result) -> c_int;
     pub fn blu_result_add_headers(res: *mut blu_result, headers_nl: *const c_char, len: u64) -> c_int;
     pub fn blu_result_num_queries(res: *const blu_result) -> u64;
+    pub fn blu_result_num_records(res: *const blu_result) -> u64;
+    pub fn blu_result_sort_by_query(ctx: *mut blu_ctx, res: *mut blu_result) -> c_int;
     pub fn blu_result_to_jsonl(res: *const blu_result, out: *mut *mut c_char, len: *mut u64) -> c_int;
     pub fn blu_result_write(res: *const blu_result, path: *const c_char, format: c_int, run_id: *const c_char) -> c_int;
     pub fn blu_result_file_to_tabular(blu_result_path: *const c_char, output_file: *const c_char, input_format: c_int, run_id: *const c_char, err: *mut c_char, errlen: size_t) -> c_int;

@@ -16,6 +16,7 @@
 #include <cerrno>
 #include <cstdio>
 #include <cstring>
+#include <exception>
 #include <filesystem>
 #include <fstream>
 #include <memory>
@@ -71,6 +72,24 @@ struct DevBuf {
         if (p) cudaFree(p);
         p = nullptr;
         cap = 0;
+    }
+};
+
+// One cudaMalloc'ed block freed by its owner: an uploaded or regrouped table, a sort's scratch.
+struct DevMem {
+    uint8_t* p = nullptr;
+    uint64_t n = 0;  // bytes of text it holds
+    DevMem() = default;
+    DevMem(const DevMem&) = delete;
+    DevMem& operator=(const DevMem&) = delete;
+    ~DevMem() {
+        if (p) cudaFree(p);
+    }
+    bool alloc(uint64_t bytes) {  // false: the device is full (the error is cleared)
+        if (cudaMalloc((void**)&p, std::max<uint64_t>(bytes, 1)) == cudaSuccess) return true;
+        cudaGetLastError();
+        p = nullptr;
+        return false;
     }
 };
 
@@ -401,6 +420,12 @@ Caps initial_caps(const blu_ctx* c, uint64_t n, bool want_pool) {
     return k;
 }
 
+inline size_t dup_table_size(const Caps& k) {
+    size_t cap = 1024;
+    while (cap < 2 * k.rec) cap <<= 1;
+    return cap;
+}
+
 void ensure_out(blu_ctx* c, const Caps& k) {
     if (!c->out) c->out = c->dev_pool->acquire();
     c->out->rec.ensure(k.rec);
@@ -409,18 +434,10 @@ void ensure_out(blu_ctx* c, const Caps& k) {
     c->d_top.ensure(k.slots);
     c->d_defer.ensure(k.defer);
     if (k.pool) c->d_pool.ensure(k.pool);
-    size_t cap = 1024;
-    while (cap < 2 * k.rec) cap <<= 1;
-    c->d_dup.ensure(cap);
+    c->d_dup.ensure(dup_table_size(k));
     if (c->keep_hashes) c->d_qhash.ensure(k.rec);
     c->d_big_rows.ensure((size_t)c->sms * kLongTopCap);
     c->d_big_cand.ensure((size_t)c->sms * kLongTopCap);
-}
-
-inline size_t dup_table_size(const Caps& k) {
-    size_t cap = 1024;
-    while (cap < 2 * k.rec) cap <<= 1;
-    return cap;
 }
 
 std::string dev_err_message(uint32_t code, uint64_t off) {
@@ -605,6 +622,59 @@ void learn_densities(blu_ctx* c, const Counters& h, uint64_t n) {
     if (h.pool_used) c->dens_pool = (double)h.pool_used / (double)n;
 }
 
+// Kernel times of a run, summed over its ranges / chunks.
+struct KernelMs {
+    double tile = 0, longrun = 0, post = 0;
+};
+
+// Reads the counter snapshot of range / chunk `slot` once its kernels have completed: its kernel times and deferred runs
+// are added up, a grammar error is raised (at `base` + err_off) before anything is done about a capacity -- a malformed
+// row is an error whatever else happened -- and on a capacity overflow the capacities are grown for the whole input of
+// `n` bytes (`scale`: see grow_caps).  true: the run has to start over.
+bool read_snapshot(blu_ctx* c, int slot, uint64_t base, Caps& k, double scale, uint64_t n, Counters& h, KernelMs& ms) {
+    const cudaEvent_t* ev = c->ev[slot];
+    CK(cudaEventSynchronize(ev[3]));
+    h = c->h_snap[slot];
+    ms.tile += ev_ms(ev[0], ev[1]);
+    ms.longrun += ev_ms(ev[1], ev[2]);
+    ms.post += ev_ms(ev[2], ev[3]);
+    c->tm.n_deferred_runs += h.n_defer;
+    check_fatal(h, base);
+    if (!overflowed(h, k)) return false;
+    grow_caps(h, k, scale, n);
+    return true;
+}
+
+// The end of a run that found no duplicate id (`h`: its last snapshot): the timings every loop reports the same way, and
+// the densities that size the next run.
+void finish_run(blu_ctx* c, const Counters& h, uint64_t n, uint64_t tiles, const KernelMs& ms) {
+    if (h.post_done == 0) throw DataErr("the blast output holds no rows");
+    c->tm.ms_tile_kernel = ms.tile;
+    c->tm.ms_longrun_kernel = ms.longrun;
+    c->tm.ms_gather_kernel = ms.post;
+    c->tm.ms_total_device = ms.tile + ms.longrun + ms.post;
+    c->tm.text_bytes = n;
+    c->tm.taxonomy_bytes = c->tax->device_bytes();
+    c->tm.n_tile_launches = tiles;
+    c->tm.n_queries = h.post_done;
+    c->tm.n_rows = h.n_rows;
+    c->tm.result_bytes = h.post_done * sizeof(blu_record) + h.bean_used * sizeof(blu_bean) + h.acc_used * sizeof(blu_acc);
+    c->tm.d2h_bytes += sizeof(Counters);
+    learn_densities(c, h, n);
+}
+
+// Synchronises the first `n` of `s` when its scope is left by an exception: nothing may still read the caller's text, or a
+// buffer that is about to be freed, when the call returns.
+struct SyncOnUnwind {
+    cudaStream_t s[3];
+    int n;
+    const int pending = std::uncaught_exceptions();
+    ~SyncOnUnwind() {
+        if (std::uncaught_exceptions() > pending)
+            for (int i = 0; i < n; i++) cudaStreamSynchronize(s[i]);
+    }
+};
+
 // Incremental download of the finished part of the result arrays on the context's download stream, so that the
 // device->host copies of one range / chunk run under the kernels (and host->device copies) of the next one.
 struct Downloader {
@@ -653,10 +723,7 @@ struct Downloader {
         CK(cudaStreamSynchronize(c->d2h_stream));
         r->n_rec = rec_done, r->n_beans = bean_done, r->n_accs = acc_done, r->pool_len = pool_done;
         r->on_host = true;
-        c->tm.d2h_bytes += bytes + sizeof(Counters);
-        c->tm.result_bytes = rec_done * sizeof(blu_record) + bean_done * sizeof(blu_bean) + acc_done * sizeof(blu_acc);
-        c->tm.n_queries = rec_done;
-        c->tm.n_rows = h.n_rows;
+        c->tm.d2h_bytes += bytes;
     }
     void abandon() {  // retry with larger device capacities: drop what was downloaded
         cudaStreamSynchronize(c->d2h_stream);
@@ -665,7 +732,7 @@ struct Downloader {
     }
 };
 
-void require_ready(blu_ctx* c) {
+void require_tax(blu_ctx* c) {
     if (!c->tax) throw std::invalid_argument("no taxonomy loaded (call blu_taxonomy_load_json first)");
 }
 
@@ -731,40 +798,34 @@ void check_device_text(const uint8_t* dtext, uint64_t n) {
     if (((uintptr_t)dtext & 15) != 0) throw std::invalid_argument("device text must be 16-byte aligned");
 }
 
-// --- text resident on the device, result downloaded -------------------------------------------------------------
-// Every range's kernels are queued up front -- a range starts where the previous one stopped (Counters.next_begin), the
-// post-pass takes its record range from the device counters -- so the GPU never waits for the host; the host trails
-// behind, reads each range's snapshot when its event fires and queues that range's download on the download stream.
-void run_device_download(blu_ctx* c, const uint8_t* dtext, uint64_t n, cudaStream_t s, ResultPartOwned* r, RunStatus& st) {
-    require_ready(c);
+// --- text resident on the device ------------------------------------------------------------------------------------
+// resident: one range, five launches, one host synchronisation; nothing but the counters crosses PCIe and the result keeps
+// the device arrays and references into the device text (SURVEY 8d(i)).
+// Otherwise the result is downloaded: every range's kernels are queued up front -- a range starts where the previous one
+// stopped (Counters.next_begin), the post-pass takes its record range from the device counters -- so the GPU never waits
+// for the host; the host trails behind, reads each range's snapshot when its event fires and queues that range's download
+// on the download stream.
+void run_device_text(blu_ctx* c, const uint8_t* dtext, uint64_t n, cudaStream_t s, ResultPartOwned* r, RunStatus& st, bool resident) {
+    SyncOnUnwind unwind{{s, c->d2h_stream}, resident ? 1 : 2};
+    require_tax(c);
     check_device_text(dtext, n);
     c->tm = blu_timings{};
     if (c->dens_rec == 0 && n > (64ull << 20)) probe_densities(c, dtext, 0, std::min<uint64_t>(n, 32ull << 20), s);
-    Caps k = initial_caps(c, n, true);
-    const std::vector<uint64_t> range_end = resident_ranges(n);
+    Caps k = initial_caps(c, n, !resident);
+    const std::vector<uint64_t> range_end = resident ? std::vector<uint64_t>{n} : resident_ranges(n);
     const int n_ranges = (int)range_end.size();
+    const Strings strings = resident ? Strings::DeviceText : Strings::Pool;
     Downloader dl(c, r);
     for (int attempt = 0; attempt < 8; attempt++) {
         begin_run(c, k, s);
         for (int ri = 0; ri < n_ranges; ri++)
-            launch_range(c, dtext, ri == 0 ? 0 : kBeginFromCounters, range_end[ri], ri + 1 == n_ranges, k, s, ri, Strings::Pool, 0);
+            launch_range(c, dtext, ri == 0 ? 0 : kBeginFromCounters, range_end[ri], ri + 1 == n_ranges, k, s, ri, strings, 0);
         bool retry = false;
         Counters h{};
-        double ms_tile = 0, ms_long = 0, ms_post = 0;
-        for (int ri = 0; ri < n_ranges; ri++) {
-            CK(cudaEventSynchronize(c->ev[ri][3]));
-            h = c->h_snap[ri];
-            ms_tile += ev_ms(c->ev[ri][0], c->ev[ri][1]);
-            ms_long += ev_ms(c->ev[ri][1], c->ev[ri][2]);
-            ms_post += ev_ms(c->ev[ri][2], c->ev[ri][3]);
-            c->tm.n_deferred_runs += h.n_defer;
-            check_fatal(h, 0);  // (before anything is done about a capacity: a malformed row is an error whatever else happened)
-            if (overflowed(h, k)) {
-                grow_caps(h, k, (double)n / (double)std::max<uint64_t>(range_end[ri], 1), n);
-                retry = true;
-                break;
-            }
-            if (ri + 1 < n_ranges && !h.dup_found) {
+        KernelMs ms;
+        for (int ri = 0; ri < n_ranges && !retry; ri++) {
+            retry = read_snapshot(c, ri, 0, k, (double)n / (double)std::max<uint64_t>(range_end[ri], 1), n, h, ms);
+            if (!retry && ri + 1 < n_ranges && !h.dup_found) {
                 if (ri == 0 && range_end[0] > 0) {
                     // size the pinned result buffers from the density of the first range
                     const double f = 1.15 * (double)n / (double)range_end[0];
@@ -775,66 +836,24 @@ void run_device_download(blu_ctx* c, const uint8_t* dtext, uint64_t n, cudaStrea
             }
         }
         if (retry) {
-            CK(cudaStreamSynchronize(s));  // the later ranges are still queued
-            dl.abandon();
+            if (!resident) {
+                CK(cudaStreamSynchronize(s));  // the later ranges are still queued
+                dl.abandon();
+            }
             c->tm = blu_timings{};
             continue;
         }
         st.note_soft(h, 0);
         st.dup_found = h.dup_found != 0;
         if (st.dup_found) {
-            dl.abandon();
+            if (!resident) dl.abandon();
             return;
         }
-        if (h.post_done == 0) throw DataErr("the blast output holds no rows");
-        c->tm.ms_tile_kernel = ms_tile;
-        c->tm.ms_longrun_kernel = ms_long;
-        c->tm.ms_gather_kernel = ms_post;
-        c->tm.ms_total_device = ms_tile + ms_long + ms_post;
-        c->tm.text_bytes = n;
-        c->tm.taxonomy_bytes = c->tax->device_bytes();
-        c->tm.n_tile_launches = (uint64_t)n_ranges;
-        dl.finish(h);
-        learn_densities(c, h, n);
-        return;
-    }
-    throw std::runtime_error("output capacity did not converge");
-}
-
-// --- text resident on the device, result stays on the device (SURVEY 8d(i)) ----------------------------------------------
-// One range, five launches, one host synchronisation; nothing but the counters crosses PCIe.
-void run_device_resident(blu_ctx* c, const uint8_t* dtext, uint64_t n, cudaStream_t s, ResultPartOwned* r, RunStatus& st) {
-    require_ready(c);
-    check_device_text(dtext, n);
-    c->tm = blu_timings{};
-    if (c->dens_rec == 0 && n > (64ull << 20)) probe_densities(c, dtext, 0, std::min<uint64_t>(n, 32ull << 20), s);
-    Caps k = initial_caps(c, n, false);
-    for (int attempt = 0; attempt < 8; attempt++) {
-        begin_run(c, k, s);
-        launch_range(c, dtext, 0, n, true, k, s, 0, Strings::DeviceText, 0);
-        CK(cudaEventSynchronize(c->ev[0][3]));
-        const Counters h = c->h_snap[0];
-        check_fatal(h, 0);
-        if (overflowed(h, k)) {
-            grow_caps(h, k, 1.0, n);
-            c->tm = blu_timings{};
-            continue;
+        finish_run(c, h, n, (uint64_t)n_ranges, ms);
+        if (!resident) {
+            dl.finish(h);
+            return;
         }
-        st.note_soft(h, 0);
-        st.dup_found = h.dup_found != 0;
-        if (!st.dup_found && h.post_done == 0) throw DataErr("the blast output holds no rows");
-        c->tm.ms_tile_kernel = ev_ms(c->ev[0][0], c->ev[0][1]);
-        c->tm.ms_longrun_kernel = ev_ms(c->ev[0][1], c->ev[0][2]);
-        c->tm.ms_gather_kernel = ev_ms(c->ev[0][2], c->ev[0][3]);
-        c->tm.ms_total_device = c->tm.ms_tile_kernel + c->tm.ms_longrun_kernel + c->tm.ms_gather_kernel;
-        c->tm.n_deferred_runs = h.n_defer;
-        c->tm.text_bytes = n;
-        c->tm.taxonomy_bytes = c->tax->device_bytes();
-        c->tm.n_tile_launches = 1;
-        c->tm.n_queries = h.post_done;
-        c->tm.n_rows = h.n_rows;
-        c->tm.d2h_bytes = sizeof(Counters);
-        c->tm.result_bytes = h.post_done * sizeof(blu_record) + h.bean_used * sizeof(blu_bean) + h.acc_used * sizeof(blu_acc);
         r->dev = std::move(c->out);
         r->dev_pool = c->dev_pool;
         r->ctx = c;
@@ -842,7 +861,6 @@ void run_device_resident(blu_ctx* c, const uint8_t* dtext, uint64_t n, cudaStrea
         r->dtext_len = n;
         r->n_rec = h.post_done, r->n_beans = h.bean_used, r->n_accs = h.acc_used;
         r->on_host = false;
-        learn_densities(c, h, n);
         return;
     }
     throw std::runtime_error("output capacity did not converge");
@@ -940,18 +958,7 @@ std::string regroup_by_query(const char* text, uint64_t n) {
 
 // The same regrouping on the GPU (blu_regroup.cu): the table -- uploaded first when it is host text -- is rewritten in HBM.
 // Used whenever the table, its regrouped copy and ~72 bytes per row fit the device; BLU_REGROUP_HOST=1 forces the host path.
-struct DevText {
-    uint8_t* p = nullptr;
-    uint64_t n = 0;
-    DevText() = default;
-    DevText(const DevText&) = delete;
-    DevText& operator=(const DevText&) = delete;
-    ~DevText() {
-        if (p) cudaFree(p);
-    }
-};
-
-bool regroup_gpu(blu_ctx* c, const char* h_text, const uint8_t* d_text, uint64_t n, cudaStream_t s, DevText& out) {
+bool regroup_gpu(blu_ctx* c, const char* h_text, const uint8_t* d_text, uint64_t n, cudaStream_t s, DevMem& out) {
     if (const char* ev = getenv("BLU_REGROUP_HOST"))
         if (atoi(ev)) return false;
     if (n == 0) return false;
@@ -960,23 +967,18 @@ bool regroup_gpu(blu_ctx* c, const char* h_text, const uint8_t* d_text, uint64_t
         s = c->stream;
     }
     CK(cudaSetDevice(c->device));
-    DevText in;
-    const auto t_begin = std::chrono::steady_clock::now();
-    (void)t_begin;
+    DevMem in;
+    const auto t0 = std::chrono::steady_clock::now();
     if (!d_text) {
         size_t free_b = 0, total_b = 0;
         CK(cudaMemGetInfo(&free_b, &total_b));
         if (2.2 * (double)n + (double)(256ull << 20) > (double)free_b) return false;
-        if (cudaMalloc((void**)&in.p, n + 512) != cudaSuccess) {
-            cudaGetLastError();
-            return false;
-        }
+        if (!in.alloc(n + 512)) return false;
         CK(cudaMemcpyAsync(in.p, h_text, n, cudaMemcpyHostToDevice, s));
         d_text = in.p;
     }
     uint64_t rows = 0;
     const bool trace = getenv("BLU_REGROUP_TRACE") != nullptr;
-    const auto t0 = t_begin;
     if (trace) cudaStreamSynchronize(s);
     const auto t1 = std::chrono::steady_clock::now();
     const int rc = regroup_device(d_text, n, s, &out.p, &out.n, &rows);
@@ -1147,7 +1149,8 @@ inline uint64_t chunk_bytes_of(const blu_ctx* c, uint64_t dflt) { return c->opts
 
 // `host_text` != nullptr: BLU_OPT_TEXT_REFS -- the result's strings stay references into that (caller-owned) text.
 void run_host_chunks(blu_ctx* c, ChunkSource& src, uint64_t n, const uint64_t chunk, ResultPartOwned* r, RunStatus& st, const char* host_text) {
-    require_ready(c);
+    SyncOnUnwind unwind{{c->copy_stream, c->stream, c->d2h_stream}, 3};  // (and nothing may still copy from a staging buffer)
+    require_tax(c);
     if (n == 0) throw DataErr("empty blast output (the reference's CsvReader fails on an empty file)");
     c->tm = blu_timings{};
     const uint64_t carry = c->carry_bytes;
@@ -1166,8 +1169,7 @@ void run_host_chunks(blu_ctx* c, ChunkSource& src, uint64_t n, const uint64_t ch
     for (int attempt = 0; attempt < 8; attempt++) {
         bool retry = false;
         uint64_t tail_len = 0;  // bytes carried from the previous chunk
-        double ms_tile = 0, ms_long = 0, ms_post = 0;
-        uint64_t launches = 0;
+        KernelMs ms;
         Counters h{};
         auto issue_h2d = [&](uint64_t ci) {
             const uint64_t off = ci * chunk, len = std::min(chunk, n - off);
@@ -1186,7 +1188,7 @@ void run_host_chunks(blu_ctx* c, ChunkSource& src, uint64_t n, const uint64_t ch
             have_caps = true;
         }
         begin_run(c, k, s);
-        for (uint64_t ci = 0; ci < n_chunks && !retry; ci++) {
+        for (uint64_t ci = 0; ci < n_chunks; ci++) {
             const uint64_t off = ci * chunk, len = std::min(chunk, n - off);
             const bool final_chunk = ci + 1 == n_chunks;
             const int slot = (int)(ci % kMaxRanges);
@@ -1206,20 +1208,9 @@ void run_host_chunks(blu_ctx* c, ChunkSource& src, uint64_t n, const uint64_t ch
                 CK(cudaStreamWaitEvent(cs, c->ev_free[(ci + 1) & 1], 0));
                 issue_h2d(ci + 1);
             }
-            CK(cudaEventSynchronize(c->ev[slot][3]));
+            retry = read_snapshot(c, slot, off - text_off, k, (double)n / (double)(off + len), n, h, ms);  // err_off is in buffer coordinates
             src.release(ci);  // `s` waited for this chunk's copy, so it has completed
-            h = c->h_snap[slot];
-            ms_tile += ev_ms(c->ev[slot][0], c->ev[slot][1]);
-            ms_long += ev_ms(c->ev[slot][1], c->ev[slot][2]);
-            ms_post += ev_ms(c->ev[slot][2], c->ev[slot][3]);
-            c->tm.n_deferred_runs += h.n_defer;
-            launches++;
-            check_fatal(h, off - text_off);  // err_off is in buffer coordinates
-            if (overflowed(h, k)) {
-                grow_caps(h, k, (double)n / (double)(off + len), n);
-                retry = true;
-                break;
-            }
+            if (retry) break;
             st.note_soft(h, off - text_off);
             if (!final_chunk) {
                 tail_len = end - h.next_begin;  // (next_begin == end: nothing is carried)
@@ -1248,38 +1239,13 @@ void run_host_chunks(blu_ctx* c, ChunkSource& src, uint64_t n, const uint64_t ch
             dl.abandon();
             return;
         }
-        if (h.post_done == 0) throw DataErr("the blast output holds no rows");
-        c->tm.ms_tile_kernel = ms_tile;
-        c->tm.ms_longrun_kernel = ms_long;
-        c->tm.ms_gather_kernel = ms_post;
-        c->tm.text_bytes = n;
-        c->tm.taxonomy_bytes = c->tax->device_bytes();
-        c->tm.n_tile_launches = launches;
+        finish_run(c, h, n, n_chunks, ms);
         dl.finish(h);
         if (host_text) r->ext_strings = host_text, r->ext_len = n;
         c->tm.ms_total_device = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-        learn_densities(c, h, n);
         return;
     }
     throw std::runtime_error("output capacity did not converge");
-}
-
-// On any failure nothing may still be reading the caller's text (or a staging buffer) when the call returns.
-void run_host_source(blu_ctx* c, ChunkSource& src, uint64_t n, uint64_t chunk, ResultPartOwned* r, RunStatus& st, const char* host_text) {
-    try {
-        run_host_chunks(c, src, n, chunk, r, st, host_text);
-    } catch (...) {
-        cudaStreamSynchronize(c->copy_stream);
-        cudaStreamSynchronize(c->stream);
-        cudaStreamSynchronize(c->d2h_stream);
-        throw;
-    }
-}
-
-void run_host_single(blu_ctx* c, const char* text, uint64_t n, ResultPartOwned* r, RunStatus& st, bool text_refs) {
-    const uint64_t chunk = chunk_bytes_of(c, 256ull << 20);
-    MemorySource src(text, chunk);
-    run_host_source(c, src, n, chunk, r, st, text_refs ? text : nullptr);
 }
 
 // ---- sharding (SURVEY 8e) ---------------------------------------------------------------------------------------
@@ -1289,6 +1255,8 @@ struct ByteView {
     const char* mem = nullptr;
     int fd = -1;
     uint64_t n = 0;
+    ByteView(const char* text, uint64_t len) : mem(text), n(len) {}
+    ByteView(int file, uint64_t len) : fd(file), n(len) {}
     mutable std::vector<char> win;
     mutable uint64_t win_lo = 0, win_hi = 0;
     char at(uint64_t i) const {
@@ -1450,53 +1418,99 @@ void settle_multi(blu_ctx* c, const std::vector<RunStatus>& st, const uint64_t* 
         if (st[i].soft_code) throw_device_error(st[i].soft_code, cuts[i] + st[i].soft_off);
 }
 
-void run_host_multi(blu_ctx* c, const char* text, uint64_t n, blu_result* r, bool text_refs) {
-    if (n == 0) throw DataErr("empty blast output (the reference's CsvReader fails on an empty file)");
-    const size_t N = c->shards.size();
-    std::vector<uint64_t> cuts(N + 1);
-    ByteView v;
-    v.mem = text, v.n = n;
-    shard_cuts(v, (int)N, cuts.data());
+// Drops what a result holds and gives it n empty parts.
+void reset_parts(blu_result* r, size_t n) {
+    for (auto& p : r->parts) p.free_buffers();
     r->parts.clear();
-    r->parts.resize(N);
-    std::vector<RunStatus> st(N);
-    auto t0 = std::chrono::steady_clock::now();
-    for_each_shard(c, [&](size_t i) {
-        c->shards[i]->tm = blu_timings{};
-        if (cuts[i + 1] > cuts[i]) run_host_single(c->shards[i].get(), text + cuts[i], cuts[i + 1] - cuts[i], &r->parts[i], st[i], text_refs);
-    });
-    std::vector<uint64_t> n_rec(N);
-    for (size_t i = 0; i < N; i++) n_rec[i] = st[i].dup_found ? 0 : r->parts[i].n_rec;
-    settle_multi(c, st, cuts.data(), n_rec);
-    aggregate_timings(c, n, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count());
-    r->n_rows = c->tm.n_rows;
+    r->parts.resize(n);
 }
 
-void run_file_multi(blu_ctx* c, int fd, uint64_t n, blu_result* r) {
-    if (n == 0) throw DataErr("empty blast output (the reference's CsvReader fails on an empty file)");
+// Bytes [begin, begin + len) of a table in memory or in a file through the host-text loop of a single-device context.
+// `sharers`: the file sources of a multi-device run that share the host's cores.
+void run_span(blu_ctx* c, const ByteView& v, uint64_t begin, uint64_t len, ResultPartOwned* p, RunStatus& st, bool text_refs, int sharers) {
+    if (v.mem) {
+        const uint64_t chunk = chunk_bytes_of(c, 256ull << 20);
+        MemorySource src(v.mem + begin, chunk);
+        run_host_chunks(c, src, len, chunk, p, st, text_refs ? v.mem + begin : nullptr);
+    } else {
+        const uint64_t chunk = chunk_bytes_of(c, 64ull << 20);
+        FileSource src(c, v.fd, begin, len, chunk, sharers);
+        run_host_chunks(c, src, len, chunk, p, st, nullptr);
+    }
+}
+
+// One table over the GPUs of a multi-device context: cut at query boundaries, each shard run on its own host thread.
+void run_sharded(blu_ctx* c, const ByteView& v, blu_result* r, bool text_refs) {
+    if (v.n == 0) throw DataErr("empty blast output (the reference's CsvReader fails on an empty file)");
     const size_t N = c->shards.size();
     std::vector<uint64_t> cuts(N + 1);
-    ByteView v;
-    v.fd = fd, v.n = n;
     shard_cuts(v, (int)N, cuts.data());
-    r->parts.clear();
-    r->parts.resize(N);
+    reset_parts(r, N);
     std::vector<RunStatus> st(N);
     auto t0 = std::chrono::steady_clock::now();
     for_each_shard(c, [&](size_t i) {
         blu_ctx* sh = c->shards[i].get();
         sh->tm = blu_timings{};
-        const uint64_t len = cuts[i + 1] - cuts[i];
-        if (!len) return;
-        const uint64_t chunk = chunk_bytes_of(sh, 64ull << 20);
-        FileSource src(sh, fd, cuts[i], len, chunk, (int)N);
-        run_host_source(sh, src, len, chunk, &r->parts[i], st[i], nullptr);
+        if (cuts[i + 1] > cuts[i]) run_span(sh, v, cuts[i], cuts[i + 1] - cuts[i], &r->parts[i], st[i], text_refs, (int)N);
     });
     std::vector<uint64_t> n_rec(N);
     for (size_t i = 0; i < N; i++) n_rec[i] = st[i].dup_found ? 0 : r->parts[i].n_rec;
     settle_multi(c, st, cuts.data(), n_rec);
-    aggregate_timings(c, n, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count());
+    aggregate_timings(c, v.n, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count());
     r->n_rows = c->tm.n_rows;
+}
+
+// A table in host memory or a file -> result, on one or several GPUs.  `text_refs` applies to host memory only.
+void run_table(blu_ctx* c, const ByteView& v, blu_result* r, bool text_refs) {
+    if (c->is_multi()) {
+        run_sharded(c, v, r, text_refs);
+        return;
+    }
+    CK(cudaSetDevice(c->device));
+    reset_parts(r, 1);
+    RunStatus st;
+    run_span(c, v, 0, v.n, &r->parts[0], st, text_refs, 1);
+    settle(st);
+    r->n_rows = c->tm.n_rows;
+}
+
+// The regrouped table (device memory of ours) through the device-text loop of a single-device context.
+void run_regrouped_device(blu_ctx* c, const DevMem& dt, cudaStream_t s, blu_result* r, bool resident) {
+    reset_parts(r, 1);
+    RunStatus st;
+    run_device_text(c, dt.p, dt.n, s, &r->parts[0], st, resident);
+    if (st.dup_found) throw std::runtime_error("a regrouped table is still not contiguous");
+    settle(st);
+    r->n_rows = c->tm.n_rows;
+}
+
+// A scattered table, host text or device text (single-device context), regrouped -- on the GPU when regroup_gpu allows it,
+// else on the host -- and run again.  The regrouped text is ours: the result's strings are copied into a pool.
+void run_scattered(blu_ctx* c, const char* h_text, const uint8_t* d_text, uint64_t n, cudaStream_t s, blu_result* r) {
+    DevMem dt;
+    if (regroup_gpu(c, h_text, d_text, n, s, dt)) {
+        if (c->is_multi()) {
+            // the shards start from host text: the regrouped table comes back once and is cut like any other
+            std::string re((size_t)dt.n, '\0');
+            CK(cudaMemcpy(re.data(), dt.p, dt.n, cudaMemcpyDeviceToHost));
+            cudaFree(dt.p);
+            dt.p = nullptr;
+            run_table(c, ByteView(re.data(), re.size()), r, false);
+        } else
+            run_regrouped_device(c, dt, c->stream, r, false);
+        c->tm.n_regrouped = 2;
+        return;
+    }
+    std::string host;
+    if (!h_text) {
+        host.resize((size_t)n);
+        CK(cudaMemcpy(host.data(), d_text, n, cudaMemcpyDeviceToHost));
+        h_text = host.data();
+    }
+    const std::string re = regroup_by_query(h_text, n);
+    std::string().swap(host);
+    run_table(c, ByteView(re.data(), re.size()), r, false);
+    c->tm.n_regrouped = 1;
 }
 
 std::unique_ptr<blu_result> new_result(blu_ctx* c) {
@@ -1571,23 +1585,11 @@ struct SortTrace {
 };
 
 // device scratch of one sort call
-struct CudaMem {
-    void* p = nullptr;
-    CudaMem() = default;
-    CudaMem(const CudaMem&) = delete;
-    CudaMem& operator=(const CudaMem&) = delete;
-    ~CudaMem() {
-        if (p) cudaFree(p);
-    }
-    template <class T>
-    T* alloc(uint64_t count) {
-        if (cudaMalloc(&p, std::max<uint64_t>(count, 1) * sizeof(T)) != cudaSuccess) {
-            cudaGetLastError();
-            throw UnsupportedErr("the query ids and the sort's scratch do not fit the device");
-        }
-        return (T*)p;
-    }
-};
+template <class T>
+T* sort_scratch(DevMem& m, uint64_t count) {
+    if (!m.alloc(std::max<uint64_t>(count, 1) * sizeof(T))) throw UnsupportedErr("the query ids and the sort's scratch do not fit the device");
+    return (T*)m.p;
+}
 
 // the ids (id_bytes), their references, the permutation, `extra` bytes and the sort's scratch must fit the free device memory
 void require_sort_fits(uint64_t n, uint64_t id_bytes, uint64_t extra) {
@@ -1612,10 +1614,10 @@ void sort_part_device(blu_ctx* c, ResultPartOwned& p) {
     const uint32_t n = (uint32_t)p.n_rec;
     SortTrace tr(s);
     require_sort_fits(n, 0, (uint64_t)n * sizeof(blu_record));
-    CudaMem m_off, m_len, m_perm;
-    uint64_t* off = m_off.alloc<uint64_t>(n);
-    uint32_t* len = m_len.alloc<uint32_t>(n);
-    uint32_t* perm = m_perm.alloc<uint32_t>(n);
+    DevMem m_off, m_len, m_perm;
+    uint64_t* off = sort_scratch<uint64_t>(m_off, n);
+    uint32_t* len = sort_scratch<uint32_t>(m_len, n);
+    uint32_t* perm = sort_scratch<uint32_t>(m_perm, n);
     CK(launch_record_ids(p.dev->rec.p, n, off, len, s));
     sort_ids_checked(p.dtext, off, len, n, perm, s);
     tr.mark("sort");
@@ -1708,11 +1710,11 @@ void sort_part_host(blu_ctx* g, ResultPartOwned& p) {
     require_sort_fits(n, id_bytes, 0);
     Pinned h_perm{g->pool, g->acquire(n * sizeof(uint32_t))};
     {
-        CudaMem m_ids, m_off, m_len, m_perm;
-        uint8_t* d_ids = m_ids.alloc<uint8_t>(id_bytes);
-        uint64_t* d_off = m_off.alloc<uint64_t>(n);
-        uint32_t* d_len = m_len.alloc<uint32_t>(n);
-        uint32_t* d_perm = m_perm.alloc<uint32_t>(n);
+        DevMem m_ids, m_off, m_len, m_perm;
+        uint8_t* d_ids = sort_scratch<uint8_t>(m_ids, id_bytes);
+        uint64_t* d_off = sort_scratch<uint64_t>(m_off, n);
+        uint32_t* d_len = sort_scratch<uint32_t>(m_len, n);
+        uint32_t* d_perm = sort_scratch<uint32_t>(m_perm, n);
         try {
             if (id_bytes) CK(cudaMemcpyAsync(d_ids, ids, id_bytes, cudaMemcpyHostToDevice, s));
             CK(cudaMemcpyAsync(d_off, off, n * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
@@ -1737,6 +1739,23 @@ void sort_part_host(blu_ctx* g, ResultPartOwned& p) {
     p.pinned->release(p.b_rec);
     p.b_rec = out;
     tr.mark("permute");
+}
+
+// What every blu_consensus_run_* entry point does with its result: made for `run`, handed out on success, freed on failure.
+template <class F>
+int run_entry(blu_ctx* c, blu_result** out, F&& run) {
+    std::unique_ptr<blu_result> r;
+    const int rc = guarded(c, [&] {
+        require_tax(c);
+        r = new_result(c);
+        run(r.get());
+    });
+    if (rc != BLU_OK) {
+        blu_result_free(r.release());
+        return rc;
+    }
+    *out = r.release();
+    return BLU_OK;
 }
 
 }  // namespace
@@ -1945,177 +1964,50 @@ int blu_taxonomy_load_json_cached(blu_ctx* c, const char* path, const char* cach
     });
 }
 
-static void require_tax(blu_ctx* c) {
-    if (!c->tax) throw std::invalid_argument("no taxonomy loaded (call blu_taxonomy_load_json first)");
-}
-
-// the regrouped table (device memory of ours) through the device-text path of a single-device context
-static void run_regrouped_device(blu_ctx* c, const DevText& dt, blu_result* r) {
-    for (auto& p : r->parts) p.free_buffers();
-    r->parts.clear();
-    r->parts.resize(1);
-    RunStatus st;
-    try {
-        run_device_download(c, dt.p, dt.n, c->stream, &r->parts[0], st);
-    } catch (...) {  // nothing may still be reading the regrouped text when it is freed
-        cudaStreamSynchronize(c->stream);
-        cudaStreamSynchronize(c->d2h_stream);
-        throw;
-    }
-    if (st.dup_found) throw std::runtime_error("a regrouped table is still not contiguous");
-    settle(st);
-    r->n_rows = c->tm.n_rows;
-}
-
-// host text -> result, on one or several GPUs
-static void run_host_once(blu_ctx* c, const char* t, uint64_t len, blu_result* r, bool text_refs) {
-    for (auto& p : r->parts) p.free_buffers();
-    r->parts.clear();
-    if (c->is_multi()) {
-        run_host_multi(c, t, len, r, text_refs);
-    } else {
-        CK(cudaSetDevice(c->device));
-        r->parts.resize(1);
-        RunStatus st;
-        run_host_single(c, t, len, &r->parts[0], st, text_refs);
-        settle(st);
-        r->n_rows = c->tm.n_rows;
-    }
-}
-
-// a scattered table in host memory: regrouped (data movement only; on the GPU when it fits, else on the host) and run.
-// The regrouped text is ours: the result's strings are copied into a pool.
-static void run_scattered_host(blu_ctx* c, const char* text, uint64_t n, blu_result* r) {
-    DevText dt;
-    if (regroup_gpu(c, text, nullptr, n, c->stream, dt)) {
-        if (c->is_multi()) {
-            // the shards start from host text: the regrouped table comes back once and is cut like any other
-            std::string re((size_t)dt.n, '\0');
-            CK(cudaMemcpy(re.data(), dt.p, dt.n, cudaMemcpyDeviceToHost));
-            cudaFree(dt.p);
-            dt.p = nullptr;
-            run_host_once(c, re.data(), re.size(), r, false);
-        } else
-            run_regrouped_device(c, dt, r);
-        c->tm.n_regrouped = 2;
-    } else {
-        const std::string re = regroup_by_query(text, n);
-        run_host_once(c, re.data(), re.size(), r, false);
-        c->tm.n_regrouped = 1;
-    }
-}
-
-static void run_host_any(blu_ctx* c, const char* text, uint64_t n, blu_result* r) {
-    try {
-        run_host_once(c, text, n, r, (c->opts.flags & BLU_OPT_TEXT_REFS) != 0);
-    } catch (const NonContiguous&) {
-        run_scattered_host(c, text, n, r);
-    }
-}
-
 int blu_consensus_run_device(blu_ctx* c, const void* dtext, uint64_t n, void* stream, blu_result** out) {
     if (!c || !out || (!dtext && n)) return fail(c, BLU_ERR_ARG, "null argument");
     *out = nullptr;
     if (c->is_multi()) return fail(c, BLU_ERR_ARG, "device-resident text belongs to one GPU: use a single-device context");
-    std::unique_ptr<blu_result> r;
-    int rc = guarded(c, [&] {
-        require_tax(c);
-        r = new_result(c);
+    return run_entry(c, out, [&](blu_result* r) {
         CK(cudaSetDevice(c->device));
         cudaStream_t s = stream ? (cudaStream_t)stream : c->stream;
         try {
-            r->parts.resize(1);
+            reset_parts(r, 1);
             RunStatus st;
-            try {
-                run_device_download(c, (const uint8_t*)dtext, n, s, &r->parts[0], st);
-            } catch (...) {  // nothing may still be reading the caller's device text when the call returns
-                cudaStreamSynchronize(s);
-                cudaStreamSynchronize(c->d2h_stream);
-                throw;
-            }
+            run_device_text(c, (const uint8_t*)dtext, n, s, &r->parts[0], st, false);
             settle(st);
             r->n_rows = c->tm.n_rows;
         } catch (const NonContiguous&) {
-            DevText dt;
-            if (regroup_gpu(c, nullptr, (const uint8_t*)dtext, n, s, dt)) {
-                run_regrouped_device(c, dt, r.get());
-                c->tm.n_regrouped = 2;
-                return;
-            }
-            // regroup on the host (data movement only), then the normal streamed path
-            std::string host(n, '\0');
-            CK(cudaMemcpy(host.data(), dtext, n, cudaMemcpyDeviceToHost));
-            std::string re = regroup_by_query(host.data(), n);
-            std::string().swap(host);
-            for (auto& p : r->parts) p.free_buffers();
-            r->parts.clear();
-            r->parts.resize(1);
-            RunStatus st;
-            run_host_single(c, re.data(), re.size(), &r->parts[0], st, false);
-            settle(st);
-            r->n_rows = c->tm.n_rows;
-            c->tm.n_regrouped = 1;
+            run_scattered(c, nullptr, (const uint8_t*)dtext, n, s, r);
         }
     });
-    if (rc != BLU_OK) {
-        blu_result_free(r.release());
-        return rc;
-    }
-    *out = r.release();
-    return BLU_OK;
 }
 
 int blu_consensus_run_device_resident(blu_ctx* c, const void* dtext, uint64_t n, void* stream, blu_result** out) {
     if (!c || !out || (!dtext && n)) return fail(c, BLU_ERR_ARG, "null argument");
     *out = nullptr;
     if (c->is_multi()) return fail(c, BLU_ERR_ARG, "device-resident text belongs to one GPU: use a single-device context");
-    std::unique_ptr<blu_result> r;
-    int rc = guarded(c, [&] {
-        require_tax(c);
-        r = new_result(c);
+    return run_entry(c, out, [&](blu_result* r) {
         CK(cudaSetDevice(c->device));
         cudaStream_t s = stream ? (cudaStream_t)stream : c->stream;
-        r->parts.resize(1);
+        reset_parts(r, 1);
         RunStatus st;
-        try {
-            run_device_resident(c, (const uint8_t*)dtext, n, s, &r->parts[0], st);
-        } catch (...) {
-            cudaStreamSynchronize(s);
-            throw;
-        }
-        if (st.dup_found) {
-            // a scattered table: regrouped in HBM (blu_regroup.cu); the result's references then point into that copy, which
-            // the result owns (blu_result_device_text)
-            DevText dt;
-            if (!regroup_gpu(c, nullptr, (const uint8_t*)dtext, n, s, dt))
-                throw UnsupportedErr("the table's queries are not contiguous and it cannot be regrouped on the device: use blu_consensus_run_device / _host / _file");
-            for (auto& p : r->parts) p.free_buffers();
-            r->parts.clear();
-            r->parts.resize(1);
-            RunStatus st2;
-            try {
-                run_device_resident(c, dt.p, dt.n, s, &r->parts[0], st2);
-            } catch (...) {
-                cudaStreamSynchronize(s);
-                throw;
-            }
-            if (st2.dup_found) throw std::runtime_error("a regrouped table is still not contiguous");
-            r->parts[0].owned_dtext = std::shared_ptr<uint8_t>(dt.p, [](uint8_t* q) { cudaFree(q); });
-            dt.p = nullptr;
-            settle(st2);
+        run_device_text(c, (const uint8_t*)dtext, n, s, &r->parts[0], st, true);
+        if (!st.dup_found) {
+            settle(st);
             r->n_rows = c->tm.n_rows;
-            c->tm.n_regrouped = 2;
             return;
         }
-        settle(st);
-        r->n_rows = c->tm.n_rows;
+        // a scattered table: regrouped in HBM (blu_regroup.cu); the result's references then point into that copy, which
+        // the result owns (blu_result_device_text)
+        DevMem dt;
+        if (!regroup_gpu(c, nullptr, (const uint8_t*)dtext, n, s, dt))
+            throw UnsupportedErr("the table's queries are not contiguous and it cannot be regrouped on the device: use blu_consensus_run_device / _host / _file");
+        run_regrouped_device(c, dt, s, r, true);
+        r->parts[0].owned_dtext = std::shared_ptr<uint8_t>(dt.p, [](uint8_t* q) { cudaFree(q); });
+        dt.p = nullptr;
+        c->tm.n_regrouped = 2;
     });
-    if (rc != BLU_OK) {
-        blu_result_free(r.release());
-        return rc;
-    }
-    *out = r.release();
-    return BLU_OK;
 }
 
 const void* blu_result_device_text(const blu_result* r, uint64_t* n) {
@@ -2172,18 +2064,13 @@ int blu_result_sort_by_query(blu_ctx* c, blu_result* r) {
 int blu_consensus_run_host(blu_ctx* c, const char* text, uint64_t n, blu_result** out) {
     if (!c || !out || (!text && n)) return fail(c, BLU_ERR_ARG, "null argument");
     *out = nullptr;
-    std::unique_ptr<blu_result> r;
-    int rc = guarded(c, [&] {
-        require_tax(c);
-        r = new_result(c);
-        run_host_any(c, text, n, r.get());
+    return run_entry(c, out, [&](blu_result* r) {
+        try {
+            run_table(c, ByteView(text, n), r, (c->opts.flags & BLU_OPT_TEXT_REFS) != 0);
+        } catch (const NonContiguous&) {
+            run_scattered(c, text, nullptr, n, c->stream, r);
+        }
     });
-    if (rc != BLU_OK) {
-        blu_result_free(r.release());
-        return rc;
-    }
-    *out = r.release();
-    return BLU_OK;
 }
 
 // Streams the file (FileSource); only a non-contiguous table (regrouping needs all rows at once) is read whole.
@@ -2200,31 +2087,11 @@ int blu_consensus_run_file(blu_ctx* c, const char* path, blu_result** out) {
     if (f.fd < 0 || fstat(f.fd, &st) != 0 || !S_ISREG(st.st_mode))
         return fail(c, BLU_ERR_IO, "Unexpected error occurred on load table.");  // mod.rs:357-364
     const uint64_t n = (uint64_t)st.st_size;
-    std::unique_ptr<blu_result> r;
-    bool regroup = false;
-    int rc = guarded(c, [&] {
-        require_tax(c);
-        r = new_result(c);
+    return run_entry(c, out, [&](blu_result* r) {
         if (n == 0) throw DataErr("empty blast output (the reference's CsvReader fails on an empty file)");
         try {
-            if (c->is_multi()) {
-                run_file_multi(c, f.fd, n, r.get());
-            } else {
-                CK(cudaSetDevice(c->device));
-                const uint64_t chunk = chunk_bytes_of(c, 64ull << 20);
-                FileSource src(c, f.fd, 0, n, chunk);
-                r->parts.resize(1);
-                RunStatus rs;
-                run_host_source(c, src, n, chunk, &r->parts[0], rs, nullptr);
-                settle(rs);
-                r->n_rows = c->tm.n_rows;
-            }
+            run_table(c, ByteView(f.fd, n), r, false);
         } catch (const NonContiguous&) {
-            regroup = true;
-        }
-    });
-    if (rc == BLU_OK && regroup) {
-        rc = guarded(c, [&] {
             std::string all((size_t)n, '\0');
             for (uint64_t off = 0; off < n;) {
                 ssize_t got = pread(f.fd, all.data() + off, (size_t)std::min<uint64_t>(n - off, 1ull << 30), (off_t)off);
@@ -2232,15 +2099,9 @@ int blu_consensus_run_file(blu_ctx* c, const char* path, blu_result** out) {
                 if (got <= 0) throw IoErr("Unexpected error occurred on load table.");
                 off += (uint64_t)got;
             }
-            run_scattered_host(c, all.data(), n, r.get());
-        });
-    }
-    if (rc != BLU_OK) {
-        blu_result_free(r.release());
-        return rc;
-    }
-    *out = r.release();
-    return BLU_OK;
+            run_scattered(c, all.data(), nullptr, n, c->stream, r);
+        }
+    });
 }
 
 int blu_result_add_headers(blu_result* r, const char* headers_nl, uint64_t len) {
@@ -2429,9 +2290,7 @@ int blu_ctx_measure_d2h(blu_ctx* c, uint64_t bytes, double* gbps) { return measu
 
 int blu_shard_cuts(const char* text, uint64_t n, int n_shards, uint64_t* cuts) {
     if (!cuts || n_shards < 1 || (!text && n)) return BLU_ERR_ARG;
-    ByteView v;
-    v.mem = text, v.n = n;
-    shard_cuts(v, n_shards, cuts);
+    shard_cuts(ByteView(text, n), n_shards, cuts);
     return BLU_OK;
 }
 
@@ -2445,9 +2304,7 @@ int blu_shard_cuts_file(const char* path, int n_shards, uint64_t* cuts) {
     }
     int rc = BLU_OK;
     try {
-        ByteView v;
-        v.fd = fd, v.n = (uint64_t)st.st_size;
-        shard_cuts(v, n_shards, cuts);
+        shard_cuts(ByteView(fd, (uint64_t)st.st_size), n_shards, cuts);
     } catch (const std::exception&) {
         rc = BLU_ERR_IO;
     }

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Device-resident step time of the C2 workload for several splits of the table into query-aligned ranges
-(BLU_RANGE_FRACS, see run_device in blu_api.cpp).  One process, one generated table; CUDA-event timing around
+(BLU_RANGE_FRACS, see resident_ranges in blu_api.cpp).  One process, one generated table; CUDA-event timing around
 each run, median of --steps after --warmup.  Measurement tool, not part of pytest / bench.py.
 
   python tools/range_split.py "1,1,1,1" "0.28,0.28,0.28,0.16" "0.39,0.28,0.19,0.14"

@@ -65,6 +65,10 @@ SYMBOLS = [
     ("blu_result_download", C.c_int, [C.c_void_p]),
     ("blu_consensus_run_file", C.c_int, [C.c_void_p, C.c_char_p, C.POINTER(C.c_void_p)]),
     ("blu_result_add_headers", C.c_int, [C.c_void_p, C.c_char_p, C.c_uint64]),
+    ("blu_consensus_run_host_configs", C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.c_void_p, C.c_uint64, C.POINTER(C.c_void_p)]),
+    ("blu_consensus_run_file_configs", C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.c_char_p, C.POINTER(C.c_void_p)]),
+    ("blu_consensus_run_device_resident_configs", C.c_int,
+     [C.POINTER(C.c_void_p), C.c_int, C.c_void_p, C.c_uint64, C.c_void_p, C.POINTER(C.c_void_p)]),
     ("blu_result_num_queries", C.c_uint64, [C.c_void_p]),
     ("blu_result_num_records", C.c_uint64, [C.c_void_p]),
     ("blu_result_sort_by_query", C.c_int, [C.c_void_p, C.c_void_p]),

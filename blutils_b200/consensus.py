@@ -390,6 +390,41 @@ class ConsensusEngine:
             pass
 
 
+def _run_configs(engines: Sequence[ConsensusEngine], call, keep=None) -> List[ConsensusOutput]:
+    n = len(engines)
+    ctxs = (C.c_void_p * max(n, 1))(*[e._h for e in engines])
+    outs = (C.c_void_p * max(n, 1))()
+    rc = call(ctxs, n, outs)
+    if rc != 0:
+        _raise(rc, (_ffi.lib().blu_last_error(engines[0]._h if n else None) or b"").decode())
+    res = [ConsensusOutput(e, outs[k]) for k, e in enumerate(engines)]
+    for r in res:
+        r._keep = keep
+    return res
+
+
+def run_host_configs(engines: Sequence[ConsensusEngine], text: Union[bytes, int], nbytes: Optional[int] = None) -> List[ConsensusOutput]:
+    """One pass over a hit table in host memory for several configurations (blu_consensus_run_host_configs): the text is
+    parsed and copied to the GPU once; result k is what engines[k].run_host(text) returns and belongs to engines[k]."""
+    if isinstance(text, (bytes, bytearray)):
+        buf = C.create_string_buffer(bytes(text), len(text)) if len(text) else C.create_string_buffer(1)
+        return _run_configs(engines, lambda c, n, o: _ffi.lib().blu_consensus_run_host_configs(c, n, C.addressof(buf), len(text), o), buf)
+    return _run_configs(engines, lambda c, n, o: _ffi.lib().blu_consensus_run_host_configs(c, n, int(text), int(nbytes), o))
+
+
+def run_file_configs(engines: Sequence[ConsensusEngine], blast_out: str) -> List[ConsensusOutput]:
+    """One pass over a hit table file for several configurations (blu_consensus_run_file_configs): the file is read once."""
+    path = os.fspath(blast_out).encode()
+    return _run_configs(engines, lambda c, n, o: _ffi.lib().blu_consensus_run_file_configs(c, n, path, o))
+
+
+def run_device_resident_configs(engines: Sequence[ConsensusEngine], dptr: int, nbytes: int, stream: int = 0) -> List[ConsensusOutput]:
+    """One pass over a hit table in HBM for several configurations (blu_consensus_run_device_resident_configs): the results
+    stay on the device; `.download()` each of them."""
+    return _run_configs(engines, lambda c, n, o: _ffi.lib().blu_consensus_run_device_resident_configs(c, n, int(dptr), int(nbytes),
+                                                                                                        int(stream) or None, o))
+
+
 def shard_cuts(text: Union[bytes, int], n_shards: int, nbytes: Optional[int] = None) -> List[int]:
     """Byte offsets that split a (contiguous) hit table into n_shards query-aligned ranges (SURVEY 8e).  Host-only."""
     cuts = (C.c_uint64 * (n_shards + 1))()

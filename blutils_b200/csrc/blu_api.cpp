@@ -426,14 +426,16 @@ inline size_t dup_table_size(const Caps& k) {
     return cap;
 }
 
-void ensure_out(blu_ctx* c, const Caps& k) {
+// `first`: the context also holds what the configurations of a pass share (see Cfg).
+void ensure_out(blu_ctx* c, const Caps& k, bool first) {
     if (!c->out) c->out = c->dev_pool->acquire();
     c->out->rec.ensure(k.rec);
     c->out->beans.ensure(k.beans);
     c->out->accs.ensure(k.accs);
+    if (k.pool) c->d_pool.ensure(k.pool);
+    if (!first) return;
     c->d_top.ensure(k.slots);
     c->d_defer.ensure(k.defer);
-    if (k.pool) c->d_pool.ensure(k.pool);
     c->d_dup.ensure(dup_table_size(k));
     if (c->keep_hashes) c->d_qhash.ensure(k.rec);
     c->d_big_rows.ensure((size_t)c->sms * kLongTopCap);
@@ -444,8 +446,9 @@ std::string dev_err_message(uint32_t code, uint64_t off) {
     return std::string(dev_err_text(code)) + " (near byte " + std::to_string(off) + " of the blast output)";
 }
 
-[[noreturn]] void throw_device_error(uint32_t code, uint64_t off) {
-    const std::string m = dev_err_message(code, off);
+// `where`: prefix of the message (which configuration of a group failed)
+[[noreturn]] void throw_device_error(uint32_t code, uint64_t off, const std::string& where = "") {
+    const std::string m = where + dev_err_message(code, off);
     if (code >= DE_INTERNAL) throw std::runtime_error(m);
     if (code >= DE_NUM_UNSUPPORTED) throw UnsupportedErr(m);
     throw DataErr(m);
@@ -466,6 +469,39 @@ struct RunStatus {
         if (h.soft_code && !soft_code) soft_code = h.soft_code, soft_off = stream_base + h.soft_off;
     }
 };
+
+// One configuration of a pass over a table: the context whose lineage tables, strategy, output arrays, counters and densities
+// its kernels use, the result part it fills, and its capacities, status and last counter snapshot.  A pass has one
+// configuration, or several (blu_consensus_run_*_configs) that share what depends on the text only: the tile kernel runs
+// once, and the first configuration's context holds the streams, events, text buffers, top-row slots, deferred runs and
+// duplicate-id table of the pass.
+struct Cfg {
+    blu_ctx* c;
+    ResultPartOwned* r;
+    Caps k{};
+    RunStatus st{};
+    Counters h{};
+};
+using Pass = std::vector<Cfg>;
+
+// Records, top-row slots and deferred runs depend on the text only: every configuration of a pass gets the largest capacity
+// any of them asks for (the fan-out kernel keeps record indices).  Beans, accession references and the pool are its own.
+void share_caps(Pass& g) {
+    Caps& k0 = g[0].k;
+    for (const Cfg& x : g) k0.rec = std::max(k0.rec, x.k.rec), k0.slots = std::max(k0.slots, x.k.slots), k0.defer = std::max(k0.defer, x.k.defer);
+    for (Cfg& x : g) x.k.rec = k0.rec, x.k.slots = k0.slots, x.k.defer = k0.defer;
+}
+
+void reset_timings(Pass& g) {
+    for (Cfg& x : g) x.c->tm = blu_timings{};
+}
+
+// A context of this pass has not seen a table like it yet (see probe_densities).
+bool unseen(const Pass& g) {
+    for (const Cfg& x : g)
+        if (x.c->dens_rec == 0) return true;
+    return false;
+}
 
 // BLU_SYNC_DEBUG=1: synchronise behind every kernel so that a device fault is attributed to the kernel that caused it
 inline void dbg_sync(cudaStream_t s, const char* what) {
@@ -497,89 +533,125 @@ enum class Strings {
 // One range / chunk, all of it queued without a host round trip: tile kernel, long-run kernel (returns at once when
 // nothing was deferred), consensus, (gather,) duplicate-id check, and the one-thread kernel that advances the device-side
 // cursors and snapshots the counters into mapped host memory.  `begin` may be kBeginFromCounters.
-void launch_range(blu_ctx* c, const uint8_t* dtext, uint64_t begin, uint64_t end, bool final_chunk, const Caps& k, cudaStream_t s, int slot,
-                  Strings strings, long long delta) {
-    RunParams p{};
-    p.text = dtext;
-    p.begin = begin;
-    p.end = end;
-    p.final_chunk = final_chunk ? 1 : 0;
-    p.strategy = c->opts.strategy;
-    p.T = c->dT;
-    p.records = c->out->rec.p;
-    p.rec_cap = k.rec;
-    p.toprows = c->d_top.p;
-    p.slot_cap = k.slots;
-    p.beans = c->out->beans.p;
-    p.bean_cap = k.beans;
-    p.accs = c->out->accs.p;
-    p.acc_cap = k.accs;
-    p.defer = c->d_defer.p;
-    p.defer_cap = (uint32_t)std::min<size_t>(k.defer, 0xFFFFFFFFu);
-    p.big_rows = c->d_big_rows.p;
-    p.big_cand = c->d_big_cand.p;
-    p.ctr = c->d_ctr;
-    cudaEvent_t* ev = c->ev[slot];
+// A pass with several configurations runs the tile kernel once, into the first one's records and counters, and the fan-out
+// kernel copies what it found to the others; the long-run, consensus and gather kernels and the advance run per
+// configuration, the duplicate-id check once (the others only relocate their references into the caller's text).
+void launch_range(const Pass& g, const uint8_t* dtext, uint64_t begin, uint64_t end, bool final_chunk, cudaStream_t s, int slot, Strings strings,
+                  long long delta) {
+    blu_ctx* c0 = g[0].c;
+    const Caps& k0 = g[0].k;
+    uint64_t launches = 0;
+    auto run_params = [&](const Cfg& x) {
+        RunParams p{};
+        p.text = dtext;
+        p.begin = begin;
+        p.end = end;
+        p.final_chunk = final_chunk ? 1 : 0;
+        p.strategy = x.c->opts.strategy;
+        p.T = x.c->dT;
+        p.records = x.c->out->rec.p;
+        p.rec_cap = x.k.rec;
+        p.toprows = c0->d_top.p;
+        p.slot_cap = k0.slots;
+        p.beans = x.c->out->beans.p;
+        p.bean_cap = x.k.beans;
+        p.accs = x.c->out->accs.p;
+        p.acc_cap = x.k.accs;
+        p.defer = c0->d_defer.p;
+        p.defer_cap = (uint32_t)std::min<size_t>(k0.defer, 0xFFFFFFFFu);
+        p.big_rows = c0->d_big_rows.p;
+        p.big_cand = c0->d_big_cand.p;
+        p.ctr = x.c->d_ctr;
+        return p;
+    };
+    cudaEvent_t* ev = c0->ev[slot];
     CK(cudaEventRecord(ev[0], s));
-    CK(launch_tile_kernel(p, tile_kernel_grid(c->device), s));
+    CK(launch_tile_kernel(run_params(g[0]), tile_kernel_grid(c0->device), s));
     dbg_sync(s, "tile_kernel");
+    launches++;
     CK(cudaEventRecord(ev[1], s));
-    CK(launch_longrun_kernel(p, c->sms, s));
-    dbg_sync(s, "longrun_kernel");
-    CK(cudaEventRecord(ev[2], s));
-    PostParams q{};
-    q.records = c->out->rec.p;
-    q.rec_cap = k.rec;
-    q.toprows = c->d_top.p;
-    q.slot_cap = k.slots;
-    q.beans = c->out->beans.p;
-    q.bean_cap = k.beans;
-    q.accs = c->out->accs.p;
-    q.acc_cap = k.accs;
-    q.text = dtext;
-    q.text_end = end;
-    q.pool = strings == Strings::Pool ? c->d_pool.p : nullptr;
-    q.pool_cap = strings == Strings::Pool ? k.pool : 0;
-    q.T = c->dT;
-    q.strategy = c->opts.strategy;
-    q.ctr = c->d_ctr;
-    CK(launch_consensus_kernel(q, c->sms, s));
-    dbg_sync(s, "consensus_kernel");
-    if (strings == Strings::Pool) {
-        CK(launch_gather_kernel(q, c->sms, s));
-        dbg_sync(s, "gather_kernel");
-        c->tm.n_kernel_launches += 1;
+    if (g.size() > 1) {
+        FanoutParams f{};
+        f.src = c0->d_ctr;
+        f.src_records = c0->out->rec.p;
+        f.n_dst = (int)g.size() - 1;
+        f.rec_cap = k0.rec;
+        for (size_t i = 1; i < g.size(); i++) f.dst[i - 1] = g[i].c->d_ctr, f.dst_records[i - 1] = g[i].c->out->rec.p;
+        CK(launch_fanout_kernel(f, c0->sms, s));
+        dbg_sync(s, "fanout_kernel");
+        launches++;
     }
-    DupParams d{};
-    d.records = c->out->rec.p;
-    d.rec_cap = k.rec;
-    d.beans = c->out->beans.p;
-    d.accs = c->out->accs.p;
-    d.strings = strings == Strings::Pool ? c->d_pool.p : dtext;
-    d.strings_len = strings == Strings::Pool ? k.pool : end;
-    d.table = c->d_dup.p;
-    d.mask = (uint32_t)(dup_table_size(k) - 1);
-    d.hashes = c->d_qhash.cap >= k.rec ? c->d_qhash.p : nullptr;
-    d.ref_delta = strings == Strings::HostText ? delta : 0;
-    d.ctr = c->d_ctr;
-    CK(launch_dup_kernel(d, c->sms, s));
-    dbg_sync(s, "dup_kernel");
-    AdvanceParams a{};
-    a.ctr = c->d_ctr;
-    a.rec_cap = k.rec;
-    a.range_end = end;
-    a.snapshot = c->d_snap + slot;
-    CK(launch_advance_kernel(a, s));
-    dbg_sync(s, "advance_kernel");
+    for (const Cfg& x : g) {
+        CK(launch_longrun_kernel(run_params(x), c0->sms, s));
+        dbg_sync(s, "longrun_kernel");
+        launches++;
+    }
+    CK(cudaEventRecord(ev[2], s));
+    for (const Cfg& x : g) {
+        PostParams q{};
+        q.records = x.c->out->rec.p;
+        q.rec_cap = x.k.rec;
+        q.toprows = c0->d_top.p;
+        q.slot_cap = k0.slots;
+        q.beans = x.c->out->beans.p;
+        q.bean_cap = x.k.beans;
+        q.accs = x.c->out->accs.p;
+        q.acc_cap = x.k.accs;
+        q.text = dtext;
+        q.text_end = end;
+        q.pool = strings == Strings::Pool ? x.c->d_pool.p : nullptr;
+        q.pool_cap = strings == Strings::Pool ? x.k.pool : 0;
+        q.T = x.c->dT;
+        q.strategy = x.c->opts.strategy;
+        q.ctr = x.c->d_ctr;
+        CK(launch_consensus_kernel(q, c0->sms, s));
+        dbg_sync(s, "consensus_kernel");
+        launches++;
+        if (strings == Strings::Pool) {
+            CK(launch_gather_kernel(q, c0->sms, s));
+            dbg_sync(s, "gather_kernel");
+            launches++;
+        }
+    }
+    for (size_t i = 0; i < g.size() && (i == 0 || strings == Strings::HostText); i++) {
+        const Cfg& x = g[i];
+        DupParams d{};
+        d.records = x.c->out->rec.p;
+        d.rec_cap = x.k.rec;
+        d.beans = x.c->out->beans.p;
+        d.accs = x.c->out->accs.p;
+        d.strings = strings == Strings::Pool ? x.c->d_pool.p : dtext;
+        d.strings_len = strings == Strings::Pool ? x.k.pool : end;
+        d.table = i == 0 ? c0->d_dup.p : nullptr;
+        d.mask = i == 0 ? (uint32_t)(dup_table_size(k0) - 1) : 0;
+        d.hashes = i == 0 && c0->d_qhash.cap >= k0.rec ? c0->d_qhash.p : nullptr;
+        d.ref_delta = strings == Strings::HostText ? delta : 0;
+        d.ctr = x.c->d_ctr;
+        CK(launch_dup_kernel(d, c0->sms, s));
+        dbg_sync(s, "dup_kernel");
+        launches++;
+    }
+    for (const Cfg& x : g) {
+        AdvanceParams a{};
+        a.ctr = x.c->d_ctr;
+        a.rec_cap = x.k.rec;
+        a.range_end = end;
+        a.snapshot = x.c->d_snap + slot;
+        CK(launch_advance_kernel(a, s));
+        dbg_sync(s, "advance_kernel");
+        launches++;
+    }
     CK(cudaEventRecord(ev[3], s));
-    c->tm.n_kernel_launches += 5;
+    c0->tm.n_kernel_launches += launches;
 }
 
 // Start of a run: output arrays, counters, the duplicate-id table.
-void begin_run(blu_ctx* c, const Caps& k, cudaStream_t s) {
-    ensure_out(c, k);
-    reset_counters_async(c, s);
-    CK(cudaMemsetAsync(c->d_dup.p, 0, dup_table_size(k) * sizeof(unsigned long long), s));
+void begin_run(const Pass& g, cudaStream_t s) {
+    for (size_t i = 0; i < g.size(); i++) {
+        ensure_out(g[i].c, g[i].k, i == 0);
+        reset_counters_async(g[i].c, s);
+    }
+    CK(cudaMemsetAsync(g[0].c->d_dup.p, 0, dup_table_size(g[0].k) * sizeof(unsigned long long), s));
 }
 
 inline bool overflowed(const Counters& h, const Caps& k) {
@@ -627,40 +699,47 @@ struct KernelMs {
     double tile = 0, longrun = 0, post = 0;
 };
 
-// Reads the counter snapshot of range / chunk `slot` once its kernels have completed: its kernel times and deferred runs
-// are added up, a grammar error is raised (at `base` + err_off) before anything is done about a capacity -- a malformed
-// row is an error whatever else happened -- and on a capacity overflow the capacities are grown for the whole input of
-// `n` bytes (`scale`: see grow_caps).  true: the run has to start over.
-bool read_snapshot(blu_ctx* c, int slot, uint64_t base, Caps& k, double scale, uint64_t n, Counters& h, KernelMs& ms) {
-    const cudaEvent_t* ev = c->ev[slot];
+// Reads the counter snapshots of range / chunk `slot` (into Cfg::h) once its kernels have completed: its kernel times and
+// deferred runs are added up, a grammar error is raised (at `base` + err_off) before anything is done about a capacity -- a
+// malformed row is an error whatever else happened -- and on a capacity overflow of any configuration its capacities are
+// grown for the whole input of `n` bytes (`scale`: see grow_caps).  true: the pass has to start over.
+bool read_snapshot(Pass& g, int slot, uint64_t base, double scale, uint64_t n, KernelMs& ms) {
+    blu_ctx* c0 = g[0].c;
+    const cudaEvent_t* ev = c0->ev[slot];
     CK(cudaEventSynchronize(ev[3]));
-    h = c->h_snap[slot];
+    for (Cfg& x : g) x.h = x.c->h_snap[slot];
     ms.tile += ev_ms(ev[0], ev[1]);
     ms.longrun += ev_ms(ev[1], ev[2]);
     ms.post += ev_ms(ev[2], ev[3]);
-    c->tm.n_deferred_runs += h.n_defer;
-    check_fatal(h, base);
-    if (!overflowed(h, k)) return false;
-    grow_caps(h, k, scale, n);
-    return true;
+    c0->tm.n_deferred_runs += g[0].h.n_defer;
+    for (const Cfg& x : g) check_fatal(x.h, base);
+    bool grew = false;
+    for (Cfg& x : g)
+        if (overflowed(x.h, x.k)) grow_caps(x.h, x.k, scale, n), grew = true;
+    if (grew) share_caps(g);
+    return grew;
 }
 
-// The end of a run that found no duplicate id (`h`: its last snapshot): the timings every loop reports the same way, and
-// the densities that size the next run.
-void finish_run(blu_ctx* c, const Counters& h, uint64_t n, uint64_t tiles, const KernelMs& ms) {
-    if (h.post_done == 0) throw DataErr("the blast output holds no rows");
-    c->tm.ms_tile_kernel = ms.tile;
-    c->tm.ms_longrun_kernel = ms.longrun;
-    c->tm.ms_gather_kernel = ms.post;
-    c->tm.ms_total_device = ms.tile + ms.longrun + ms.post;
-    c->tm.text_bytes = n;
-    c->tm.taxonomy_bytes = c->tax->device_bytes();
-    c->tm.n_tile_launches = tiles;
-    c->tm.n_queries = h.post_done;
-    c->tm.n_rows = h.n_rows;
-    c->tm.result_bytes = h.post_done * sizeof(blu_record) + h.bean_used * sizeof(blu_bean) + h.acc_used * sizeof(blu_acc);
-    c->tm.d2h_bytes += sizeof(Counters);
-    learn_densities(c, h, n);
+// The end of a pass that found no duplicate id (Cfg::h: the last snapshots): the timings every loop reports the same way,
+// and the densities that size the next run.
+void finish_run(Pass& g, uint64_t n, uint64_t tiles, const KernelMs& ms) {
+    if (g[0].h.post_done == 0) throw DataErr("the blast output holds no rows");
+    for (const Cfg& x : g) {
+        blu_ctx* c = x.c;
+        const Counters& h = x.h;
+        c->tm.ms_tile_kernel = ms.tile;
+        c->tm.ms_longrun_kernel = ms.longrun;
+        c->tm.ms_gather_kernel = ms.post;
+        c->tm.ms_total_device = ms.tile + ms.longrun + ms.post;
+        c->tm.text_bytes = n;
+        c->tm.taxonomy_bytes = c->tax->device_bytes();
+        c->tm.n_tile_launches = tiles;
+        c->tm.n_queries = h.post_done;
+        c->tm.n_rows = h.n_rows;
+        c->tm.result_bytes = h.post_done * sizeof(blu_record) + h.bean_used * sizeof(blu_bean) + h.acc_used * sizeof(blu_acc);
+        c->tm.d2h_bytes += sizeof(Counters);
+        learn_densities(c, h, n);
+    }
 }
 
 // Synchronises the first `n` of `s` when its scope is left by an exception: nothing may still read the caller's text, or a
@@ -675,15 +754,17 @@ struct SyncOnUnwind {
     }
 };
 
-// Incremental download of the finished part of the result arrays on the context's download stream, so that the
-// device->host copies of one range / chunk run under the kernels (and host->device copies) of the next one.
+// Incremental download of the finished part of the result arrays on the pass's download stream (that of its first
+// context), so that the device->host copies of one range / chunk run under the kernels (and host->device copies) of the
+// next one.
 struct Downloader {
     blu_ctx* c;
     ResultPartOwned* r;
+    cudaStream_t ds;
     uint64_t rec_done = 0, bean_done = 0, acc_done = 0, pool_done = 0;
     uint64_t bytes = 0;
 
-    Downloader(blu_ctx* ctx, ResultPartOwned* res) : c(ctx), r(res) { r->pinned = c->pool; }
+    Downloader(blu_ctx* ctx, ResultPartOwned* res, cudaStream_t stream) : c(ctx), r(res), ds(stream) { r->pinned = c->pool; }
 
     static void grow(blu_ctx* c, PinnedBuf& b, size_t need, size_t keep, cudaStream_t ds) {
         if (b.cap >= need && b.p) return;
@@ -697,7 +778,6 @@ struct Downloader {
     }
     // capacity for at least these totals (called with estimates first, exact numbers at the end)
     void reserve(uint64_t rec, uint64_t beans, uint64_t accs, uint64_t pool) {
-        cudaStream_t ds = c->d2h_stream;
         grow(c, r->b_rec, rec * sizeof(blu_record), rec_done * sizeof(blu_record), ds);
         grow(c, r->b_beans, beans * sizeof(blu_bean), bean_done * sizeof(blu_bean), ds);
         grow(c, r->b_accs, accs * sizeof(blu_acc), acc_done * sizeof(blu_acc), ds);
@@ -705,7 +785,6 @@ struct Downloader {
     }
     // everything below the cursors of snapshot `h` is final on the device (its post-pass has completed)
     void push(const Counters& h) {
-        cudaStream_t ds = c->d2h_stream;
         const uint64_t rec = h.post_done, beans = h.bean_used, accs = h.acc_used, pool = h.pool_used;
         reserve(rec, beans, accs, pool);
         if (rec > rec_done)
@@ -720,13 +799,13 @@ struct Downloader {
     }
     void finish(const Counters& h) {
         push(h);
-        CK(cudaStreamSynchronize(c->d2h_stream));
+        CK(cudaStreamSynchronize(ds));
         r->n_rec = rec_done, r->n_beans = bean_done, r->n_accs = acc_done, r->pool_len = pool_done;
         r->on_host = true;
         c->tm.d2h_bytes += bytes;
     }
     void abandon() {  // retry with larger device capacities: drop what was downloaded
-        cudaStreamSynchronize(c->d2h_stream);
+        cudaStreamSynchronize(ds);
         rec_done = bean_done = acc_done = pool_done = 0;
         bytes = 0;
     }
@@ -739,31 +818,30 @@ void require_tax(blu_ctx* c) {
 // Output densities of a table this context has not seen the like of: the kernels run once over a small prefix (results
 // discarded), so that the arrays of the real run are sized for what the table holds instead of for the shortest rows the
 // grammar allows (1.5 GB of records for a 3.8 GB table; more than a B200 has for a 77 GB one).
-void probe_densities(blu_ctx* c, const uint8_t* dtext, uint64_t begin, uint64_t end, cudaStream_t s) {
+// A pass with several configurations probes once, for every context that has not seen such a table.
+void probe_densities(Pass& g, const uint8_t* dtext, uint64_t begin, uint64_t end, cudaStream_t s) {
     const uint64_t len = end - begin;
     if (len < (1u << 20)) return;
-    const blu_timings keep = c->tm;
-    Caps k = initial_caps(c, len, false);
-    begin_run(c, k, s);
-    launch_range(c, dtext, begin, end, false, k, s, 0, Strings::DeviceText, 0);
-    CK(cudaEventSynchronize(c->ev[0][3]));
-    const Counters h = c->h_snap[0];
-    c->tm = keep;
-    if (overflowed(h, k) || h.err_code || h.post_done < 64) return;  // (the real run reports whatever is wrong)
-    const uint64_t covered = h.next_begin > begin && h.next_begin <= end ? h.next_begin - begin : len;
-    learn_densities(c, h, covered);
-    c->dens_pool = c->dens_rec * 48.0 + c->dens_acc * 24.0;  // (ids + accessions; an underestimate is grown by the retry)
+    const blu_timings keep = g[0].c->tm;
+    for (Cfg& x : g) x.k = initial_caps(x.c, len, false);
+    share_caps(g);
+    begin_run(g, s);
+    launch_range(g, dtext, begin, end, false, s, 0, Strings::DeviceText, 0);
+    CK(cudaEventSynchronize(g[0].c->ev[0][3]));
+    g[0].c->tm = keep;
+    for (const Cfg& x : g) {
+        blu_ctx* c = x.c;
+        const Counters h = c->h_snap[0];
+        if (c->dens_rec != 0 || overflowed(h, x.k) || h.err_code || h.post_done < 64) continue;  // (the real run reports whatever is wrong)
+        const uint64_t covered = h.next_begin > begin && h.next_begin <= end ? h.next_begin - begin : len;
+        learn_densities(c, h, covered);
+        c->dens_pool = c->dens_rec * 48.0 + c->dens_acc * 24.0;  // (ids + accessions; an underestimate is grown by the retry)
+    }
 }
 
 struct NonContiguous : std::runtime_error {
     using std::runtime_error::runtime_error;
 };
-
-// What a single-device entry point does with the status of its run.
-void settle(const RunStatus& st) {
-    if (st.dup_found) throw NonContiguous("a query id occurs in two non-adjacent groups of rows");
-    if (st.soft_code) throw_device_error(st.soft_code, st.soft_off);
-}
 
 std::vector<uint64_t> resident_ranges(uint64_t n) {
     // Large resident tables are processed in a few query-aligned ranges so that the download of one range's records
@@ -805,62 +883,74 @@ void check_device_text(const uint8_t* dtext, uint64_t n) {
 // stopped (Counters.next_begin), the post-pass takes its record range from the device counters -- so the GPU never waits
 // for the host; the host trails behind, reads each range's snapshot when its event fires and queues that range's download
 // on the download stream.
-void run_device_text(blu_ctx* c, const uint8_t* dtext, uint64_t n, cudaStream_t s, ResultPartOwned* r, RunStatus& st, bool resident) {
-    SyncOnUnwind unwind{{s, c->d2h_stream}, resident ? 1 : 2};
-    require_tax(c);
+void run_device_text(Pass& g, const uint8_t* dtext, uint64_t n, cudaStream_t s, bool resident) {
+    blu_ctx* c0 = g[0].c;
+    SyncOnUnwind unwind{{s, c0->d2h_stream}, resident ? 1 : 2};
+    for (const Cfg& x : g) require_tax(x.c);
     check_device_text(dtext, n);
-    c->tm = blu_timings{};
-    if (c->dens_rec == 0 && n > (64ull << 20)) probe_densities(c, dtext, 0, std::min<uint64_t>(n, 32ull << 20), s);
-    Caps k = initial_caps(c, n, !resident);
+    reset_timings(g);
+    if (unseen(g) && n > (64ull << 20)) probe_densities(g, dtext, 0, std::min<uint64_t>(n, 32ull << 20), s);
+    for (Cfg& x : g) x.k = initial_caps(x.c, n, !resident);
+    share_caps(g);
     const std::vector<uint64_t> range_end = resident ? std::vector<uint64_t>{n} : resident_ranges(n);
     const int n_ranges = (int)range_end.size();
     const Strings strings = resident ? Strings::DeviceText : Strings::Pool;
-    Downloader dl(c, r);
+    std::vector<Downloader> dl;
+    for (const Cfg& x : g) dl.emplace_back(x.c, x.r, c0->d2h_stream);
     for (int attempt = 0; attempt < 8; attempt++) {
-        begin_run(c, k, s);
+        begin_run(g, s);
         for (int ri = 0; ri < n_ranges; ri++)
-            launch_range(c, dtext, ri == 0 ? 0 : kBeginFromCounters, range_end[ri], ri + 1 == n_ranges, k, s, ri, strings, 0);
+            launch_range(g, dtext, ri == 0 ? 0 : kBeginFromCounters, range_end[ri], ri + 1 == n_ranges, s, ri, strings, 0);
         bool retry = false;
-        Counters h{};
         KernelMs ms;
         for (int ri = 0; ri < n_ranges && !retry; ri++) {
-            retry = read_snapshot(c, ri, 0, k, (double)n / (double)std::max<uint64_t>(range_end[ri], 1), n, h, ms);
-            if (!retry && ri + 1 < n_ranges && !h.dup_found) {
-                if (ri == 0 && range_end[0] > 0) {
-                    // size the pinned result buffers from the density of the first range
-                    const double f = 1.15 * (double)n / (double)range_end[0];
-                    dl.reserve((uint64_t)(h.post_done * f) + 4096, (uint64_t)(h.bean_used * f) + 8192, (uint64_t)(h.acc_used * f) + 8192,
-                               (uint64_t)(h.pool_used * f) + 65536);
+            retry = read_snapshot(g, ri, 0, (double)n / (double)std::max<uint64_t>(range_end[ri], 1), n, ms);
+            if (!retry && ri + 1 < n_ranges && !g[0].h.dup_found)
+                for (size_t i = 0; i < g.size(); i++) {
+                    const Counters& h = g[i].h;
+                    if (ri == 0 && range_end[0] > 0) {
+                        // size the pinned result buffers from the density of the first range
+                        const double f = 1.15 * (double)n / (double)range_end[0];
+                        dl[i].reserve((uint64_t)(h.post_done * f) + 4096, (uint64_t)(h.bean_used * f) + 8192, (uint64_t)(h.acc_used * f) + 8192,
+                                      (uint64_t)(h.pool_used * f) + 65536);
+                    }
+                    dl[i].push(h);  // runs on the download stream under the next ranges' kernels
                 }
-                dl.push(h);  // runs on the download stream under the next ranges' kernels
-            }
         }
         if (retry) {
             if (!resident) {
                 CK(cudaStreamSynchronize(s));  // the later ranges are still queued
-                dl.abandon();
+                for (Downloader& d : dl) d.abandon();
             }
-            c->tm = blu_timings{};
+            reset_timings(g);
             continue;
         }
-        st.note_soft(h, 0);
-        st.dup_found = h.dup_found != 0;
-        if (st.dup_found) {
-            if (!resident) dl.abandon();
+        for (Cfg& x : g) {
+            x.st.note_soft(x.h, 0);
+            x.st.dup_found = g[0].h.dup_found != 0;
+        }
+        if (g[0].st.dup_found) {
+            if (!resident)
+                for (Downloader& d : dl) d.abandon();
             return;
         }
-        finish_run(c, h, n, (uint64_t)n_ranges, ms);
-        if (!resident) {
-            dl.finish(h);
-            return;
+        finish_run(g, n, (uint64_t)n_ranges, ms);
+        for (size_t i = 0; i < g.size(); i++) {
+            const Counters& h = g[i].h;
+            if (!resident) {
+                dl[i].finish(h);
+                continue;
+            }
+            blu_ctx* c = g[i].c;
+            ResultPartOwned* r = g[i].r;
+            r->dev = std::move(c->out);
+            r->dev_pool = c->dev_pool;
+            r->ctx = c;
+            r->dtext = dtext;
+            r->dtext_len = n;
+            r->n_rec = h.post_done, r->n_beans = h.bean_used, r->n_accs = h.acc_used;
+            r->on_host = false;
         }
-        r->dev = std::move(c->out);
-        r->dev_pool = c->dev_pool;
-        r->ctx = c;
-        r->dtext = dtext;
-        r->dtext_len = n;
-        r->n_rec = h.post_done, r->n_beans = h.bean_used, r->n_accs = h.acc_used;
-        r->on_host = false;
         return;
     }
     throw std::runtime_error("output capacity did not converge");
@@ -1148,11 +1238,13 @@ class FileSource : public ChunkSource {
 inline uint64_t chunk_bytes_of(const blu_ctx* c, uint64_t dflt) { return c->opts.chunk_bytes ? ((c->opts.chunk_bytes + 127) & ~127ull) : dflt; }
 
 // `host_text` != nullptr: BLU_OPT_TEXT_REFS -- the result's strings stay references into that (caller-owned) text.
-void run_host_chunks(blu_ctx* c, ChunkSource& src, uint64_t n, const uint64_t chunk, ResultPartOwned* r, RunStatus& st, const char* host_text) {
+// Several configurations share the chunks: each crosses PCIe once, into the first context's buffers.
+void run_host_chunks(Pass& g, ChunkSource& src, uint64_t n, const uint64_t chunk, const char* host_text) {
+    blu_ctx* c = g[0].c;
     SyncOnUnwind unwind{{c->copy_stream, c->stream, c->d2h_stream}, 3};  // (and nothing may still copy from a staging buffer)
-    require_tax(c);
+    for (const Cfg& x : g) require_tax(x.c);
     if (n == 0) throw DataErr("empty blast output (the reference's CsvReader fails on an empty file)");
-    c->tm = blu_timings{};
+    reset_timings(g);
     const uint64_t carry = c->carry_bytes;
     const uint64_t n_chunks = (n + chunk - 1) / chunk;
     const bool single = n_chunks == 1;
@@ -1162,15 +1254,14 @@ void run_host_chunks(blu_ctx* c, ChunkSource& src, uint64_t n, const uint64_t ch
     if (!single) c->d_text[1].ensure(buf_bytes);
     const Strings strings = host_text ? Strings::HostText : Strings::Pool;
     cudaStream_t s = c->stream, cs = c->copy_stream;
-    Downloader dl(c, r);
+    std::vector<Downloader> dl;
+    for (const Cfg& x : g) dl.emplace_back(x.c, x.r, c->d2h_stream);
     auto t0 = std::chrono::steady_clock::now();
-    Caps k{};
     bool have_caps = false;
     for (int attempt = 0; attempt < 8; attempt++) {
         bool retry = false;
         uint64_t tail_len = 0;  // bytes carried from the previous chunk
         KernelMs ms;
-        Counters h{};
         auto issue_h2d = [&](uint64_t ci) {
             const uint64_t off = ci * chunk, len = std::min(chunk, n - off);
             CK(cudaMemcpyAsync(c->d_text[ci & 1].p + text_off, src.acquire(ci), len, cudaMemcpyHostToDevice, cs));
@@ -1180,14 +1271,15 @@ void run_host_chunks(blu_ctx* c, ChunkSource& src, uint64_t n, const uint64_t ch
         issue_h2d(0);
         if (!have_caps) {
             // a table this context has not seen the like of: the first chunk's first megabytes tell how dense its output is
-            if (c->dens_rec == 0 && n > (64ull << 20)) {
+            if (unseen(g) && n > (64ull << 20)) {
                 CK(cudaStreamWaitEvent(s, c->ev_h2d[0], 0));
-                probe_densities(c, c->d_text[0].p, text_off, text_off + std::min<uint64_t>(std::min(chunk, n), 32ull << 20), s);
+                probe_densities(g, c->d_text[0].p, text_off, text_off + std::min<uint64_t>(std::min(chunk, n), 32ull << 20), s);
             }
-            k = initial_caps(c, n, strings == Strings::Pool);
+            for (Cfg& x : g) x.k = initial_caps(x.c, n, strings == Strings::Pool);
+            share_caps(g);
             have_caps = true;
         }
-        begin_run(c, k, s);
+        begin_run(g, s);
         for (uint64_t ci = 0; ci < n_chunks; ci++) {
             const uint64_t off = ci * chunk, len = std::min(chunk, n - off);
             const bool final_chunk = ci + 1 == n_chunks;
@@ -1203,45 +1295,49 @@ void run_host_chunks(blu_ctx* c, ChunkSource& src, uint64_t n, const uint64_t ch
             CK(cudaEventRecord(c->ev_free[(ci + 1) & 1], s));  // previous buffer no longer read after this point
             const uint64_t begin = text_off - tail_len, end = text_off + len;
             // buffer offset d of this chunk is byte off + d - text_off of the caller's text
-            launch_range(c, buf, begin, end, final_chunk, k, s, slot, strings, (long long)off - (long long)text_off);
+            launch_range(g, buf, begin, end, final_chunk, s, slot, strings, (long long)off - (long long)text_off);
             if (!final_chunk) {  // behind the launches: a file source may block here until the next chunk has been read
                 CK(cudaStreamWaitEvent(cs, c->ev_free[(ci + 1) & 1], 0));
                 issue_h2d(ci + 1);
             }
-            retry = read_snapshot(c, slot, off - text_off, k, (double)n / (double)(off + len), n, h, ms);  // err_off is in buffer coordinates
+            retry = read_snapshot(g, slot, off - text_off, (double)n / (double)(off + len), n, ms);  // err_off is in buffer coordinates
             src.release(ci);  // `s` waited for this chunk's copy, so it has completed
             if (retry) break;
-            st.note_soft(h, off - text_off);
+            for (Cfg& x : g) x.st.note_soft(x.h, off - text_off);
             if (!final_chunk) {
-                tail_len = end - h.next_begin;  // (next_begin == end: nothing is carried)
+                tail_len = end - g[0].h.next_begin;  // (next_begin == end: nothing is carried)
                 if (tail_len > carry) throw UnsupportedErr("a single query spans more than the 64 MiB carry buffer between streamed chunks");
-                if (!h.dup_found) {
-                    if (ci == 0) {
-                        const double f = 1.15 * (double)n / (double)len;
-                        dl.reserve((uint64_t)(h.post_done * f) + 4096, (uint64_t)(h.bean_used * f) + 8192, (uint64_t)(h.acc_used * f) + 8192,
-                                   strings == Strings::Pool ? (uint64_t)(h.pool_used * f) + 65536 : 0);
+                if (!g[0].h.dup_found)
+                    for (size_t i = 0; i < g.size(); i++) {
+                        const Counters& h = g[i].h;
+                        if (ci == 0) {
+                            const double f = 1.15 * (double)n / (double)len;
+                            dl[i].reserve((uint64_t)(h.post_done * f) + 4096, (uint64_t)(h.bean_used * f) + 8192, (uint64_t)(h.acc_used * f) + 8192,
+                                          strings == Strings::Pool ? (uint64_t)(h.pool_used * f) + 65536 : 0);
+                        }
+                        dl[i].push(h);  // result download of this chunk runs beside the next chunks' host->device copies
                     }
-                    dl.push(h);  // result download of this chunk runs beside the next chunks' host->device copies
-                }
             }
         }
         if (retry) {
             CK(cudaStreamSynchronize(cs));
             CK(cudaStreamSynchronize(s));
-            dl.abandon();
+            for (Downloader& d : dl) d.abandon();
             src.restart();
-            c->tm = blu_timings{};
-            st = RunStatus{};
+            reset_timings(g);
+            for (Cfg& x : g) x.st = RunStatus{};
             continue;
         }
-        st.dup_found = h.dup_found != 0;
-        if (st.dup_found) {
-            dl.abandon();
+        for (Cfg& x : g) x.st.dup_found = g[0].h.dup_found != 0;
+        if (g[0].st.dup_found) {
+            for (Downloader& d : dl) d.abandon();
             return;
         }
-        finish_run(c, h, n, n_chunks, ms);
-        dl.finish(h);
-        if (host_text) r->ext_strings = host_text, r->ext_len = n;
+        finish_run(g, n, n_chunks, ms);
+        for (size_t i = 0; i < g.size(); i++) {
+            dl[i].finish(g[i].h);
+            if (host_text) g[i].r->ext_strings = host_text, g[i].r->ext_len = n;
+        }
         c->tm.ms_total_device = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
         return;
     }
@@ -1425,17 +1521,18 @@ void reset_parts(blu_result* r, size_t n) {
     r->parts.resize(n);
 }
 
-// Bytes [begin, begin + len) of a table in memory or in a file through the host-text loop of a single-device context.
+// Bytes [begin, begin + len) of a table in memory or in a file through the host-text loop of single-device contexts.
 // `sharers`: the file sources of a multi-device run that share the host's cores.
-void run_span(blu_ctx* c, const ByteView& v, uint64_t begin, uint64_t len, ResultPartOwned* p, RunStatus& st, bool text_refs, int sharers) {
+void run_span(Pass& g, const ByteView& v, uint64_t begin, uint64_t len, bool text_refs, int sharers) {
+    blu_ctx* c = g[0].c;
     if (v.mem) {
         const uint64_t chunk = chunk_bytes_of(c, 256ull << 20);
         MemorySource src(v.mem + begin, chunk);
-        run_host_chunks(c, src, len, chunk, p, st, text_refs ? v.mem + begin : nullptr);
+        run_host_chunks(g, src, len, chunk, text_refs ? v.mem + begin : nullptr);
     } else {
         const uint64_t chunk = chunk_bytes_of(c, 64ull << 20);
         FileSource src(c, v.fd, begin, len, chunk, sharers);
-        run_host_chunks(c, src, len, chunk, p, st, nullptr);
+        run_host_chunks(g, src, len, chunk, nullptr);
     }
 }
 
@@ -1451,7 +1548,10 @@ void run_sharded(blu_ctx* c, const ByteView& v, blu_result* r, bool text_refs) {
     for_each_shard(c, [&](size_t i) {
         blu_ctx* sh = c->shards[i].get();
         sh->tm = blu_timings{};
-        if (cuts[i + 1] > cuts[i]) run_span(sh, v, cuts[i], cuts[i + 1] - cuts[i], &r->parts[i], st[i], text_refs, (int)N);
+        if (cuts[i + 1] <= cuts[i]) return;
+        Pass g{Cfg{sh, &r->parts[i]}};
+        run_span(g, v, cuts[i], cuts[i + 1] - cuts[i], text_refs, (int)N);
+        st[i] = g[0].st;
     });
     std::vector<uint64_t> n_rec(N);
     for (size_t i = 0; i < N; i++) n_rec[i] = st[i].dup_found ? 0 : r->parts[i].n_rec;
@@ -1460,33 +1560,60 @@ void run_sharded(blu_ctx* c, const ByteView& v, blu_result* r, bool text_refs) {
     r->n_rows = c->tm.n_rows;
 }
 
-// A table in host memory or a file -> result, on one or several GPUs.  `text_refs` applies to host memory only.
-void run_table(blu_ctx* c, const ByteView& v, blu_result* r, bool text_refs) {
+// The configurations of one call and the results they fill: one for blu_consensus_run_*, up to kMaxConfigs single-device
+// contexts of one GPU for blu_consensus_run_*_configs.
+struct Member {
+    blu_ctx* c;
+    blu_result* r;
+};
+using Group = std::vector<Member>;
+
+// A single-device pass over the group: every result gets one empty part.
+Pass new_pass(const Group& g) {
+    Pass p;
+    for (const Member& m : g) {
+        reset_parts(m.r, 1);
+        p.push_back(Cfg{m.c, &m.r->parts[0]});
+    }
+    return p;
+}
+
+// What a single-device pass leaves for its caller: a repeated id (the table is regrouped and run again), else the
+// consensus-class error of the lowest configuration that has one -- named by its index when the pass has several.
+void settle(const Group& g, const Pass& p) {
+    if (p[0].st.dup_found) throw NonContiguous("a query id occurs in two non-adjacent groups of rows");
+    for (size_t i = 0; i < p.size(); i++)
+        if (p[i].st.soft_code) throw_device_error(p[i].st.soft_code, p[i].st.soft_off, p.size() > 1 ? "ctxs[" + std::to_string(i) + "]: " : "");
+    for (const Member& m : g) m.r->n_rows = m.c->tm.n_rows;
+}
+
+// A table in host memory or a file -> results, on one or several GPUs (a group has one context then).  `text_refs` applies
+// to host memory only.
+void run_table(const Group& g, const ByteView& v, bool text_refs) {
+    blu_ctx* c = g[0].c;
     if (c->is_multi()) {
-        run_sharded(c, v, r, text_refs);
+        run_sharded(c, v, g[0].r, text_refs);
         return;
     }
     CK(cudaSetDevice(c->device));
-    reset_parts(r, 1);
-    RunStatus st;
-    run_span(c, v, 0, v.n, &r->parts[0], st, text_refs, 1);
-    settle(st);
-    r->n_rows = c->tm.n_rows;
+    Pass p = new_pass(g);
+    run_span(p, v, 0, v.n, text_refs, 1);
+    settle(g, p);
 }
 
-// The regrouped table (device memory of ours) through the device-text loop of a single-device context.
-void run_regrouped_device(blu_ctx* c, const DevMem& dt, cudaStream_t s, blu_result* r, bool resident) {
-    reset_parts(r, 1);
-    RunStatus st;
-    run_device_text(c, dt.p, dt.n, s, &r->parts[0], st, resident);
-    if (st.dup_found) throw std::runtime_error("a regrouped table is still not contiguous");
-    settle(st);
-    r->n_rows = c->tm.n_rows;
+// The regrouped table (device memory of ours) through the device-text loop of single-device contexts.
+void run_regrouped_device(const Group& g, const DevMem& dt, cudaStream_t s, bool resident) {
+    Pass p = new_pass(g);
+    run_device_text(p, dt.p, dt.n, s, resident);
+    if (p[0].st.dup_found) throw std::runtime_error("a regrouped table is still not contiguous");
+    settle(g, p);
 }
 
-// A scattered table, host text or device text (single-device context), regrouped -- on the GPU when regroup_gpu allows it,
-// else on the host -- and run again.  The regrouped text is ours: the result's strings are copied into a pool.
-void run_scattered(blu_ctx* c, const char* h_text, const uint8_t* d_text, uint64_t n, cudaStream_t s, blu_result* r) {
+// A scattered table, host text or device text, regrouped once -- on the GPU of the first context when regroup_gpu allows it,
+// else on the host -- and run again for every configuration.  The regrouped text is ours: the results' strings are copied
+// into pools.
+void run_scattered(const Group& g, const char* h_text, const uint8_t* d_text, uint64_t n, cudaStream_t s) {
+    blu_ctx* c = g[0].c;
     DevMem dt;
     if (regroup_gpu(c, h_text, d_text, n, s, dt)) {
         if (c->is_multi()) {
@@ -1495,9 +1622,9 @@ void run_scattered(blu_ctx* c, const char* h_text, const uint8_t* d_text, uint64
             CK(cudaMemcpy(re.data(), dt.p, dt.n, cudaMemcpyDeviceToHost));
             cudaFree(dt.p);
             dt.p = nullptr;
-            run_table(c, ByteView(re.data(), re.size()), r, false);
+            run_table(g, ByteView(re.data(), re.size()), false);
         } else
-            run_regrouped_device(c, dt, c->stream, r, false);
+            run_regrouped_device(g, dt, c->stream, false);
         c->tm.n_regrouped = 2;
         return;
     }
@@ -1509,7 +1636,7 @@ void run_scattered(blu_ctx* c, const char* h_text, const uint8_t* d_text, uint64
     }
     const std::string re = regroup_by_query(h_text, n);
     std::string().swap(host);
-    run_table(c, ByteView(re.data(), re.size()), r, false);
+    run_table(g, ByteView(re.data(), re.size()), false);
     c->tm.n_regrouped = 1;
 }
 
@@ -1741,21 +1868,149 @@ void sort_part_host(blu_ctx* g, ResultPartOwned& p) {
     tr.mark("permute");
 }
 
-// What every blu_consensus_run_* entry point does with its result: made for `run`, handed out on success, freed on failure.
+// A pass with several configurations: every context reports the shared pass -- the first one's launches, copies and kernel
+// times -- and the bytes all of them downloaded; result and taxonomy bytes stay each context's own.
+void share_timings(const std::vector<blu_ctx*>& cs) {
+    if (cs.size() < 2) return;
+    uint64_t d2h = 0;
+    for (blu_ctx* c : cs) d2h += c->tm.d2h_bytes;
+    for (blu_ctx* c : cs) {
+        const uint64_t result = c->tm.result_bytes, tax = c->tm.taxonomy_bytes;
+        c->tm = cs[0]->tm;
+        c->tm.result_bytes = result, c->tm.taxonomy_bytes = tax, c->tm.d2h_bytes = d2h;
+    }
+}
+
+// What every blu_consensus_run_* entry point does with its results: one per context, made for `run`, handed out on
+// success, all freed on failure; the message of a failure goes to every context.
 template <class F>
-int run_entry(blu_ctx* c, blu_result** out, F&& run) {
-    std::unique_ptr<blu_result> r;
-    const int rc = guarded(c, [&] {
-        require_tax(c);
-        r = new_result(c);
-        run(r.get());
+int run_entry(const std::vector<blu_ctx*>& cs, blu_result** outs, F&& run) {
+    std::vector<std::unique_ptr<blu_result>> rs;
+    const int rc = guarded(cs[0], [&] {
+        Group g;
+        for (blu_ctx* c : cs) {
+            require_tax(c);
+            rs.push_back(new_result(c));
+            g.push_back(Member{c, rs.back().get()});
+        }
+        run(g);
+        share_timings(cs);
     });
+    for (blu_ctx* c : cs) c->err = cs[0]->err;
     if (rc != BLU_OK) {
-        blu_result_free(r.release());
+        for (auto& r : rs) blu_result_free(r.release());
         return rc;
     }
-    *out = r.release();
+    for (size_t i = 0; i < rs.size(); i++) outs[i] = rs[i].release();
     return BLU_OK;
+}
+
+int fail_all(const std::vector<blu_ctx*>& cs, int code, const std::string& msg) {
+    for (blu_ctx* c : cs) fail(c, code, msg);
+    return code;
+}
+
+// blu_consensus_run_host and _host_configs
+int host_entry(const std::vector<blu_ctx*>& cs, const char* text, uint64_t n, blu_result** outs) {
+    return run_entry(cs, outs, [&](const Group& g) {
+        try {
+            run_table(g, ByteView(text, n), (g[0].c->opts.flags & BLU_OPT_TEXT_REFS) != 0);
+        } catch (const NonContiguous&) {
+            run_scattered(g, text, nullptr, n, g[0].c->stream);
+        }
+    });
+}
+
+// blu_consensus_run_file and _file_configs: the file is streamed (FileSource); only a non-contiguous table (regrouping needs
+// all rows at once) is read whole.
+int file_entry(const std::vector<blu_ctx*>& cs, const char* path, blu_result** outs) {
+    struct Fd {
+        int fd;
+        ~Fd() {
+            if (fd >= 0) close(fd);
+        }
+    } f{open(path, O_RDONLY | O_CLOEXEC)};
+    struct stat st;
+    if (f.fd < 0 || fstat(f.fd, &st) != 0 || !S_ISREG(st.st_mode))
+        return fail_all(cs, BLU_ERR_IO, "Unexpected error occurred on load table.");  // mod.rs:357-364
+    const uint64_t n = (uint64_t)st.st_size;
+    return run_entry(cs, outs, [&](const Group& g) {
+        if (n == 0) throw DataErr("empty blast output (the reference's CsvReader fails on an empty file)");
+        try {
+            run_table(g, ByteView(f.fd, n), false);
+        } catch (const NonContiguous&) {
+            std::string all((size_t)n, '\0');
+            for (uint64_t off = 0; off < n;) {
+                ssize_t got = pread(f.fd, all.data() + off, (size_t)std::min<uint64_t>(n - off, 1ull << 30), (off_t)off);
+                if (got < 0 && errno == EINTR) continue;
+                if (got <= 0) throw IoErr("Unexpected error occurred on load table.");
+                off += (uint64_t)got;
+            }
+            run_scattered(g, all.data(), nullptr, n, g[0].c->stream);
+        }
+    });
+}
+
+// blu_consensus_run_device_resident and _device_resident_configs
+int resident_entry(const std::vector<blu_ctx*>& cs, const void* dtext, uint64_t n, void* stream, blu_result** outs) {
+    return run_entry(cs, outs, [&](const Group& g) {
+        blu_ctx* c = g[0].c;
+        CK(cudaSetDevice(c->device));
+        cudaStream_t s = stream ? (cudaStream_t)stream : c->stream;
+        Pass p = new_pass(g);
+        run_device_text(p, (const uint8_t*)dtext, n, s, true);
+        if (!p[0].st.dup_found) {
+            settle(g, p);
+            return;
+        }
+        // a scattered table: regrouped in HBM (blu_regroup.cu); the results' references then point into that copy, which
+        // the results own together (blu_result_device_text)
+        DevMem dt;
+        if (!regroup_gpu(c, nullptr, (const uint8_t*)dtext, n, s, dt))
+            throw UnsupportedErr("the table's queries are not contiguous and it cannot be regrouped on the device: use blu_consensus_run_device / _host / _file");
+        run_regrouped_device(g, dt, s, true);
+        const std::shared_ptr<uint8_t> owned(dt.p, [](uint8_t* q) { cudaFree(q); });
+        dt.p = nullptr;
+        for (const Member& m : g) m.r->parts[0].owned_dtext = owned;
+        c->tm.n_regrouped = 2;
+    });
+}
+
+// The rules of a group of configurations (include/blu_consensus.h); the message of the first one broken, or "".
+std::string group_error(const std::vector<blu_ctx*>& cs) {
+    const blu_ctx* c0 = cs[0];
+    for (size_t i = 0; i < cs.size(); i++) {
+        const blu_ctx* c = cs[i];
+        const std::string at = "ctxs[" + std::to_string(i) + "]: ";
+        if (c->is_multi()) return at + "a multi-device context cannot be part of a group of configurations";
+        if (!c->tax) return at + "no taxonomy loaded (call blu_taxonomy_load_json first)";
+        for (size_t j = 0; j < i; j++)
+            if (cs[j] == c) return at + "the same context as ctxs[" + std::to_string(j) + "]";
+        if (c->device != c0->device) return at + "on another device than ctxs[0]";
+        if (c->opts.chunk_bytes != c0->opts.chunk_bytes) return at + "chunk_bytes differs from that of ctxs[0]";
+        if (c->opts.flags != c0->opts.flags) return at + "flags differ from those of ctxs[0]";
+    }
+    return "";
+}
+
+// Checks the arguments every _configs entry point takes: 0 and the contexts in `cs`, or the error code.  The message goes to
+// every context listed and to blu_last_error(NULL).
+int take_group(blu_ctx* const* ctxs, int n, blu_result** outs, std::vector<blu_ctx*>& cs) {
+    auto refuse = [&](const std::string& msg) {
+        fail(nullptr, BLU_ERR_ARG, msg);
+        for (int i = 0; ctxs && i < n; i++)
+            if (ctxs[i]) fail(ctxs[i], BLU_ERR_ARG, msg);
+        return BLU_ERR_ARG;
+    };
+    if (!ctxs || n < 1 || n > kMaxConfigs) return refuse("a group holds 1 to 8 contexts");
+    for (int i = 0; i < n; i++)
+        if (!ctxs[i]) return refuse("ctxs[" + std::to_string(i) + "] is null");
+    if (!outs) return refuse("null argument");
+    cs.assign(ctxs, ctxs + n);
+    for (int i = 0; i < n; i++) outs[i] = nullptr;
+    if (n == 1) return BLU_OK;
+    const std::string e = group_error(cs);
+    return e.empty() ? BLU_OK : refuse(e);
 }
 
 }  // namespace
@@ -1968,17 +2223,15 @@ int blu_consensus_run_device(blu_ctx* c, const void* dtext, uint64_t n, void* st
     if (!c || !out || (!dtext && n)) return fail(c, BLU_ERR_ARG, "null argument");
     *out = nullptr;
     if (c->is_multi()) return fail(c, BLU_ERR_ARG, "device-resident text belongs to one GPU: use a single-device context");
-    return run_entry(c, out, [&](blu_result* r) {
+    return run_entry({c}, out, [&](const Group& g) {
         CK(cudaSetDevice(c->device));
         cudaStream_t s = stream ? (cudaStream_t)stream : c->stream;
         try {
-            reset_parts(r, 1);
-            RunStatus st;
-            run_device_text(c, (const uint8_t*)dtext, n, s, &r->parts[0], st, false);
-            settle(st);
-            r->n_rows = c->tm.n_rows;
+            Pass p = new_pass(g);
+            run_device_text(p, (const uint8_t*)dtext, n, s, false);
+            settle(g, p);
         } catch (const NonContiguous&) {
-            run_scattered(c, nullptr, (const uint8_t*)dtext, n, s, r);
+            run_scattered(g, nullptr, (const uint8_t*)dtext, n, s);
         }
     });
 }
@@ -1987,27 +2240,15 @@ int blu_consensus_run_device_resident(blu_ctx* c, const void* dtext, uint64_t n,
     if (!c || !out || (!dtext && n)) return fail(c, BLU_ERR_ARG, "null argument");
     *out = nullptr;
     if (c->is_multi()) return fail(c, BLU_ERR_ARG, "device-resident text belongs to one GPU: use a single-device context");
-    return run_entry(c, out, [&](blu_result* r) {
-        CK(cudaSetDevice(c->device));
-        cudaStream_t s = stream ? (cudaStream_t)stream : c->stream;
-        reset_parts(r, 1);
-        RunStatus st;
-        run_device_text(c, (const uint8_t*)dtext, n, s, &r->parts[0], st, true);
-        if (!st.dup_found) {
-            settle(st);
-            r->n_rows = c->tm.n_rows;
-            return;
-        }
-        // a scattered table: regrouped in HBM (blu_regroup.cu); the result's references then point into that copy, which
-        // the result owns (blu_result_device_text)
-        DevMem dt;
-        if (!regroup_gpu(c, nullptr, (const uint8_t*)dtext, n, s, dt))
-            throw UnsupportedErr("the table's queries are not contiguous and it cannot be regrouped on the device: use blu_consensus_run_device / _host / _file");
-        run_regrouped_device(c, dt, s, r, true);
-        r->parts[0].owned_dtext = std::shared_ptr<uint8_t>(dt.p, [](uint8_t* q) { cudaFree(q); });
-        dt.p = nullptr;
-        c->tm.n_regrouped = 2;
-    });
+    return resident_entry({c}, dtext, n, stream, out);
+}
+
+int blu_consensus_run_device_resident_configs(blu_ctx* const* ctxs, int n_ctx, const void* dtext, uint64_t n, void* stream, blu_result** outs) {
+    std::vector<blu_ctx*> cs;
+    if (int rc = take_group(ctxs, n_ctx, outs, cs)) return rc;
+    if (n_ctx == 1) return blu_consensus_run_device_resident(cs[0], dtext, n, stream, outs);
+    if (!dtext && n) return fail_all(cs, BLU_ERR_ARG, "null argument");
+    return resident_entry(cs, dtext, n, stream, outs);
 }
 
 const void* blu_result_device_text(const blu_result* r, uint64_t* n) {
@@ -2064,44 +2305,29 @@ int blu_result_sort_by_query(blu_ctx* c, blu_result* r) {
 int blu_consensus_run_host(blu_ctx* c, const char* text, uint64_t n, blu_result** out) {
     if (!c || !out || (!text && n)) return fail(c, BLU_ERR_ARG, "null argument");
     *out = nullptr;
-    return run_entry(c, out, [&](blu_result* r) {
-        try {
-            run_table(c, ByteView(text, n), r, (c->opts.flags & BLU_OPT_TEXT_REFS) != 0);
-        } catch (const NonContiguous&) {
-            run_scattered(c, text, nullptr, n, c->stream, r);
-        }
-    });
+    return host_entry({c}, text, n, out);
 }
 
-// Streams the file (FileSource); only a non-contiguous table (regrouping needs all rows at once) is read whole.
+int blu_consensus_run_host_configs(blu_ctx* const* ctxs, int n_ctx, const char* text, uint64_t n, blu_result** outs) {
+    std::vector<blu_ctx*> cs;
+    if (int rc = take_group(ctxs, n_ctx, outs, cs)) return rc;
+    if (n_ctx == 1) return blu_consensus_run_host(cs[0], text, n, outs);
+    if (!text && n) return fail_all(cs, BLU_ERR_ARG, "null argument");
+    return host_entry(cs, text, n, outs);
+}
+
 int blu_consensus_run_file(blu_ctx* c, const char* path, blu_result** out) {
     if (!c || !path || !out) return fail(c, BLU_ERR_ARG, "null argument");
     *out = nullptr;
-    struct Fd {
-        int fd;
-        ~Fd() {
-            if (fd >= 0) close(fd);
-        }
-    } f{open(path, O_RDONLY | O_CLOEXEC)};
-    struct stat st;
-    if (f.fd < 0 || fstat(f.fd, &st) != 0 || !S_ISREG(st.st_mode))
-        return fail(c, BLU_ERR_IO, "Unexpected error occurred on load table.");  // mod.rs:357-364
-    const uint64_t n = (uint64_t)st.st_size;
-    return run_entry(c, out, [&](blu_result* r) {
-        if (n == 0) throw DataErr("empty blast output (the reference's CsvReader fails on an empty file)");
-        try {
-            run_table(c, ByteView(f.fd, n), r, false);
-        } catch (const NonContiguous&) {
-            std::string all((size_t)n, '\0');
-            for (uint64_t off = 0; off < n;) {
-                ssize_t got = pread(f.fd, all.data() + off, (size_t)std::min<uint64_t>(n - off, 1ull << 30), (off_t)off);
-                if (got < 0 && errno == EINTR) continue;
-                if (got <= 0) throw IoErr("Unexpected error occurred on load table.");
-                off += (uint64_t)got;
-            }
-            run_scattered(c, all.data(), nullptr, n, c->stream, r);
-        }
-    });
+    return file_entry({c}, path, out);
+}
+
+int blu_consensus_run_file_configs(blu_ctx* const* ctxs, int n_ctx, const char* path, blu_result** outs) {
+    std::vector<blu_ctx*> cs;
+    if (int rc = take_group(ctxs, n_ctx, outs, cs)) return rc;
+    if (n_ctx == 1) return blu_consensus_run_file(cs[0], path, outs);
+    if (!path) return fail_all(cs, BLU_ERR_ARG, "null argument");
+    return file_entry(cs, path, outs);
 }
 
 int blu_result_add_headers(blu_result* r, const char* headers_nl, uint64_t len) {

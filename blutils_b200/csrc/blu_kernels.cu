@@ -11,6 +11,8 @@
 //                    rows, bit score beyond int32, first row without a predecessor in its window).
 //   gather_kernel  : copies query ids and accessions of finished queries into the result's string pool.
 //   dup_kernel     : detects a query id that occurs in two separate runs (non-contiguous input).
+//   fanout_kernel  : several configurations in one pass: copies the tile kernel's record headers and text cursors from the
+//                    first configuration to the others.
 //
 // Reference semantics: see blu_core.cuh.  Geometry and roofline accounting: DESIGN.md.
 #include <cuda_runtime.h>
@@ -2453,24 +2455,26 @@ __global__ void __launch_bounds__(256) dup_kernel(const __grid_constant__ DupPar
     for (unsigned long long i = rb + (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (unsigned long long)gridDim.x * blockDim.x) {
         blu_record& r = p.records[i];
         if (r.query_off + (unsigned long long)r.query_len > p.strings_len) continue;  // (a gather pass that overflowed: the host reruns)
-        unsigned long long h = 0xcbf29ce484222325ull;
-        const uint8_t* q = p.strings + r.query_off;
-        for (unsigned k = 0; k < r.query_len; k++) {
-            h ^= q[k];
-            h *= 0x100000001b3ull;
-        }
-        h = mix64(h ^ r.query_len);
-        if (h == 0) h = 1;
-        if (p.hashes) p.hashes[i] = h;
-        unsigned slot = (unsigned)h & p.mask;
-        for (unsigned t = 0; t <= p.mask; t++) {
-            const unsigned long long old = atomicCAS(p.table + slot, 0ull, h);
-            if (old == 0ull) break;
-            if (old == h) {
-                p.ctr->dup_found = 1;
-                break;
+        if (p.table) {
+            unsigned long long h = 0xcbf29ce484222325ull;
+            const uint8_t* q = p.strings + r.query_off;
+            for (unsigned k = 0; k < r.query_len; k++) {
+                h ^= q[k];
+                h *= 0x100000001b3ull;
             }
-            slot = (slot + 1) & p.mask;
+            h = mix64(h ^ r.query_len);
+            if (h == 0) h = 1;
+            if (p.hashes) p.hashes[i] = h;
+            unsigned slot = (unsigned)h & p.mask;
+            for (unsigned t = 0; t <= p.mask; t++) {
+                const unsigned long long old = atomicCAS(p.table + slot, 0ull, h);
+                if (old == 0ull) break;
+                if (old == h) {
+                    p.ctr->dup_found = 1;
+                    break;
+                }
+                slot = (slot + 1) & p.mask;
+            }
         }
         if (p.ref_delta) {
             r.query_off = (unsigned long long)((long long)r.query_off + p.ref_delta);
@@ -2501,6 +2505,36 @@ __global__ void __launch_bounds__(256) dup_merge_kernel(const unsigned long long
             }
             slot = (slot + 1) & mask;
         }
+    }
+}
+
+// Tile kernel output -> the other configurations of a pass (see FanoutParams).  Threads 0..n_dst-1 of block 0 copy the
+// cursors; the whole grid copies the record headers, 16 bytes per thread and step.
+__global__ void __launch_bounds__(256) fanout_kernel(const __grid_constant__ FanoutParams p) {
+    const Counters* s = p.src;
+    const unsigned long long rb = s->post_done;
+    unsigned long long re = s->rec_count;
+    if (re > p.rec_cap) re = p.rec_cap;
+    if (!s->cap_overflow && re > rb) {  // (after an overflow every configuration runs again: nothing to copy)
+        constexpr unsigned long long kPer = sizeof(blu_record) / sizeof(uint4);
+        const unsigned long long n = (re - rb) * kPer;
+        const uint4* src = reinterpret_cast<const uint4*>(p.src_records + rb);
+        const unsigned long long stride = (unsigned long long)gridDim.x * blockDim.x;
+        for (unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i < n * (unsigned long long)p.n_dst; i += stride) {
+            const unsigned long long d = i / n, j = i - d * n;
+            reinterpret_cast<uint4*>(p.dst_records[d] + rb)[j] = src[j];
+        }
+    }
+    if (blockIdx.x == 0 && (int)threadIdx.x < p.n_dst) {
+        Counters* d = p.dst[threadIdx.x];
+        // the long-run kernel adds one record per finished deferred run in every configuration: the record counts agree
+        if (d->post_done != rb) report(d, DE_INTERNAL, 0);
+        d->rec_count = s->rec_count;
+        d->slot_count = s->slot_count;
+        d->n_defer = s->n_defer;
+        if (s->tail_start < d->tail_start) d->tail_start = s->tail_start;
+        if (s->err_code && !d->err_code) d->err_code = s->err_code, d->err_off = s->err_off;
+        if (s->cap_overflow) d->cap_overflow = 1;
     }
 }
 
@@ -2561,6 +2595,11 @@ cudaError_t launch_gather_kernel(const PostParams& p, int sms, cudaStream_t s) {
 
 cudaError_t launch_dup_kernel(const DupParams& p, int sms, cudaStream_t s) {
     dup_kernel<<<sms * 8, 256, 0, s>>>(p);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_fanout_kernel(const FanoutParams& p, int sms, cudaStream_t s) {
+    fanout_kernel<<<sms * 4, 256, 0, s>>>(p);
     return cudaGetLastError();
 }
 

@@ -86,11 +86,29 @@ struct DupParams {
     blu_acc* accs;
     const uint8_t* strings;     // what blu_record.query_off refers to: the string pool, or the text when nothing was gathered
     uint64_t strings_len;
-    unsigned long long* table;  // open addressing, 0 = empty
+    unsigned long long* table;  // open addressing, 0 = empty; nullptr: no check, only the relocation below (the other
+                                // configurations of a pass: their ids are the first configuration's)
     uint32_t mask;
     unsigned long long* hashes; // optional: the 64-bit id hash of every record (multi-device runs merge them), or nullptr
     long long ref_delta;        // added to every string offset after hashing (device-buffer -> caller's text coordinates)
     Counters* ctr;
+};
+
+// Configurations of one pass over a table (blu_consensus_run_*_configs): the tile kernel runs once, into the first one's
+// records and counters; everything after it runs once per configuration.
+constexpr int kMaxConfigs = 8;
+
+// Behind the tile kernel of a pass with several configurations: the record headers it wrote, [src->post_done,
+// src->rec_count), and the cursors that depend on the text only (record / slot / deferred-run counts, the open tail, the
+// first grammar error, a capacity overflow) are copied from the first configuration to the others.  Every configuration
+// of a pass has the same record capacity, so the headers keep their indices.
+struct FanoutParams {
+    const Counters* src;
+    const blu_record* src_records;
+    Counters* dst[kMaxConfigs - 1];
+    blu_record* dst_records[kMaxConfigs - 1];
+    int n_dst;
+    uint64_t rec_cap;
 };
 
 // End of a range / chunk: post_done <- rec_count, the per-range counters are reset (next_begin <- tail_start or range_end)
@@ -125,6 +143,7 @@ cudaError_t launch_longrun_kernel(const RunParams& p, int grid, cudaStream_t s);
 cudaError_t launch_consensus_kernel(const PostParams& p, int sms, cudaStream_t s);
 cudaError_t launch_gather_kernel(const PostParams& p, int sms, cudaStream_t s);
 cudaError_t launch_dup_kernel(const DupParams& p, int sms, cudaStream_t s);
+cudaError_t launch_fanout_kernel(const FanoutParams& p, int sms, cudaStream_t s);
 cudaError_t launch_advance_kernel(const AdvanceParams& p, cudaStream_t s);
 cudaError_t launch_dup_merge_kernel(const unsigned long long* hashes, unsigned long long n, unsigned long long* table, uint32_t mask,
                                     unsigned int* dup_found, int sms, cudaStream_t s);

@@ -179,6 +179,31 @@ int blu_consensus_run_file(blu_ctx* ctx, const char* blast_out_path, blu_result*
  * (mod.rs:84-102).  Call before serialising. */
 int blu_result_add_headers(blu_result* res, const char* headers_nl, uint64_t len);
 
+/* ---- several configurations in one pass ---------------------------------------------------------------------------
+ * One pass over the table, one result per context: outs[k] is what blu_consensus_run_*(ctxs[k], ...) returns on its own --
+ * the same blu_result_checksum, canonical JSONL, counts and writer bytes (record order is unspecified, as it is there).
+ * The text is parsed once (and, from host memory or a file, copied to the device once); only the consensus and what
+ * follows it runs per context.  outs[k] belongs to ctxs[k]: blu_result_sort_by_query(ctxs[k], outs[k]),
+ * blu_result_download, blu_result_add_headers and the writers work on it as on any result.
+ *   - 1 <= n_ctx <= 8.  n_ctx == 1 is blu_consensus_run_*(ctxs[0], ...) itself.
+ *   - Otherwise all contexts are distinct single-device contexts of one device, each with a taxonomy loaded (the
+ *     taxonomies may differ: a textLineage and a numericLineage context can be grouped), and opts.chunk_bytes and
+ *     opts.flags are equal across the group.  Anything else returns BLU_ERR_ARG; the message names the context.
+ *   - All or nothing: on an error no result is returned and every context of the group carries the message.  A
+ *     grammar-class error of the table is the same for every configuration; a consensus-class one (e.g. an empty adjusted
+ *     taxonomy, which depends on the cutoffs) fails the call with the error of the lowest-index context that has one, and
+ *     the message starts with "ctxs[k]: ".  BLU_ERR_UNSUPPORTED limits are those of a single run.
+ *   - A table whose queries are not contiguous is regrouped once, and every configuration runs over the regrouped text;
+ *     the device-resident results share the regrouped copy (blu_result_device_text), which lives until the last of them
+ *     is freed.
+ *   - blu_ctx_last_timings of every context reports the shared pass: n_tile_launches, h2d_bytes and text_bytes are those
+ *     of one single-context run, n_kernel_launches counts every launch of the pass, d2h_bytes everything the pass
+ *     downloaded; result_bytes and taxonomy_bytes are the context's own. */
+int blu_consensus_run_host_configs(blu_ctx* const* ctxs, int n_ctx, const char* text, uint64_t n_bytes, blu_result** outs);
+int blu_consensus_run_file_configs(blu_ctx* const* ctxs, int n_ctx, const char* path, blu_result** outs);
+int blu_consensus_run_device_resident_configs(blu_ctx* const* ctxs, int n_ctx, const void* dtext, uint64_t n_bytes, void* stream,
+                                              blu_result** outs);
+
 /* ---- results -------------------------------------------------------------------------------------------- */
 uint64_t blu_result_num_queries(const blu_result* res);
 /* Records with hits only (blu_result_num_queries also counts hit-less headers). */

@@ -37,6 +37,10 @@ extern "C" {
     pub fn blu_taxonomy_load_json_cached(ctx: *mut blu_ctx, path: *const c_char, cache_path: *const c_char, cache_state: *mut c_int) -> c_int;
     pub fn blu_consensus_run_file(ctx: *mut blu_ctx, blast_out: *const c_char, out: *mut *mut blu_result) -> c_int;
     pub fn blu_consensus_run_host(ctx: *mut blu_ctx, text: *const c_char, n: u64, out: *mut *mut blu_result) -> c_int;
+    pub fn blu_consensus_run_host_configs(ctxs: *const *mut blu_ctx, n_ctx: c_int, text: *const c_char, n: u64, outs: *mut *mut blu_result) -> c_int;
+    pub fn blu_consensus_run_file_configs(ctxs: *const *mut blu_ctx, n_ctx: c_int, blast_out: *const c_char, outs: *mut *mut blu_result) -> c_int;
+    pub fn blu_consensus_run_device_resident_configs(ctxs: *const *mut blu_ctx, n_ctx: c_int, dtext: *const c_void, n: u64, stream: *mut c_void,
+                                                     outs: *mut *mut blu_result) -> c_int;
     pub fn blu_result_add_headers(res: *mut blu_result, headers_nl: *const c_char, len: u64) -> c_int;
     pub fn blu_result_num_queries(res: *const blu_result) -> u64;
     pub fn blu_result_num_records(res: *const blu_result) -> u64;

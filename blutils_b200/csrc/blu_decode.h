@@ -1,5 +1,6 @@
 // blu_decode.h -- host-side decoding of the binary consensus records into the reference's result objects and
-// the writer of `write_blutils_output` (reference core/src/use_cases/write_blutils_output.rs:33-250).
+// the writer of `write_blutils_output` (reference core/src/use_cases/write_blutils_output.rs:33-250), and the TSV layout of
+// build-tabular that blu_tabular.h shares.
 // Header-only so that the C ABI (blu_api.cpp) and the test-only host simulation (tests/csrc) share it.
 #pragma once
 #include <sys/stat.h>
@@ -48,24 +49,26 @@ struct ResultView {
 };
 
 // ---------------------------------------------------------------------------------------------------------------
-// decoding: records -> the reference's JSON objects
+// decoding: records -> the reference's result objects
 // ---------------------------------------------------------------------------------------------------------------
 inline std::string_view rec_query(const ResultPart& p, const blu_record& rc) { return std::string_view(p.pool + rc.query_off, rc.query_len); }
 
-// serde form of Option<LinnaeanRank> for max_allowed_rank (bbci.rs:22-30): DefaultRank -> the enum variant,
-// NonDefaultRank(name) -> Other(name) where name = rank.to_string()
-inline void append_allowed_rank(std::string& o, const HostTaxonomy& T, const std::vector<uint8_t>& in_bb, uint32_t pos) {
-    const RankInfo& ri = T.ranks[T.pos_rank[pos]];
-    json_escape(o, in_bb[T.pos_rank[pos]] ? ri.full : ri.display);
+// serde_yaml 0.9 scalars (defined below)
+inline void yaml_str(std::string& o, std::string_view s);
+inline void yaml_f64(std::string& o, double v);
+
+// A field is built here before it is escaped or placed: one string per thread, so no allocation per record.
+inline std::string& scratch() {
+    thread_local std::string s;
+    s.clear();
+    return s;
 }
 
 struct Decoder {
-    const ResultView* r;
     const HostTaxonomy& T;
     std::vector<uint8_t> in_bb;  // per rank id: default rank present in the cutoff backbone
-    Decoder(const ResultView* res) : r(res), T(*res->tax) {
-        const Cutoffs& cut = res->cut;
-        auto bb = make_backbone(cut);
+    explicit Decoder(const ResultView* r) : T(*r->tax) {
+        auto bb = make_backbone(r->cut);
         in_bb.resize(T.ranks.size());
         for (size_t i = 0; i < T.ranks.size(); i++) {
             in_bb[i] = 0;
@@ -74,112 +77,110 @@ struct Decoder {
                     if (b.def == T.ranks[i].def) in_bb[i] = 1;
         }
     }
-    // `"taxon":{...}` object body (TaxonomyBean, taxonomy_bean.rs:5-17) in compact or pretty layout
-    void taxon(std::string& o, const ResultPart& part, const blu_record& rc, bool pretty, int ind) const {
+
+    // ---- the fields of a record: the writers read the taxonomy tables through these only ----
+    // TaxonomyBean (taxonomy_bean.rs:5-17)
+    std::string_view reached_rank(const blu_record& rc) const { return T.ranks[T.pos_rank[T.lin_off[rc.ref_lineage] + rc.reached_pos]].full; }
+    // serde form of Option<LinnaeanRank> for max_allowed_rank (bbci.rs:22-30), nullptr = None: DefaultRank -> the enum variant,
+    // NonDefaultRank(name) -> Other(name) where name = rank.to_string()
+    const std::string* allowed_rank(const blu_record& rc) const {
+        if (rc.allowed_pos < 0) return nullptr;
+        const uint32_t k = T.pos_rank[T.lin_off[rc.ref_lineage] + rc.allowed_pos];
+        return in_bb[k] ? &T.ranks[k].full : &T.ranks[k].display;
+    }
+    std::string_view identifier(const blu_record& rc) const { return T.idents[T.pos_ident[T.lin_off[rc.ref_lineage] + rc.reached_pos]]; }
+    // `taxonomy`: the kept positions of the reference lineage
+    void append_taxonomy(std::string& o, const blu_record& rc) const {
         const uint32_t lo = T.lin_off[rc.ref_lineage];
+        bool first = true;
+        for (int j = 0; j < T.lin_len(rc.ref_lineage); j++)
+            if (rc.keep_mask >> j & 1) {
+                if (!first) o.push_back(';');
+                first = false;
+                T.append_bean(o, lo + j);
+            }
+    }
+    // ConsensusBean (consensus_result.rs:37-45) b of a record: rank and identifier at the record's bean level of the bean's
+    // first lineage, `taxonomy` that whole lineage
+    const blu_bean& bean(const ResultPart& p, const blu_record& rc, uint32_t b) const { return p.beans[rc.bean_base + b]; }
+    std::string_view bean_rank(const blu_record& rc, const blu_bean& bn) const { return T.ranks[T.pos_rank[T.lin_off[bn.first_lineage] + rc.bean_level]].full; }
+    std::string_view bean_identifier(const blu_record& rc, const blu_bean& bn) const { return T.idents[T.pos_ident[T.lin_off[bn.first_lineage] + rc.bean_level]]; }
+    uint32_t occurrences(const blu_bean& bn) const { return bn.occurrences; }
+    void append_lineage(std::string& o, const blu_bean& bn) const { T.append_lineage(o, bn.first_lineage); }
+    std::string_view accession(const ResultPart& p, const blu_record& rc, const blu_bean& bn, uint32_t a) const {
+        const blu_acc& ac = p.accs[rc.acc_base + bn.acc_begin + a];
+        return std::string_view(p.pool + BLU_ACC_OFF(ac), BLU_ACC_LEN(ac));
+    }
+
+    // ---- serde_json ----
+    // `"taxon":{...}` object body in compact or pretty layout
+    void taxon(std::string& o, const ResultPart& part, const blu_record& rc, bool pretty, int ind) const {
         auto nl = [&](int extra) {
             if (!pretty) return;
             o.push_back('\n');
             o.append((size_t)(ind + extra) * 2, ' ');
         };
-        const char* colon = pretty ? ": " : ":";
+        auto key = [&](int extra, const char* k) {
+            nl(extra);
+            o.push_back('"');
+            o += k;
+            o += pretty ? "\": " : "\":";
+        };
+        std::string& s = scratch();
         o.push_back('{');
-        nl(1);
-        o += "\"reachedRank\"";
-        o += colon;
-        json_escape(o, T.ranks[T.pos_rank[lo + rc.reached_pos]].full);
+        key(1, "reachedRank");
+        json_escape(o, reached_rank(rc));
         o.push_back(',');
-        nl(1);
-        o += "\"maxAllowedRank\"";
-        o += colon;
-        if (rc.allowed_pos < 0)
-            o += "null";
+        key(1, "maxAllowedRank");
+        if (const std::string* a = allowed_rank(rc))
+            json_escape(o, *a);
         else
-            append_allowed_rank(o, T, in_bb, lo + rc.allowed_pos);
+            o += "null";
         o.push_back(',');
-        nl(1);
-        o += "\"identifier\"";
-        o += colon;
-        json_escape(o, T.idents[T.pos_ident[lo + rc.reached_pos]]);
+        key(1, "identifier");
+        json_escape(o, identifier(rc));
         o.push_back(',');
-        nl(1);
-        o += "\"percIdentity\"";
-        o += colon;
+        key(1, "percIdentity");
         json_f64(o, rc.perc_identity);
         o.push_back(',');
-        nl(1);
-        o += "\"bitScore\"";
-        o += colon;
+        key(1, "bitScore");
         json_f64(o, (double)rc.bit_score);
         o.push_back(',');
-        nl(1);
-        o += "\"taxonomy\"";
-        o += colon;
-        {
-            std::string t;
-            bool first = true;
-            const int k = T.lin_len(rc.ref_lineage);
-            for (int j = 0; j < k; j++)
-                if (rc.keep_mask >> j & 1) {
-                    if (!first) t.push_back(';');
-                    first = false;
-                    T.append_bean(t, lo + j);
-                }
-            json_escape(o, t);
-        }
+        key(1, "taxonomy");
+        append_taxonomy(s, rc);
+        json_escape(o, s);
         o.push_back(',');
-        nl(1);
-        o += "\"mutated\"";
-        o += colon;
-        o += rc.mutated ? "true" : "false";
-        o.push_back(',');
-        nl(1);
-        o += "\"singleMatch\"";
-        o += colon;
-        o += rc.single_match ? "true" : "false";
-        o.push_back(',');
-        nl(1);
-        o += "\"consensusBeans\"";
-        o += colon;
+        key(1, "mutated");
+        o += rc.mutated ? "true," : "false,";
+        key(1, "singleMatch");
+        o += rc.single_match ? "true," : "false,";
+        key(1, "consensusBeans");
         o.push_back('[');
-        std::string lineage;
         for (uint32_t b = 0; b < rc.n_beans; b++) {
-            const blu_bean& bn = part.beans[rc.bean_base + b];
-            const uint32_t bp = T.lin_off[bn.first_lineage] + rc.bean_level;
+            const blu_bean& bn = bean(part, rc, b);
             if (b) o.push_back(',');
             nl(2);
             o.push_back('{');
-            nl(3);
-            o += "\"rank\"";
-            o += colon;
-            json_escape(o, T.ranks[T.pos_rank[bp]].full);
+            key(3, "rank");
+            json_escape(o, bean_rank(rc, bn));
             o.push_back(',');
-            nl(3);
-            o += "\"identifier\"";
-            o += colon;
-            json_escape(o, T.idents[T.pos_ident[bp]]);
+            key(3, "identifier");
+            json_escape(o, bean_identifier(rc, bn));
             o.push_back(',');
-            nl(3);
-            o += "\"occurrences\"";
-            o += colon;
-            o += std::to_string(bn.occurrences);
+            key(3, "occurrences");
+            o += std::to_string(occurrences(bn));
             o.push_back(',');
-            nl(3);
-            o += "\"taxonomy\"";
-            o += colon;
-            lineage.clear();
-            T.append_lineage(lineage, bn.first_lineage);
-            json_escape(o, lineage);
+            key(3, "taxonomy");
+            s.clear();
+            append_lineage(s, bn);
+            json_escape(o, s);
             o.push_back(',');
-            nl(3);
-            o += "\"accessions\"";
-            o += colon;
+            key(3, "accessions");
             o.push_back('[');
             for (uint32_t a = 0; a < bn.n_acc; a++) {
-                const blu_acc& ac = part.accs[rc.acc_base + bn.acc_begin + a];
                 if (a) o.push_back(',');
                 nl(4);
-                json_escape(o, std::string_view(part.pool + BLU_ACC_OFF(ac), BLU_ACC_LEN(ac)));
+                json_escape(o, accession(part, rc, bn, a));
             }
             if (bn.n_acc) nl(3);
             o.push_back(']');
@@ -222,6 +223,56 @@ struct Decoder {
         nl(0);
         o.push_back('}');
     }
+
+    // ---- serde_yaml 0.9: one QueryWithConsensus as an item of the block sequence `results` (write_blutils_output.rs:216-248) ----
+    void yaml_object(std::string& o, std::string_view query, const ResultPart* part, const blu_record* rc, std::string_view run_id) const {
+        o += "- runId: ";
+        yaml_str(o, run_id);
+        o += "\n  query: ";
+        yaml_str(o, query);
+        if (!rc) {
+            o += "\n  taxon: null\n";
+            return;
+        }
+        std::string& s = scratch();
+        o += "\n  taxon:\n    reachedRank: ";
+        yaml_str(o, reached_rank(*rc));
+        o += "\n    maxAllowedRank: ";
+        if (const std::string* a = allowed_rank(*rc))
+            yaml_str(o, *a);
+        else
+            o += "null";
+        o += "\n    identifier: ";
+        yaml_str(o, identifier(*rc));
+        o += "\n    percIdentity: ";
+        yaml_f64(o, rc->perc_identity);
+        o += "\n    bitScore: ";
+        yaml_f64(o, (double)rc->bit_score);
+        o += "\n    taxonomy: ";
+        append_taxonomy(s, *rc);
+        yaml_str(o, s);
+        o += rc->mutated ? "\n    mutated: true" : "\n    mutated: false";
+        o += rc->single_match ? "\n    singleMatch: true" : "\n    singleMatch: false";
+        o += rc->n_beans ? "\n    consensusBeans:\n" : "\n    consensusBeans: []\n";
+        for (uint32_t b = 0; b < rc->n_beans; b++) {
+            const blu_bean& bn = bean(*part, *rc, b);
+            o += "    - rank: ";
+            yaml_str(o, bean_rank(*rc, bn));
+            o += "\n      identifier: ";
+            yaml_str(o, bean_identifier(*rc, bn));
+            o += "\n      occurrences: " + std::to_string(occurrences(bn));
+            o += "\n      taxonomy: ";
+            s.clear();
+            append_lineage(s, bn);
+            yaml_str(o, s);
+            o += bn.n_acc ? "\n      accessions:\n" : "\n      accessions: []\n";
+            for (uint32_t a = 0; a < bn.n_acc; a++) {
+                o += "      - ";
+                yaml_str(o, accession(*part, *rc, bn, a));
+                o.push_back('\n');
+            }
+        }
+    }
 };
 
 struct Entry {
@@ -229,6 +280,17 @@ struct Entry {
     const blu_record* rec;  // nullptr = NoConsensusFound
     const ResultPart* part;
 };
+
+// write_blutils_output.rs:87-111 flattens the results: the records of every part in part order, then the hit-less headers
+inline std::vector<Entry> all_entries(const ResultView* r) {
+    std::vector<Entry> v;
+    v.reserve(r->n_rec() + (r->hitless_ ? r->hitless_->size() : 0));
+    for (auto& p : r->parts)
+        for (uint64_t i = 0; i < p.n_rec; i++) v.push_back({rec_query(p, p.rec[i]), &p.rec[i], &p});
+    if (r->hitless_)
+        for (auto& h : *r->hitless_) v.push_back({std::string_view(h), nullptr, nullptr});
+    return v;
+}
 
 inline unsigned host_threads() {
     unsigned n = std::thread::hardware_concurrency();
@@ -252,23 +314,14 @@ void parallel_ranges(size_t n, F&& f) {
 // equal ids keep their file order, like the reference's sort_by).  Records sorted on the GPU already (ResultView::sorted) are
 // only merged with the sorted hit-less headers, records first among equal ids: the same order.
 inline std::vector<Entry> sorted_entries(const ResultView* r) {
-    std::vector<Entry> v;
-    v.reserve(r->n_rec() + (r->hitless_ ? r->hitless_->size() : 0));
-    for (auto& p : r->parts)
-        for (uint64_t i = 0; i < p.n_rec; i++) v.push_back({rec_query(p, p.rec[i]), &p.rec[i], &p});
+    std::vector<Entry> v = all_entries(r);
     auto less = [](const Entry& a, const Entry& b) { return a.query < b.query; };
     if (r->sorted) {
-        std::vector<Entry> h;
-        if (r->hitless_)
-            for (auto& x : *r->hitless_) h.push_back({std::string_view(x), nullptr, nullptr});
-        if (h.empty()) return v;
-        std::stable_sort(h.begin(), h.end(), less);
-        std::vector<Entry> out(v.size() + h.size());
-        std::merge(v.begin(), v.end(), h.begin(), h.end(), out.begin(), less);
-        return out;
+        const auto headers = v.begin() + (std::ptrdiff_t)r->n_rec();
+        std::stable_sort(headers, v.end(), less);
+        std::inplace_merge(v.begin(), headers, v.end(), less);
+        return v;
     }
-    if (r->hitless_)
-        for (auto& h : *r->hitless_) v.push_back({std::string_view(h), nullptr, nullptr});
     const size_t n = v.size();
     unsigned nt = (unsigned)std::min<size_t>(host_threads(), std::max<size_t>(1, n / 65536));
     if (nt <= 1) {
@@ -642,11 +695,7 @@ inline std::string view_to_jsonl(const ResultView* r, uint64_t max_entries = ~0u
     std::vector<Entry> ent;
     const uint64_t total = r->n_rec() + (r->hitless_ ? r->hitless_->size() : 0);
     if (max_entries < total && !r->sorted) {
-        ent.reserve(total);
-        for (auto& p : r->parts)
-            for (uint64_t i = 0; i < p.n_rec; i++) ent.push_back({rec_query(p, p.rec[i]), &p.rec[i], &p});
-        if (r->hitless_)
-            for (auto& h : *r->hitless_) ent.push_back({std::string_view(h), nullptr, nullptr});
+        ent = all_entries(r);
         // (ties keep their file order like the stable full sort: compare the position as the last key)
         std::vector<uint64_t> idx(total);
         for (uint64_t i = 0; i < total; i++) idx[i] = i;
@@ -678,222 +727,172 @@ inline std::string view_to_jsonl(const ResultView* r, uint64_t max_entries = ~0u
     return out;
 }
 
+// write_blutils_output.rs:42-52: the extension is forced to match the format (the last dot after the last '/' starts it)
+inline std::string with_extension(const char* path, const char* ext) {
+    std::string target = path;
+    const size_t slash = target.find_last_of('/');
+    const size_t dot = target.find_last_of('.');
+    if (dot != std::string::npos && (slash == std::string::npos || dot > slash)) target.resize(dot);
+    return target + ext;
+}
+
 inline int view_write(const ResultView* r, const char* path, int format, const char* run_id_in) {
-    {
-        Decoder d(r);
-        auto ent = sorted_entries(r);
-        const std::string run_id = run_id_in ? std::string(run_id_in) : uuid_v4();
-        std::string target;
-        FILE* f = stdout;
-        if (path) {
-            // write_blutils_output.rs:42-52: the extension is forced to match the format
-            target = path;
-            size_t slash = target.find_last_of('/');
-            size_t dot = target.find_last_of('.');
-            if (dot != std::string::npos && (slash == std::string::npos || dot > slash)) target.resize(dot);
-            target += format == BLU_FORMAT_JSON ? ".json" : format == BLU_FORMAT_JSONL ? ".jsonl" : ".yaml";
-            {
-                std::error_code ec;
-                auto parent = std::filesystem::path(target).parent_path();
-                if (!parent.empty()) std::filesystem::create_directories(parent, ec);  // write_blutils_output.rs:64-73
-            }
-            f = fopen(target.c_str(), "wb");
-            if (!f) return BLU_ERR_IO;
+    Decoder d(r);
+    auto ent = sorted_entries(r);
+    const std::string run_id = run_id_in ? std::string(run_id_in) : uuid_v4();
+    FILE* f = stdout;
+    if (path) {
+        const std::string target = with_extension(path, format == BLU_FORMAT_JSON ? ".json" : format == BLU_FORMAT_JSONL ? ".jsonl" : ".yaml");
+        {
+            std::error_code ec;
+            auto parent = std::filesystem::path(target).parent_path();
+            if (!parent.empty()) std::filesystem::create_directories(parent, ec);  // write_blutils_output.rs:64-73
         }
-        const bool pretty = format == BLU_FORMAT_JSON && path != nullptr;  // to_string_pretty to a file, compact to stdout
-        bool wok = true;
-        auto put = [&](const char* t) { fwrite(t, 1, strlen(t), f); };
-        if (format == BLU_FORMAT_JSON) {
-            put(pretty ? "{\n  \"results\": [" : "{\"results\":[");
-            wok &= ordered_parallel_write(f, ent.size(), [&](std::string& o, size_t i) {
-                if (i) o.push_back(',');
-                if (pretty) o += "\n    ";
-                d.object(o, ent[i].query, ent[i].part, ent[i].rec, run_id.c_str(), pretty, 2);
-            });
-            if (pretty)
-                put(ent.empty() ? "],\n  \"config\": null\n}" : "\n  ],\n  \"config\": null\n}");
-            else
-                put("],\"config\":null}");
-        } else if (format == BLU_FORMAT_JSONL) {
-            put("null\n");  // serde_json::to_string(&config) with config = None
-            wok &= ordered_parallel_write(f, ent.size(), [&](std::string& o, size_t i) {
-                d.object(o, ent[i].query, ent[i].part, ent[i].rec, run_id.c_str(), false, 0);
-                o.push_back('\n');
-            });
-        } else {
-            // serde_yaml 0.9 block style of BlutilsOutput{results, config}
-            const HostTaxonomy& T = *r->tax;
-            put(ent.empty() ? "results: []\n" : "results:\n");
-            wok &= ordered_parallel_write(f, ent.size(), [&](std::string& o, size_t i) {
-                const Entry& en = ent[i];
-                std::string tmp;
-                o += "- runId: ";
-                yaml_str(o, run_id);
-                o += "\n  query: ";
-                yaml_str(o, en.query);
-                if (!en.rec) {
-                    o += "\n  taxon: null\n";
-                    return;
-                }
-                const blu_record& rc = *en.rec;
-                const uint32_t lo = T.lin_off[rc.ref_lineage];
-                o += "\n  taxon:\n    reachedRank: ";
-                yaml_str(o, T.ranks[T.pos_rank[lo + rc.reached_pos]].full);
-                o += "\n    maxAllowedRank: ";
-                if (rc.allowed_pos < 0)
-                    o += "null";
-                else {
-                    const RankInfo& ri = T.ranks[T.pos_rank[lo + rc.allowed_pos]];
-                    yaml_str(o, d.in_bb[T.pos_rank[lo + rc.allowed_pos]] ? ri.full : ri.display);
-                }
-                o += "\n    identifier: ";
-                yaml_str(o, T.idents[T.pos_ident[lo + rc.reached_pos]]);
-                o += "\n    percIdentity: ";
-                yaml_f64(o, rc.perc_identity);
-                o += "\n    bitScore: ";
-                yaml_f64(o, (double)rc.bit_score);
-                o += "\n    taxonomy: ";
-                {
-                    bool first = true;
-                    for (int j = 0; j < T.lin_len(rc.ref_lineage); j++)
-                        if (rc.keep_mask >> j & 1) {
-                            if (!first) tmp.push_back(';');
-                            first = false;
-                            T.append_bean(tmp, lo + j);
-                        }
-                }
-                yaml_str(o, tmp);
-                o += rc.mutated ? "\n    mutated: true" : "\n    mutated: false";
-                o += rc.single_match ? "\n    singleMatch: true" : "\n    singleMatch: false";
-                if (!rc.n_beans)
-                    o += "\n    consensusBeans: []\n";
-                else
-                    o += "\n    consensusBeans:\n";
-                for (uint32_t b = 0; b < rc.n_beans; b++) {
-                    const blu_bean& bn = en.part->beans[rc.bean_base + b];
-                    const uint32_t bp = T.lin_off[bn.first_lineage] + rc.bean_level;
-                    o += "    - rank: ";
-                    yaml_str(o, T.ranks[T.pos_rank[bp]].full);
-                    o += "\n      identifier: ";
-                    yaml_str(o, T.idents[T.pos_ident[bp]]);
-                    o += "\n      occurrences: " + std::to_string(bn.occurrences);
-                    o += "\n      taxonomy: ";
-                    tmp.clear();
-                    T.append_lineage(tmp, bn.first_lineage);
-                    yaml_str(o, tmp);
-                    if (!bn.n_acc)
-                        o += "\n      accessions: []\n";
-                    else
-                        o += "\n      accessions:\n";
-                    for (uint32_t a = 0; a < bn.n_acc; a++) {
-                        const blu_acc& ac = en.part->accs[rc.acc_base + bn.acc_begin + a];
-                        o += "      - ";
-                        yaml_str(o, std::string_view(en.part->pool + BLU_ACC_OFF(ac), BLU_ACC_LEN(ac)));
-                        o.push_back('\n');
-                    }
-                }
-            });
-            put("config: null\n");
-        }
-        if (path)
-            wok &= fclose(f) == 0;
-        else
-            fflush(stdout);
-        return wok ? BLU_OK : BLU_ERR_IO;
+        f = fopen(target.c_str(), "wb");
+        if (!f) return BLU_ERR_IO;
     }
+    const bool pretty = format == BLU_FORMAT_JSON && path != nullptr;  // to_string_pretty to a file, compact to stdout
+    bool wok = true;
+    auto put = [&](const char* t) { fwrite(t, 1, strlen(t), f); };
+    if (format == BLU_FORMAT_JSON) {
+        put(pretty ? "{\n  \"results\": [" : "{\"results\":[");
+        wok &= ordered_parallel_write(f, ent.size(), [&](std::string& o, size_t i) {
+            if (i) o.push_back(',');
+            if (pretty) o += "\n    ";
+            d.object(o, ent[i].query, ent[i].part, ent[i].rec, run_id.c_str(), pretty, 2);
+        });
+        if (pretty)
+            put(ent.empty() ? "],\n  \"config\": null\n}" : "\n  ],\n  \"config\": null\n}");
+        else
+            put("],\"config\":null}");
+    } else if (format == BLU_FORMAT_JSONL) {
+        put("null\n");  // serde_json::to_string(&config) with config = None
+        wok &= ordered_parallel_write(f, ent.size(), [&](std::string& o, size_t i) {
+            d.object(o, ent[i].query, ent[i].part, ent[i].rec, run_id.c_str(), false, 0);
+            o.push_back('\n');
+        });
+    } else {
+        // serde_yaml 0.9 block style of BlutilsOutput{results, config}
+        put(ent.empty() ? "results: []\n" : "results:\n");
+        wok &= ordered_parallel_write(f, ent.size(), [&](std::string& o, size_t i) { d.yaml_object(o, ent[i].query, ent[i].part, ent[i].rec, run_id); });
+        put("config: null\n");
+    }
+    if (path)
+        wok &= fclose(f) == 0;
+    else
+        fflush(stdout);
+    return wok ? BLU_OK : BLU_ERR_IO;
 }
 
 
-// parse_consensus_as_tabular (reference core/src/use_cases/parse_consensus_as_tabular/mod.rs:15-173), emitted
-// straight from the binary records instead of re-reading the JSON.  Byte-exact quirks kept:
+// ---------------------------------------------------------------------------------------------------------------
+// build-tabular: the 12-column TSV of parse_consensus_as_tabular (reference core/src/use_cases/parse_consensus_as_tabular/
+// mod.rs:15-173), for the records (view_write_tabular) and for a result file (result_file_to_tabular, blu_tabular.h).
+// Byte-exact quirks kept:
 //   * to stdout every piece goes through println! (one '\n' each), so a query without taxon, whose piece already ends
 //     in '\n', is followed by an empty line;
 //   * to a file the pieces are written as they are -- the reference never adds the line breaks there (mod.rs:58-66 +
 //     shared/write_file_or_stdout.rs), so only the taxon-less pieces end a line;
 //   * floats use Rust's Display (845.0 -> "845").
+// The header and every piece after it are followed by tsv_end_piece.
+// ---------------------------------------------------------------------------------------------------------------
+inline void tsv_end_piece(std::string& o, bool to_stdout) {
+    if (to_stdout) o.push_back('\n');
+}
+
+inline void tsv_header(std::string& o) {
+    o += "run-id\tquery\ttype\trank\tidentifier\tperc-identity\tbit-score\ttaxonomy\tmutated\tsingle-match\toccurrences\taccessions";
+}
+
+// a query without taxon: no run id, no other column
+inline void tsv_no_taxon(std::string& o, std::string_view query) {
+    o.append(query);
+    o += "\tnull\n";
+}
+
+inline void tsv_consensus(std::string& o, std::string_view run_id, std::string_view query, std::string_view rank, std::string_view identifier,
+                          double perc_identity, double bit_score, std::string_view taxonomy, bool mutated, bool single_match) {
+    o.append(run_id);
+    o.push_back('\t');
+    o.append(query);
+    o += "\tconsensus\t";
+    o.append(rank);
+    o.push_back('\t');
+    o.append(identifier);
+    o.push_back('\t');
+    rust_display_f64(o, perc_identity);
+    o.push_back('\t');
+    rust_display_f64(o, bit_score);
+    o.push_back('\t');
+    o.append(taxonomy);
+    o += mutated ? "\ttrue" : "\tfalse";
+    o += single_match ? "\ttrue" : "\tfalse";
+    o += "\tnull\tnull";
+}
+
+// one consensus bean, up to the accessions column; the caller then appends every accession with tsv_accession.  bit_score is
+// the taxon's.
+inline void tsv_blast_match(std::string& o, std::string_view run_id, std::string_view query, std::string_view rank, std::string_view identifier,
+                            double bit_score, std::string_view taxonomy, int64_t occurrences) {
+    o.append(run_id);
+    o.push_back('\t');
+    o.append(query);
+    o += "\tblast-match\t";
+    o.append(rank);
+    o.push_back('\t');
+    o.append(identifier);
+    o += "\tnull\t";
+    rust_display_f64(o, bit_score);
+    o.push_back('\t');
+    o.append(taxonomy);
+    o += "\tnull\tnull\t";
+    o += std::to_string(occurrences);
+    o.push_back('\t');
+}
+
+inline void tsv_accession(std::string& o, size_t i, std::string_view accession) {
+    if (i) o += ", ";
+    o.append(accession);
+}
+
+// The TSV straight from the binary records instead of re-reading the JSON.
 inline int view_write_tabular(const ResultView* r, const char* path, const char* run_id_in) {
     Decoder d(r);
-    const HostTaxonomy& T = *r->tax;
     auto ent = sorted_entries(r);
     const std::string run_id = run_id_in ? std::string(run_id_in) : uuid_v4();
     const bool to_stdout = path == nullptr;
     FILE* f = stdout;
     if (path) {
-        std::string target = path;
-        size_t slash = target.find_last_of('/');
-        size_t dot = target.find_last_of('.');
-        if (dot != std::string::npos && (slash == std::string::npos || dot > slash)) target.resize(dot);
-        target += ".tsv";
+        const std::string target = with_extension(path, ".tsv");
         std::remove(target.c_str());
         f = fopen(target.c_str(), "wb");  // (the reference appends to a file it has just removed; pwrite needs a non-append descriptor)
         if (!f) return BLU_ERR_IO;
     }
     {
-        std::string h = "run-id\tquery\ttype\trank\tidentifier\tperc-identity\tbit-score\ttaxonomy\tmutated\tsingle-match\toccurrences\taccessions";
-        if (to_stdout) h.push_back('\n');
+        std::string h;
+        tsv_header(h);
+        tsv_end_piece(h, to_stdout);
         fwrite(h.data(), 1, h.size(), f);
     }
     const bool ok = ordered_parallel_write(f, ent.size(), [&](std::string& o, size_t ei) {
         const Entry& en = ent[ei];
-        auto piece_done = [&]() {
-            if (to_stdout) o.push_back('\n');
-        };
         if (!en.rec) {
-            o.append(en.query);
-            o += "\tnull\n";
-            piece_done();
+            tsv_no_taxon(o, en.query);
+            tsv_end_piece(o, to_stdout);
             return;
         }
         const blu_record& rc = *en.rec;
-        const uint32_t lo = T.lin_off[rc.ref_lineage];
-        o += run_id;
-        o.push_back('\t');
-        o.append(en.query);
-        o += "\tconsensus\t";
-        o += T.ranks[T.pos_rank[lo + rc.reached_pos]].full;
-        o.push_back('\t');
-        o += T.idents[T.pos_ident[lo + rc.reached_pos]];
-        o.push_back('\t');
-        rust_display_f64(o, rc.perc_identity);
-        o.push_back('\t');
-        rust_display_f64(o, (double)rc.bit_score);
-        o.push_back('\t');
-        {
-            bool first = true;
-            for (int j = 0; j < T.lin_len(rc.ref_lineage); j++)
-                if (rc.keep_mask >> j & 1) {
-                    if (!first) o.push_back(';');
-                    first = false;
-                    T.append_bean(o, lo + j);
-                }
-        }
-        o += rc.mutated ? "\ttrue" : "\tfalse";
-        o += rc.single_match ? "\ttrue" : "\tfalse";
-        o += "\tnull\tnull";
-        piece_done();
+        std::string& s = scratch();
+        d.append_taxonomy(s, rc);
+        tsv_consensus(o, run_id, en.query, d.reached_rank(rc), d.identifier(rc), rc.perc_identity, (double)rc.bit_score, s, rc.mutated, rc.single_match);
+        tsv_end_piece(o, to_stdout);
         for (uint32_t b = 0; b < rc.n_beans; b++) {
-            const blu_bean& bn = en.part->beans[rc.bean_base + b];
-            const uint32_t bp = T.lin_off[bn.first_lineage] + rc.bean_level;
-            o += run_id;
-            o.push_back('\t');
-            o.append(en.query);
-            o += "\tblast-match\t";
-            o += T.ranks[T.pos_rank[bp]].full;
-            o.push_back('\t');
-            o += T.idents[T.pos_ident[bp]];
-            o += "\tnull\t";
-            rust_display_f64(o, (double)rc.bit_score);
-            o.push_back('\t');
-            T.append_lineage(o, bn.first_lineage);
-            o += "\tnull\tnull\t";
-            o += std::to_string(bn.occurrences);
-            o.push_back('\t');
-            for (uint32_t a = 0; a < bn.n_acc; a++) {
-                const blu_acc& ac = en.part->accs[rc.acc_base + bn.acc_begin + a];
-                if (a) o += ", ";
-                o.append(en.part->pool + BLU_ACC_OFF(ac), BLU_ACC_LEN(ac));
-            }
-            piece_done();
+            const blu_bean& bn = d.bean(*en.part, rc, b);
+            s.clear();
+            d.append_lineage(s, bn);
+            tsv_blast_match(o, run_id, en.query, d.bean_rank(rc, bn), d.bean_identifier(rc, bn), (double)rc.bit_score, s, d.occurrences(bn));
+            for (uint32_t a = 0; a < bn.n_acc; a++) tsv_accession(o, a, d.accession(*en.part, rc, bn, a));
+            tsv_end_piece(o, to_stdout);
         }
     });
     if (path)

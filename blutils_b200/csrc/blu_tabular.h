@@ -51,6 +51,15 @@ struct TabResult {  // QueryWithConsensus, consensus_result.rs:7-13
 
 namespace tabular_detail {
 
+// PathBuf::set_extension: the extension starts at the last '.' of the file name, unless that dot begins the name
+inline std::string set_extension(const char* path, const char* ext) {
+    std::string p = path;
+    const size_t slash = p.find_last_of('/');
+    const size_t dot = p.find_last_of('.');
+    if (dot != std::string::npos && dot > (slash == std::string::npos ? 0 : slash + 1)) p.resize(dot);
+    return p + ext;
+}
+
 // uuid::Uuid from a string (hyphenated, simple, braced or urn form) -> its Display form (hyphenated, lower case)
 inline std::string parse_uuid(JsonCursor& c, const std::string& s) {
     std::string_view v(s);
@@ -363,12 +372,7 @@ inline int result_file_to_tabular(const char* in_path, const char* out_path, int
     if (from_stdin)
         buf.assign(std::istreambuf_iterator<char>(std::cin), std::istreambuf_iterator<char>());
     else {
-        std::string probe = in_path;  // PathBuf::set_extension("json")
-        const size_t slash = probe.find_last_of('/');
-        const size_t dot = probe.find_last_of('.');
-        if (dot != std::string::npos && dot > (slash == std::string::npos ? 0 : slash + 1)) probe.resize(dot);
-        probe += ".json";
-        if (!std::ifstream(probe).good()) {
+        if (!std::ifstream(set_extension(in_path, ".json")).good()) {
             err = std::string("The file `") + in_path + "` does not exist.";
             return BLU_ERR_IO;
         }
@@ -465,11 +469,7 @@ inline int result_file_to_tabular(const char* in_path, const char* out_path, int
     const bool to_stdout = out_path == nullptr;
     FILE* f = stdout;
     if (out_path) {
-        std::string target = out_path;  // set_extension("tsv"), remove an existing file, append (mod.rs:54-66)
-        const size_t slash = target.find_last_of('/');
-        const size_t dot = target.find_last_of('.');
-        if (dot != std::string::npos && dot > (slash == std::string::npos ? 0 : slash + 1)) target.resize(dot);
-        target += ".tsv";
+        const std::string target = set_extension(out_path, ".tsv");  // remove an existing file, append (mod.rs:54-66)
         std::remove(target.c_str());
         f = fopen(target.c_str(), "ab");
         if (!f) {
@@ -479,45 +479,28 @@ inline int result_file_to_tabular(const char* in_path, const char* out_path, int
     }
     std::string o;
     auto piece_done = [&]() {
-        if (to_stdout) o.push_back('\n');
+        tsv_end_piece(o, to_stdout);
         if (o.size() > (8u << 20)) {
             fwrite(o.data(), 1, o.size(), f);
             o.clear();
         }
     };
-    o += "run-id\tquery\ttype\trank\tidentifier\tperc-identity\tbit-score\ttaxonomy\tmutated\tsingle-match\toccurrences\taccessions";
+    auto or_null = [](bool has, const std::string& s) { return has ? std::string_view(s) : std::string_view("null"); };
+    tsv_header(o);
     piece_done();
     for (const TabResult& r : results) {
         if (!r.has_taxon) {
-            o += r.query;
-            o += "\tnull\n";
+            tsv_no_taxon(o, r.query);
             piece_done();
             continue;
         }
         const std::string& rid = r.has_run_id ? r.run_id : fallback;
         const TabTaxon& t = r.taxon;
-        o += rid, o += '\t', o += r.query, o += "\tconsensus\t", o += t.reached_rank, o += '\t', o += t.identifier, o += '\t';
-        rust_display_f64(o, t.perc_identity);
-        o += '\t';
-        rust_display_f64(o, t.bit_score);
-        o += '\t';
-        o += t.has_taxonomy ? t.taxonomy : std::string("null");
-        o += t.mutated ? "\ttrue" : "\tfalse";
-        o += t.single_match ? "\ttrue" : "\tfalse";
-        o += "\tnull\tnull";
+        tsv_consensus(o, rid, r.query, t.reached_rank, t.identifier, t.perc_identity, t.bit_score, or_null(t.has_taxonomy, t.taxonomy), t.mutated, t.single_match);
         piece_done();
         for (const TabBean& b : t.beans) {
-            o += rid, o += '\t', o += r.query, o += "\tblast-match\t", o += b.rank, o += '\t', o += b.identifier, o += "\tnull\t";
-            rust_display_f64(o, t.bit_score);
-            o += '\t';
-            o += b.has_taxonomy ? b.taxonomy : std::string("null");
-            o += "\tnull\tnull\t";
-            o += std::to_string(b.occurrences);
-            o += '\t';
-            for (size_t a = 0; a < b.accessions.size(); a++) {
-                if (a) o += ", ";
-                o += b.accessions[a];
-            }
+            tsv_blast_match(o, rid, r.query, b.rank, b.identifier, t.bit_score, or_null(b.has_taxonomy, b.taxonomy), b.occurrences);
+            for (size_t a = 0; a < b.accessions.size(); a++) tsv_accession(o, a, b.accessions[a]);
             piece_done();
         }
     }

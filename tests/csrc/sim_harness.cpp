@@ -253,14 +253,33 @@ extern "C" int blu_sim_run(const int64_t* taxids, const uint64_t* off, const cha
 }
 
 // Same, the result written by the product's writers (blu_decode.h): format 0 / 1 / 2 = JSON / JSONL / YAML (write_blutils_output.rs),
-// 3 = the build-tabular TSV; path NULL = stdout.
+// 3 = the build-tabular TSV; path NULL = stdout.  sorted: the records in query-id order, as blu_result_sort_by_query leaves them.
+// two_parts: the records split into two parts that share the bean, accession and string arrays, as a multi-device result
+// (the second half first unless sorted).
 extern "C" int blu_sim_run_write(const int64_t* taxids, const uint64_t* off, const char* blob, uint64_t n, int taxon, int has_custom,
-                                 const int32_t* custom8, int strategy, const char* text, uint64_t nbytes, const char* out_path, int format,
-                                 const char* run_id, char* err, int errlen) {
+                                 const int32_t* custom8, int strategy, const char* text, uint64_t nbytes, const char* headers_nl, uint64_t headers_len,
+                                 int sorted, int two_parts, const char* out_path, int format, const char* run_id, char* err, int errlen) {
     int wrc = 0;
-    const int rc = sim_run_impl(taxids, off, blob, n, taxon, has_custom, custom8, strategy, text, nbytes, nullptr, 0,
-                                [&](const ResultView& v) { wrc = format == 3 ? view_write_tabular(&v, out_path, run_id) : view_write(&v, out_path, format, run_id); },
-                                err, errlen);
+    auto write = [&](const ResultView& v0) {
+        ResultView v = v0;
+        const ResultPart& p = v0.parts[0];
+        std::vector<blu_record> recs(p.rec, p.rec + p.n_rec);
+        if (sorted) {
+            std::stable_sort(recs.begin(), recs.end(), [&](const blu_record& a, const blu_record& b) { return rec_query(p, a) < rec_query(p, b); });
+            v.sorted = true;
+        }
+        ResultPart lo = p, hi = p;
+        lo.rec = recs.data();
+        if (two_parts) {
+            lo.n_rec = p.n_rec / 2;
+            hi.rec = recs.data() + lo.n_rec;
+            hi.n_rec = p.n_rec - lo.n_rec;
+            v.parts = sorted ? std::vector<ResultPart>{lo, hi} : std::vector<ResultPart>{hi, lo};
+        } else
+            v.parts = {lo};
+        wrc = format == 3 ? view_write_tabular(&v, out_path, run_id) : view_write(&v, out_path, format, run_id);
+    };
+    const int rc = sim_run_impl(taxids, off, blob, n, taxon, has_custom, custom8, strategy, text, nbytes, headers_nl, headers_len, write, err, errlen);
     if (rc == BLU_OK && wrc != 0) {
         snprintf(err, errlen, "writer failed (%d)", wrc);
         return wrc;

@@ -77,9 +77,11 @@ def run(taxids: Sequence[int], lineages: Sequence[str], taxon: str, strategy: st
         lib().blu_sim_free(out)
 
 
-def run_write(taxids: Sequence[int], lineages: Sequence[str], taxon: str, strategy: str, text: bytes, out_path: str, fmt: str, run_id: str,
-              custom=None) -> int:
-    """The same run, written by the product's writers: fmt json (pretty, to a file) / jsonl / yaml / tsv.  Returns rc."""
+def run_write(taxids: Sequence[int], lineages: Sequence[str], taxon: str, strategy: str, text: bytes, out_path: Optional[str], fmt: str, run_id: str,
+              custom=None, headers: Optional[List[str]] = None, sorted_records: bool = False, two_parts: bool = False) -> int:
+    """The same run, written by the product's writers: fmt json (pretty to a file, compact to stdout) / jsonl / yaml / tsv;
+    out_path None = stdout.  sorted_records: records in query-id order (a sorted result); two_parts: the records as two parts (a
+    multi-device result).  Returns rc."""
     enc = [s.encode() for s in lineages]
     off = np.zeros(len(enc) + 1, dtype=np.uint64)
     if enc:
@@ -87,13 +89,14 @@ def run_write(taxids: Sequence[int], lineages: Sequence[str], taxon: str, strate
     ids = np.asarray(list(taxids), dtype=np.int64)
     c8 = _c8(custom)
     err = C.create_string_buffer(512)
+    hb = "\n".join(headers).encode() if headers else None
     f = lib().blu_sim_run_write
     f.restype = C.c_int
-    f.argtypes = [C.c_void_p, C.c_void_p, C.c_char_p, C.c_uint64, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_char_p, C.c_uint64, C.c_char_p, C.c_int, C.c_char_p,
-                  C.c_char_p, C.c_int]
+    f.argtypes = [C.c_void_p, C.c_void_p, C.c_char_p, C.c_uint64, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_char_p, C.c_uint64, C.c_char_p, C.c_uint64,
+                  C.c_int, C.c_int, C.c_char_p, C.c_int, C.c_char_p, C.c_char_p, C.c_int]
     return f(ids.ctypes.data, off.ctypes.data, b"".join(enc), len(enc), TAXON[taxon], 1 if c8 is not None else 0,
-             C.cast(c8, C.c_void_p) if c8 is not None else None, STRATEGY[strategy], text, len(text), out_path.encode(),
-             {"json": 0, "jsonl": 1, "yaml": 2, "tsv": 3}[fmt], run_id.encode(), err, 512)
+             C.cast(c8, C.c_void_p) if c8 is not None else None, STRATEGY[strategy], text, len(text), hb, len(hb) if hb else 0, int(sorted_records),
+             int(two_parts), None if out_path is None else out_path.encode(), {"json": 0, "jsonl": 1, "yaml": 2, "tsv": 3}[fmt], run_id.encode(), err, 512)
 
 
 def interpolate(ranks: Sequence[str], taxon: str, custom=None) -> List[float]:

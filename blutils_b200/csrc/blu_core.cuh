@@ -930,9 +930,111 @@ BLU_HD uint32_t heavy_parse_row_masked(const uint8_t* win, const uint64_t* tabw,
     return DE_NONE;
 }
 
+// ---- record stages ----------------------------------------------------------------------------------------------
+// A record starts as record_header() (no consensus, no beans).  The tile kernel turns it into a pending record for the
+// consensus kernel; write_outcome() then sets what the consensus decided.  The host only ever sees status 0 and 1.
+constexpr uint8_t kStatusNoConsensus = 0;  // NoConsensusFound: a hit-less header, or a query whose consensus failed
+constexpr uint8_t kStatusFound = 1;        // ConsensusFound
+constexpr uint8_t kStatusPending = 2;      // waiting for the consensus kernel (device only)
+
+BLU_HD blu_record record_header(uint64_t query_off, uint32_t query_len, uint32_t n_rows, int64_t bit_score) {
+    blu_record r;
+    r.query_off = query_off;
+    r.query_len = query_len;
+    r.n_rows = n_rows;
+    r.keep_mask = 0;
+    r.perc_identity = 0.0;
+    r.bit_score = bit_score;
+    r.ref_lineage = 0;
+    r.bean_base = 0;
+    r.n_beans = 0;
+    r.acc_base = 0;
+    r.status = kStatusNoConsensus;
+    r.single_match = 0;
+    r.mutated = 0;
+    r.reached_pos = 0;
+    r.allowed_pos = -1;
+    r.bean_level = 0;
+    r.pad[0] = r.pad[1] = 0;
+    return r;
+}
+
+// Until the consensus kernel has run, a pending record's bean_base / n_beans hold the query's first top-row slot and the
+// size of its top group: only these three functions know that.
+BLU_HD blu_record pending_record(blu_record r, uint32_t slot, uint32_t n_top) {
+    r.status = kStatusPending;
+    r.bean_base = slot;
+    r.n_beans = n_top;
+    return r;
+}
+BLU_HD uint32_t pending_slot(const blu_record& r) { return r.bean_base; }
+BLU_HD uint32_t pending_rows(const blu_record& r) { return r.n_beans; }
+
+// What the consensus decides for a query: every record field but the header and where its beans / accession references
+// went.  Outcome{} is a failure (ok = false).
+struct Outcome {
+    uint64_t keep_mask;   // the cutoff part (cutoff_outcome / apply_cutoffs) ...
+    int reached_pos, allowed_pos;
+    bool mutated;
+    double perc_identity;  // ... and what the top group decided
+    uint32_t ref_lineage, n_beans;
+    int bean_level;
+    bool single_match, ok;
+};
+
+// The cutoff part (build_blast_consensus_identity.rs:22-37,66-95): `keep` = the reference-lineage positions that go into the
+// output taxonomy, `allowed` = maxAllowedRank's position or -1, `idx` = the bean's position, the reached one when nothing is
+// kept (adjusted_taxonomy.last().unwrap_or(_bean)).
+BLU_HD Outcome cutoff_outcome(uint64_t keep, int allowed, int idx, bool mutated) {
+    Outcome o = {};
+    o.keep_mask = keep;
+    o.reached_pos = keep ? 63 - blu_clz64(keep) : idx;
+    o.allowed_pos = allowed;
+    o.mutated = mutated;
+    return o;
+}
+
+// A consensus found: the cutoff part `o` plus the reference row's identity and lineage, the beans and their level.
+BLU_HD Outcome found_outcome(Outcome o, double perc_identity, uint32_t ref_lineage, uint32_t n_beans, int bean_level, bool single_match) {
+    o.perc_identity = perc_identity;
+    o.ref_lineage = ref_lineage;
+    o.n_beans = n_beans;
+    o.bean_level = bean_level;
+    o.single_match = single_match;
+    o.ok = true;
+    return o;
+}
+
+// A single match (find_single_query_consensus.rs:74-150): `keep` = every position whose cutoff the row passes (not empty);
+// one bean at the last of them, no maxAllowedRank.
+BLU_HD Outcome single_outcome(uint64_t keep, double perc_identity, uint32_t ref_lineage) {
+    const Outcome cut = cutoff_outcome(keep, -1, 0, false);
+    return found_outcome(cut, perc_identity, ref_lineage, 1, cut.reached_pos, true);
+}
+
+// The record fields an outcome decides.  A failed query keeps its id (the duplicate-id check must see it) and owns no beans
+// or accession references.
+BLU_HD void write_outcome(blu_record* rec, const Outcome& o) {
+    if (o.ok) {
+        rec->keep_mask = o.keep_mask;
+        rec->perc_identity = o.perc_identity;
+        rec->ref_lineage = o.ref_lineage;
+        rec->n_beans = o.n_beans;
+        rec->single_match = o.single_match ? 1 : 0;
+        rec->mutated = o.mutated ? 1 : 0;
+        rec->reached_pos = (int8_t)o.reached_pos;
+        rec->allowed_pos = (int8_t)o.allowed_pos;
+        rec->bean_level = (int8_t)o.bean_level;
+        rec->status = kStatusFound;
+    } else {
+        rec->bean_base = 0, rec->n_beans = 0, rec->acc_base = 0;
+        rec->status = kStatusNoConsensus;
+    }
+}
+
 // ---- consensus --------------------------------------------------------------------------------------------------
-// Where the per-query output goes.  `beans`/`accs` point at this query's reserved entries (g of each; the caller has
-// stored their indices in rec->bean_base / rec->acc_base).
+// Where the per-query output goes: the record (its header written, bean_base / acc_base set), and its reserved beans /
+// accession references (g of each).  The consensus writes the record through write_outcome().
 struct QueryOut {
     blu_record* rec;
     blu_bean* beans;
@@ -948,8 +1050,8 @@ BLU_HD int bytes_cmp(const uint8_t* a, int la, const uint8_t* b, int lb) {
     return la - lb;
 }
 
-// rank selection for a reference lineage (build_blast_consensus_identity.rs:22-37,66-95)
-BLU_HD void apply_cutoffs(const LinTables& T, uint32_t ref_lin, double identity, bool whole_filter, int idx, blu_record* rec) {
+// the cutoff part of an outcome, by rank selection on a reference lineage (build_blast_consensus_identity.rs:22-37,66-95)
+BLU_HD Outcome apply_cutoffs(const LinTables& T, uint32_t ref_lin, double identity, bool whole_filter, int idx) {
     const uint32_t o = T.lin_off[ref_lin];
     const int k = (int)(T.lin_off[ref_lin + 1] - o);
     int allowed = -1;
@@ -959,19 +1061,13 @@ BLU_HD void apply_cutoffs(const LinTables& T, uint32_t ref_lin, double identity,
             break;
         }
     uint64_t mask = 0;
-    int kept = 0, last = -1;
+    int kept = 0;
     for (int j = 0; j < k; j++)
         if (identity >= T.cut[o + j]) {  // linnaean_ranks.rs:208
-            if (whole_filter || kept <= idx) {  // enumerate AFTER the filter, take_while(index <= bean_index)
-                mask |= 1ULL << j;
-                last = j;
-            }
+            if (whole_filter || kept <= idx) mask |= 1ULL << j;  // enumerate AFTER the filter, take_while(index <= bean_index)
             kept++;
         }
-    rec->keep_mask = mask;
-    rec->allowed_pos = (int8_t)allowed;
-    rec->reached_pos = (int8_t)(last >= 0 ? last : idx);  // adjusted_taxonomy.last().unwrap_or(_bean)
-    rec->mutated = (allowed >= 0 && T.rank_cls[o + idx] != T.allowed_cls[o + allowed]) ? 1 : 0;
+    return cutoff_outcome(mask, allowed, idx, allowed >= 0 && T.rank_cls[o + idx] != T.allowed_cls[o + allowed]);
 }
 
 // |G| == 1 (find_single_query_consensus.rs:74-150)
@@ -985,23 +1081,16 @@ BLU_HD uint32_t consensus_single(const TopRow& r, const LinTables& T, QueryOut o
             mask |= 1ULL << j;
             last = j;
         }
-    if (last < 0) return DE_EMPTY_ADJUSTED;
-    blu_record* rec = out.rec;
-    rec->keep_mask = mask;
-    rec->perc_identity = r.pident;
-    rec->ref_lineage = r.lin;
-    rec->n_beans = 1;
-    rec->status = 1;
-    rec->single_match = 1;
-    rec->mutated = 0;
-    rec->reached_pos = (int8_t)last;
-    rec->allowed_pos = -1;
-    rec->bean_level = (int8_t)last;
+    if (last < 0) {
+        write_outcome(out.rec, Outcome{});
+        return DE_EMPTY_ADJUSTED;
+    }
     out.beans[0].first_lineage = r.lin;
     out.beans[0].occurrences = 1;
     out.beans[0].acc_begin = 0;
     out.beans[0].n_acc = 1;
     out.accs[0].ref = (r.acc_off << 16) | (uint64_t)r.acc_len;
+    write_outcome(out.rec, single_outcome(mask, r.pident, r.lin));
     return DE_NONE;
 }
 
@@ -1084,7 +1173,10 @@ BLU_HD_NOINLINE uint32_t consensus_multi(const TopRow* rows, int g, const uint8_
     int idx, level;
     bool single;
     double identity;
-    if (diverge == 0) return DE_ROOT_DISAGREE;
+    if (diverge == 0) {
+        write_outcome(out.rec, Outcome{});
+        return DE_ROOT_DISAGREE;
+    }
     if (diverge > 0) {
         for (int r = 0; r < g; r++)
             if (rows[r].pident > max_pident) max_pident = rows[r].pident;  // fold from 0.0 (fmtc.rs:182-185)
@@ -1162,14 +1254,7 @@ BLU_HD_NOINLINE uint32_t consensus_multi(const TopRow* rows, int g, const uint8_
         out.beans[bi].acc_begin = begin;
         out.beans[bi].n_acc = na - begin;
     }
-    blu_record* rec = out.rec;
-    rec->perc_identity = ref.pident;
-    rec->ref_lineage = ref.lin;
-    rec->n_beans = (uint32_t)nb;
-    rec->status = 1;
-    rec->single_match = 0;
-    rec->bean_level = (int8_t)level;
-    apply_cutoffs(T, ref.lin, identity, single && nb == 1, idx, rec);
+    write_outcome(out.rec, found_outcome(apply_cutoffs(T, ref.lin, identity, single && nb == 1, idx), ref.pident, ref.lin, (uint32_t)nb, level, false));
     return DE_NONE;
 }
 

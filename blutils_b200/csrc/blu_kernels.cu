@@ -83,6 +83,17 @@ __device__ __forceinline__ void report_soft(Counters* ctr, uint32_t err, unsigne
     if (atomicCAS(&ctr->soft_code, 0u, err) == 0u) ctr->soft_off = off;
 }
 
+// Reserves n entries of an output array of `cap` entries through its cursor in Counters: `base` = the first one.  false: they
+// do not fit -- cap_overflow is set and nothing may be written there; the cursor still counts them, so that the host can size
+// the arrays for the run it starts over.
+template <class C>
+__device__ __forceinline__ bool reserve(Counters* ctr, C Counters::*cursor, unsigned long long n, unsigned long long cap, C& base) {
+    base = atomicAdd(&(ctr->*cursor), (C)n);
+    if ((unsigned long long)base + n <= cap) return true;
+    ctr->cap_overflow = 1;
+    return false;
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 // shared-memory window + row index (used by both kernels)
 // ---------------------------------------------------------------------------------------------------------------
@@ -446,11 +457,8 @@ struct StreamSmem {
 static_assert((sizeof(StreamSmem) + 1024) * kTileCtasPerSm <= 227 * 1024, "tile CTAs must fit one SM");
 
 __device__ __forceinline__ void push_defer(const RunParams& p, unsigned long long off, unsigned check_prev) {
-    unsigned i = atomicAdd(&p.ctr->n_defer, 1u);
-    if (i < p.defer_cap)
-        p.defer[i] = (off << 1) | check_prev;
-    else
-        p.ctr->cap_overflow = 1;
+    unsigned i;
+    if (reserve(p.ctr, &Counters::n_defer, 1, p.defer_cap, i)) p.defer[i] = (off << 1) | check_prev;
 }
 
 __device__ __forceinline__ void stream_issue_load(StreamSmem& S, int buf, const uint8_t* text, unsigned long long lo, int bytes) {
@@ -632,25 +640,7 @@ __device__ __forceinline__ void drain_topq(const RunParams& p, StreamSmem& S, co
 }
 
 __device__ __forceinline__ void write_record(blu_record* dst, const StagedRec& sr) {
-    blu_record rec;
-    rec.query_off = sr.abs;
-    rec.query_len = sr.qlen;
-    rec.n_rows = sr.nrows;
-    rec.keep_mask = 0;
-    rec.perc_identity = 0.0;
-    rec.bit_score = (int64_t)sr.mx;
-    rec.ref_lineage = 0;
-    rec.bean_base = sr.slot;     // first top-row slot / size of the top group until the consensus kernel has run
-    rec.n_beans = sr.gtot;
-    rec.acc_base = 0;
-    rec.status = 2;              // waiting for the consensus kernel
-    rec.single_match = 0;
-    rec.mutated = 0;
-    rec.reached_pos = 0;
-    rec.allowed_pos = -1;
-    rec.bean_level = 0;
-    rec.pad[0] = rec.pad[1] = 0;
-    *dst = rec;
+    *dst = pending_record(record_header(sr.abs, sr.qlen, sr.nrows, (int64_t)sr.mx), sr.slot, sr.gtot);
 }
 
 // Flushes the buffered record headers: ONE global atomic reserves their (dense) place in the record array, then every
@@ -658,14 +648,7 @@ __device__ __forceinline__ void write_record(blu_record* dst, const StagedRec& s
 __device__ __forceinline__ void flush_records(const RunParams& p, StreamSmem& S, int tid) {
     const int n = S.rec_cnt < kRecBuf ? S.rec_cnt : kRecBuf;
     if (n == 0) return;
-    if (tid == 0) {
-        const unsigned long long rec_base = atomicAdd(&p.ctr->rec_count, (unsigned long long)n);
-        S.rec_base = rec_base;
-        if (rec_base + (unsigned long long)n > p.rec_cap) {
-            S.out_ok = 0;
-            p.ctr->cap_overflow = 1;
-        }
-    }
+    if (tid == 0 && !reserve(p.ctr, &Counters::rec_count, n, p.rec_cap, S.rec_base)) S.out_ok = 0;
     __syncthreads();
     if (S.out_ok) {
         const unsigned long long rec_base = S.rec_base;
@@ -738,16 +721,12 @@ __device__ __forceinline__ void tile_segment(const RunParams& p, StreamSmem& S, 
             // the CTA's first slab of top-row slots (about 40 per window of the segment, at most kSlotSlab)
             const unsigned long long est = ((seg_hi - seg_lo) / (unsigned long long)kTile + 1ull) * 40ull + (unsigned long long)kSlotLow;
             const uint32_t slab = est < (unsigned long long)kSlotSlab ? (uint32_t)est : kSlotSlab;
-            const unsigned long long rs = atomicAdd(&p.ctr->slot_count, (unsigned long long)slab);
+            unsigned long long rs;
+            S.out_ok = reserve(p.ctr, &Counters::slot_count, slab, p.slot_cap, rs) ? 1 : 0;  // (slot_cap < 2^32: slot numbers fit the 32-bit fields)
             S.slot_cur = (uint32_t)rs;
             S.slot_end = (uint32_t)rs + slab;
             S.slots_taken = slab;
             S.rec_cnt = 0;
-            S.out_ok = 1;
-            if (rs + (unsigned long long)slab > p.slot_cap) {  // (slot_cap < 2^32: slot numbers fit the 32-bit fields)
-                S.out_ok = 0;
-                p.ctr->cap_overflow = 1;
-            }
         }
     }
     for (int i = tid; i < 7; i += kTileThreads) S.tabm[kUnits + i] = S.digm[kUnits + i] = S.nlm[kUnits + i] = 0u;
@@ -1132,12 +1111,9 @@ __device__ __forceinline__ void tile_segment(const RunParams& p, StreamSmem& S, 
                     if (g_tot > 0) {
                         slot = atoms_add(&S.slot_cur, (uint32_t)g_tot);
                         if (slot + (uint32_t)g_tot > S.slot_end || slot + (uint32_t)g_tot < slot) {
-                            const unsigned long long rs = atomicAdd(&p.ctr->slot_count, (unsigned long long)g_tot);
+                            unsigned long long rs;
+                            if (!reserve(p.ctr, &Counters::slot_count, g_tot, p.slot_cap, rs)) S.out_ok = 0;
                             slot = (uint32_t)rs;
-                            if (rs + (unsigned long long)g_tot > p.slot_cap) {
-                                S.out_ok = 0;
-                                p.ctr->cap_overflow = 1;
-                            }
                         }
                     }
                     StagedRec sr;
@@ -1147,11 +1123,8 @@ __device__ __forceinline__ void tile_segment(const RunParams& p, StreamSmem& S, 
                         S.rec_buf[ri] = sr;
                     else {
                         // record buffer full (a window of very short queries): this record is reserved on its own
-                        const unsigned long long ri2 = atomicAdd(&p.ctr->rec_count, 1ull);
-                        if (ri2 < p.rec_cap)
-                            write_record(p.records + ri2, sr);
-                        else
-                            p.ctr->cap_overflow = 1;
+                        unsigned long long ri2;
+                        if (reserve(p.ctr, &Counters::rec_count, 1, p.rec_cap, ri2)) write_record(p.records + ri2, sr);
                     }
                 }
                 if (kind & RK_DEFER) push_defer(p, abs, 0);
@@ -1231,13 +1204,10 @@ __device__ __forceinline__ void tile_segment(const RunParams& p, StreamSmem& S, 
                 const unsigned long long est = (unsigned long long)(S.slots_taken / (uint32_t)win_idx + 8u) * left + (unsigned long long)kSlotLow;
                 const uint32_t slab = est < (unsigned long long)kSlotSlab ? (uint32_t)est : kSlotSlab;
                 S.slots_taken += slab;
-                const unsigned long long rs = atomicAdd(&p.ctr->slot_count, (unsigned long long)slab);
+                unsigned long long rs;
+                if (!reserve(p.ctr, &Counters::slot_count, slab, p.slot_cap, rs)) S.out_ok = 0;
                 S.slot_cur = (uint32_t)rs;
                 S.slot_end = (uint32_t)rs + slab;
-                if (rs + (unsigned long long)slab > p.slot_cap) {
-                    S.out_ok = 0;
-                    p.ctr->cap_overflow = 1;
-                }
             }
         }
         if (need_flush) flush_records(p, S, tid);
@@ -1627,14 +1597,10 @@ __device__ uint32_t long_consensus(LongSmem& S, const RunParams& p, const TopRow
     for (int j = tid; j < nb; j += kLongThreads) Q.abeg[Q.bsort[j]] = Q.tmp[j];
     // ---- output: one record, nb beans, nkept accession references, all compact --------------------------------------------
     if (tid == 0) {
-        const unsigned long long ri = atomicAdd(&p.ctr->rec_count, 1ull);
-        const unsigned long long bb = atomicAdd(&p.ctr->bean_used, (unsigned long long)nb);
-        const unsigned long long ab = atomicAdd(&p.ctr->acc_used, (unsigned long long)nkept);
-        S.bcast64[1] = ri, S.bcast64[2] = bb, S.bcast64[3] = ab;
-        if (ri >= p.rec_cap || bb + (unsigned long long)nb > p.bean_cap || ab + (unsigned long long)nkept > p.acc_cap) {
-            p.ctr->cap_overflow = 1;
-            S.bcast64[1] = ~0ull;
-        }
+        unsigned long long ri, bb, ab;
+        const bool fits = reserve(p.ctr, &Counters::rec_count, 1, p.rec_cap, ri) & reserve(p.ctr, &Counters::bean_used, nb, p.bean_cap, bb) &
+                          reserve(p.ctr, &Counters::acc_used, nkept, p.acc_cap, ab);
+        S.bcast64[1] = fits ? ri : ~0ull, S.bcast64[2] = bb, S.bcast64[3] = ab;
     }
     __syncthreads();
     if (S.bcast64[1] == ~0ull) return DE_NONE;  // the host grows the arrays and reruns
@@ -1656,20 +1622,9 @@ __device__ uint32_t long_consensus(LongSmem& S, const RunParams& p, const TopRow
         }
     if (tid == 0) {
         blu_record* rec = p.records + ri;
-        rec->query_off = s;
-        rec->query_len = qlen;
-        rec->n_rows = (uint32_t)nrows;
-        rec->bit_score = mx;
-        rec->perc_identity = ref.pident;
-        rec->ref_lineage = ref.lin;
-        rec->bean_base = (uint32_t)bean_base;
-        rec->n_beans = (uint32_t)nb;
-        rec->acc_base = (uint32_t)acc_base;
-        rec->status = 1;
-        rec->single_match = 0;
-        rec->bean_level = (int8_t)level;
-        rec->pad[0] = rec->pad[1] = 0;
-        apply_cutoffs(T, ref.lin, identity, single && nb == 1, idx, rec);
+        *rec = record_header(s, qlen, (uint32_t)nrows, mx);
+        rec->bean_base = (uint32_t)bean_base, rec->acc_base = (uint32_t)acc_base;
+        write_outcome(rec, found_outcome(apply_cutoffs(T, ref.lin, identity, single && nb == 1, idx), ref.pident, ref.lin, (uint32_t)nb, level, false));
     }
     return DE_NONE;
 }
@@ -1845,37 +1800,16 @@ __global__ void __launch_bounds__(kLongThreads, 1) longrun_kernel(const __grid_c
             // a single top row, or a query whose consensus failed: the record is written here.  A failed query still leaves
             // a record (status 0) so that the duplicate-id check sees its id: a fragment of a scattered query may fail
             // although the merged query would not, and then the table is regrouped and run again.
-            const unsigned long long ri = atomicAdd(&p.ctr->rec_count, 1ull);
-            unsigned long long bb = 0, ab = 0;
-            if (!soft) {
-                bb = atomicAdd(&p.ctr->bean_used, 1ull);
-                ab = atomicAdd(&p.ctr->acc_used, 1ull);
-            }
-            if (ri >= p.rec_cap || bb + 1 > p.bean_cap || ab + 1 > p.acc_cap)
-                p.ctr->cap_overflow = 1;
-            else {
+            unsigned long long ri, bb = 0, ab = 0;
+            bool fits = reserve(p.ctr, &Counters::rec_count, 1, p.rec_cap, ri);
+            if (!soft) fits = reserve(p.ctr, &Counters::bean_used, 1, p.bean_cap, bb) & reserve(p.ctr, &Counters::acc_used, 1, p.acc_cap, ab) & fits;
+            if (fits) {
                 blu_record* rec = p.records + ri;
-                rec->query_off = s;
-                rec->query_len = ql;
-                rec->n_rows = (uint32_t)nrows;
-                rec->keep_mask = 0;
-                rec->perc_identity = 0.0;
-                rec->bit_score = mx;
-                rec->ref_lineage = 0;
-                rec->bean_base = (uint32_t)bb;
-                rec->n_beans = 0;
-                rec->acc_base = (uint32_t)ab;
-                rec->status = 0;
-                rec->single_match = rec->mutated = 0;
-                rec->reached_pos = 0, rec->allowed_pos = -1, rec->bean_level = 0;
-                rec->pad[0] = rec->pad[1] = 0;
+                *rec = record_header(s, ql, (uint32_t)nrows, mx);  // (as it stays when the consensus failed)
                 if (!soft) {
-                    QueryOut out{rec, p.beans + bb, p.accs + ab};
-                    const uint32_t ce = consensus_single(rows[0], p.T, out);
-                    if (ce) {
-                        report_soft(p.ctr, ce, s);
-                        rec->status = 0, rec->n_beans = 0;
-                    }
+                    rec->bean_base = (uint32_t)bb, rec->acc_base = (uint32_t)ab;
+                    const uint32_t ce = consensus_single(rows[0], p.T, QueryOut{rec, p.beans + bb, p.accs + ab});
+                    if (ce) report_soft(p.ctr, ce, s);
                 }
             }
         }
@@ -1916,13 +1850,9 @@ constexpr int kConsThreads = 128;
 
 // What a lane holds once its query's consensus is computed; written out after the output space has been reserved.
 struct ConsLane {
-    // lane 0 of the group: the record
-    unsigned long long keep_mask;
-    double perc_identity;
-    uint32_t ref_lineage;
-    int nb, nkept;         // beans / kept accession references of the query (0: the query failed or is not this pass's)
-    int reached, allowed, level;
-    bool mutated, single, ok;
+    // lane 0 of the group: the record (out.ok = false: the query failed or is not this pass's)
+    Outcome out;
+    int nkept;             // kept accession references of the query
     // every lane: its bean (leaders) and its accession reference (kept rows)
     bool leader, keeps;
     blu_bean bean;
@@ -1941,8 +1871,8 @@ __device__ __forceinline__ ConsLane cons_compute(const PostParams& p, bool valid
     auto seg = [&](unsigned b) { return W == 32 ? b : ((b >> gsh) & WM); };
     const unsigned ltm = (1u << sl) - 1u;
     ConsLane o;
-    o.keep_mask = 0, o.perc_identity = 0.0, o.ref_lineage = 0, o.nb = 0, o.nkept = 0, o.reached = 0, o.allowed = -1, o.level = 0;
-    o.mutated = false, o.single = false, o.ok = false, o.leader = false, o.keeps = false, o.bean_idx = 0, o.acc_idx = 0, o.acc_ref = 0;
+    o.out = Outcome{};
+    o.nkept = 0, o.leader = false, o.keeps = false, o.bean_idx = 0, o.acc_idx = 0, o.acc_ref = 0;
     o.bean.first_lineage = 0, o.bean.occurrences = 0, o.bean.acc_begin = 0, o.bean.n_acc = 0;
     const bool on = valid && sl < g;
     // ---- the rows as the tile kernel left them: the join (left_join on subject_taxid == taxid, mod.rs:72-76) ------------
@@ -2151,21 +2081,16 @@ __device__ __forceinline__ ConsLane cons_compute(const PostParams& p, bool valid
         if (sl == 0) report_soft(p.ctr, DE_EMPTY_ADJUSTED, query_off);
         failed = true;
     }
-    o.ok = valid && !failed;
-    if (!o.ok) return o;
+    if (!valid || failed) return o;
     o.leader = leader;
     o.keeps = on && !dropped;
     o.bean.first_lineage = r.lin, o.bean.occurrences = (uint32_t)occ, o.bean.acc_begin = (uint32_t)acc_begin, o.bean.n_acc = (uint32_t)nacc_bean;
     o.bean_idx = brank;
     o.acc_idx = my_begin + my_idx;
     o.acc_ref = (r.acc_off << 16) | (unsigned long long)r.acc_len;
-    o.nb = nb;
     o.nkept = __popc(kept);
-    o.ref_lineage = ref_lin;
-    o.level = level;
     if (g == 1) {
-        const int last = 63 - __clzll((long long)ge);
-        o.keep_mask = ge, o.perc_identity = ref_pid, o.single = true, o.mutated = false, o.reached = last, o.allowed = -1, o.level = last;
+        o.out = single_outcome(ge, ref_pid, ref_lin);
     } else {
         const int allowed = notgt ? (__ffsll((long long)notgt) - 1) : -1;
         unsigned long long mask = ge;
@@ -2179,31 +2104,10 @@ __device__ __forceinline__ ConsLane cons_compute(const PostParams& p, bool valid
             }
             mask = mk;
         }
-        const int last = mask ? 63 - __clzll((long long)mask) : -1;
-        o.keep_mask = mask, o.perc_identity = ref_pid, o.single = false, o.allowed = allowed, o.reached = last >= 0 ? last : idx;
-        o.mutated = sl == 0 && allowed >= 0 && T.rank_cls[ref_o + idx] != T.allowed_cls[ref_o + allowed];
+        const Outcome cut = cutoff_outcome(mask, allowed, idx, sl == 0 && allowed >= 0 && T.rank_cls[ref_o + idx] != T.allowed_cls[ref_o + allowed]);
+        o.out = found_outcome(cut, ref_pid, ref_lin, (uint32_t)nb, level, false);
     }
     return o;
-}
-
-// the record fields the consensus decides (everything but where its beans / accession references end up)
-__device__ __forceinline__ void cons_write_record(blu_record* rec, const ConsLane& o) {
-    if (o.ok) {
-        rec->keep_mask = o.keep_mask;
-        rec->perc_identity = o.perc_identity;
-        rec->ref_lineage = o.ref_lineage;
-        rec->n_beans = (uint32_t)o.nb;
-        rec->single_match = o.single ? 1 : 0;
-        rec->mutated = o.mutated ? 1 : 0;
-        rec->reached_pos = (int8_t)o.reached;
-        rec->allowed_pos = (int8_t)o.allowed;
-        rec->bean_level = (int8_t)o.level;
-        rec->status = 1;
-    } else {
-        // a failed query keeps its id (the duplicate-id check must see it) and owns no beans / accession references
-        rec->bean_base = 0, rec->n_beans = 0, rec->acc_base = 0;
-        rec->status = 0;
-    }
 }
 
 constexpr int kConsWarps = kConsThreads / 32;
@@ -2253,9 +2157,9 @@ __global__ void __launch_bounds__(kConsThreads, BLU_CONS_MINB) consensus_kernel(
         unsigned long long slot = 0, qoff = 0;
         if (qi < re) {
             rows_sum += rec->n_rows;
-            if (rec->status == 2) {
-                g = (int)rec->n_beans;
-                slot = rec->bean_base;
+            if (rec->status == kStatusPending) {
+                g = (int)pending_rows(*rec);
+                slot = pending_slot(*rec);
                 qoff = rec->query_off;
                 if (g >= 1 && slot + (unsigned long long)g <= p.slot_cap) cls = g <= 8 ? 1 : (g <= 32 ? 2 : 3);  // (else: cannot happen without cap_overflow)
             }
@@ -2263,7 +2167,7 @@ __global__ void __launch_bounds__(kConsThreads, BLU_CONS_MINB) consensus_kernel(
         St.nb[lane] = 0, St.na[lane] = 0;
         if (cls == 3) {
             report(p.ctr, DE_INTERNAL, qoff);  // (the tile kernel hands top groups of more than 32 rows to the long-run kernel)
-            rec->status = 0, rec->n_beans = 0;
+            write_outcome(rec, Outcome{});
         }
         // ---- the narrow queries, listed by top-group size ------------------------------------------------------------------------
         int n8 = 0;
@@ -2287,12 +2191,12 @@ __global__ void __launch_bounds__(kConsThreads, BLU_CONS_MINB) consensus_kernel(
             const int gq = __shfl_sync(FULL, g, q);
             const unsigned long long slotq = __shfl_sync(FULL, slot, q), qoffq = __shfl_sync(FULL, qoff, q);
             const ConsLane o = cons_compute<8>(p, valid, gq, slotq, qoffq, lane);
-            if (o.ok && o.leader) St.beans[q][o.bean_idx] = o.bean;
-            if (o.ok && o.keeps) St.accs[q][o.acc_idx] = o.acc_ref;
+            if (o.out.ok && o.leader) St.beans[q][o.bean_idx] = o.bean;
+            if (o.out.ok && o.keeps) St.accs[q][o.acc_idx] = o.acc_ref;
             if (valid && sl8 == 0) {
-                St.nb[q] = o.ok ? o.nb : 0;
-                St.na[q] = o.ok ? o.nkept : 0;
-                cons_write_record(p.records + base + (unsigned long long)q, o);
+                St.nb[q] = o.out.ok ? (int)o.out.n_beans : 0;
+                St.na[q] = o.out.ok ? o.nkept : 0;
+                write_outcome(p.records + base + (unsigned long long)q, o.out);
             }
         }
         __syncwarp();
@@ -2306,13 +2210,12 @@ __global__ void __launch_bounds__(kConsThreads, BLU_CONS_MINB) consensus_kernel(
         }
         const int tot_b = __shfl_sync(FULL, ib, 31), tot_a = __shfl_sync(FULL, ia, 31);
         unsigned long long bb = 0, ab = 0;
+        int fits = 1;
         if (lane == 0) {
-            if (tot_b) bb = atomicAdd(&p.ctr->bean_used, (unsigned long long)tot_b);
-            if (tot_a) ab = atomicAdd(&p.ctr->acc_used, (unsigned long long)tot_a);
+            if (tot_b) fits = reserve(p.ctr, &Counters::bean_used, tot_b, p.bean_cap, bb);
+            if (tot_a) fits &= reserve(p.ctr, &Counters::acc_used, tot_a, p.acc_cap, ab);
         }
-        bb = __shfl_sync(FULL, bb, 0), ab = __shfl_sync(FULL, ab, 0);
-        const bool fits = bb + (unsigned long long)tot_b <= p.bean_cap && ab + (unsigned long long)tot_a <= p.acc_cap;
-        if (!fits && lane == 0) p.ctr->cap_overflow = 1;
+        bb = __shfl_sync(FULL, bb, 0), ab = __shfl_sync(FULL, ab, 0), fits = __shfl_sync(FULL, fits, 0);
         const unsigned long long my_b = bb + (unsigned long long)(ib - vb), my_a = ab + (unsigned long long)(ia - va);
         if (fits) {
             if (vb > 0) {
@@ -2339,20 +2242,16 @@ __global__ void __launch_bounds__(kConsThreads, BLU_CONS_MINB) consensus_kernel(
             const ConsLane ow = cons_compute<32>(p, true, gw2, slotw, qoffw, lane);
             unsigned long long wb = 0, wa = 0;
             int wfits = 1;
-            if (lane == 0 && ow.ok) {
-                wb = atomicAdd(&p.ctr->bean_used, (unsigned long long)ow.nb);
-                wa = atomicAdd(&p.ctr->acc_used, (unsigned long long)ow.nkept);
-                wfits = wb + (unsigned long long)ow.nb <= p.bean_cap && wa + (unsigned long long)ow.nkept <= p.acc_cap;
-                if (!wfits) p.ctr->cap_overflow = 1;
-            }
+            if (lane == 0 && ow.out.ok)
+                wfits = reserve(p.ctr, &Counters::bean_used, ow.out.n_beans, p.bean_cap, wb) & reserve(p.ctr, &Counters::acc_used, ow.nkept, p.acc_cap, wa);
             wb = __shfl_sync(FULL, wb, 0), wa = __shfl_sync(FULL, wa, 0), wfits = __shfl_sync(FULL, wfits, 0);
-            if (ow.ok && wfits) {
+            if (ow.out.ok && wfits) {
                 if (ow.leader) p.beans[wb + ow.bean_idx] = ow.bean;
                 if (ow.keeps) p.accs[wa + ow.acc_idx].ref = ow.acc_ref;
             }
             if (lane == 0) {
-                cons_write_record(recw, ow);
-                if (ow.ok && wfits) recw->bean_base = (uint32_t)wb, recw->acc_base = (uint32_t)wa;
+                write_outcome(recw, ow.out);
+                if (ow.out.ok && wfits) recw->bean_base = (uint32_t)wb, recw->acc_base = (uint32_t)wa;
             }
         }
     }
@@ -2384,7 +2283,7 @@ __global__ void __launch_bounds__(256) gather_kernel(const __grid_constant__ Pos
         if (live) {
             qoff = rec->query_off, qlen = rec->query_len;
             bytes = qlen;
-            if (rec->status == 1) {
+            if (rec->status == kStatusFound) {
                 abase = rec->acc_base;
                 const uint32_t nbn = rec->n_beans;
                 if (nbn) {
@@ -2403,13 +2302,11 @@ __global__ void __launch_bounds__(256) gather_kernel(const __grid_constant__ Pos
         }
         const unsigned long long total = __shfl_sync(FULL, inc, 31);
         unsigned long long wbase = 0;
-        if (lane == 31 && total) wbase = atomicAdd(&p.ctr->pool_used, total);
+        int fits = 1;
+        // (counting pass, no pool: nothing to overflow, pool_used ends up as the size the pool needs)
+        if (lane == 31 && total) fits = reserve(p.ctr, &Counters::pool_used, total, p.pool ? p.pool_cap : ~0ull, wbase);
         wbase = __shfl_sync(FULL, wbase, 31);
-        if (!p.pool) continue;  // counting pass: pool_used ends up as the size the pool needs
-        if (wbase + total > p.pool_cap) {
-            if (lane == 0) p.ctr->cap_overflow = 1;
-            continue;
-        }
+        if (!p.pool || !__shfl_sync(FULL, fits, 31)) continue;
         const unsigned long long mine = wbase + inc - bytes;  // where this lane's record's strings start
         // ---- copy, string by string, the whole warp on each --------------------------------------------------------------
         uint32_t namax = nacc;
@@ -2478,7 +2375,7 @@ __global__ void __launch_bounds__(256) dup_kernel(const __grid_constant__ DupPar
         }
         if (p.ref_delta) {
             r.query_off = (unsigned long long)((long long)r.query_off + p.ref_delta);
-            if (r.status == 1 && r.n_beans) {
+            if (r.status == kStatusFound && r.n_beans) {
                 const blu_bean lb = p.beans[(unsigned long long)r.bean_base + r.n_beans - 1];
                 const unsigned nacc = lb.acc_begin + lb.n_acc;
                 for (unsigned a = 0; a < nacc; a++) {

@@ -179,12 +179,7 @@ static int sim_run_impl(const int64_t* taxids, const uint64_t* off, const char* 
                 }
             const size_t g = top.size();
             if (g > 65535) return BLU_ERR_UNSUPPORTED;
-            blu_record rec;
-            memset(&rec, 0, sizeof rec);
-            rec.query_off = rows[h].s;
-            rec.query_len = (uint32_t)rows[h].qlen;
-            rec.n_rows = (uint32_t)(e - h);
-            rec.bit_score = mx;
+            blu_record rec = record_header(rows[h].s, (uint32_t)rows[h].qlen, (uint32_t)(e - h), mx);
             rec.bean_base = (uint32_t)beans.size();
             rec.acc_base = (uint32_t)accs.size();
             beans.resize(beans.size() + g);

@@ -1,6 +1,10 @@
 """The generated cases of tests/test_properties_hypothesis.py through the CUDA path (C ABI): lineage maps with non-Linnaean levels,
 unequal lengths, rank names that occur twice and fully tied beans; hit groups that tie on the truncated bit score; custom cutoff
-tables; rows with odd fields.  Derandomised: every run draws the same cases."""
+tables; rows with odd fields.  Derandomised: every run draws the same cases.
+
+These cases have top groups of 1..4 rows nearly always, so they reach the 8-lane consensus only; the same cases rewritten into
+top groups of 9..1000 rows and bit scores beyond int32 (the 32-lane and the block-parallel consensus) are in
+tests/test_gpu_consensus_classes.py."""
 import pytest
 from hypothesis import HealthCheck, given, settings
 from hypothesis import strategies as st

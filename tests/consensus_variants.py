@@ -1,4 +1,4 @@
-"""Variants of the generated cases of tests/test_properties_hypothesis.py that reach every consensus implementation of the GPU.
+"""Variants of the generated cases of tests/generators.py that reach every consensus implementation of the GPU.
 
 The size of a query's top bit-score group picks the implementation on the GPU:
 
@@ -29,7 +29,7 @@ twin that differs at the root makes its query a root-level disagreement: an erro
 No GPU imports: the CPU tests use the generator as the GPU tests do."""
 from hypothesis import strategies as st
 
-from test_properties_hypothesis import lineage_maps, tables  # noqa: F401  (the strategies the variants start from)
+from generators import lineage_maps, tables  # noqa: F401  (the strategies the variants start from)
 
 LIFT = 3_000_000_000
 INT32_MAX = 2 ** 31 - 1

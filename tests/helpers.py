@@ -1,10 +1,14 @@
-"""Shared test helpers: seeded random taxonomies / hit tables for small parity cases.
+"""Shared test helpers: seeded random taxonomies / hit tables for small parity cases, the cutoff tables and lineage maps
+several modules use, and the constructors of engines and device-resident texts.
 
 Generators avoid, by construction, inputs on which the reference is non-deterministic (bean full
-ties: same identifier under different ranks) unless a test asks for error cases explicitly."""
+ties: same identifier under different ranks) unless a test asks for error cases explicitly.
+
+Nothing here imports blutils_b200 or torch at module level: the CPU-only suite collects every module."""
 from __future__ import annotations
 
 import json
+import math
 import os
 import random
 import sys
@@ -13,6 +17,155 @@ from typing import Dict, List, Optional, Tuple
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
+
+# The 16S cutoffs of the reference's custom-taxon YAML example.
+CUTOFFS_16S = {"domain": 50, "kingdom": 60, "phylum": 75, "class": 80, "order": 85, "family": 92, "genus": 97, "species": 99}
+
+# A small lineage map; IDS5 adds a 16-digit taxid, so that the taxids have 1 .. 16 digits (lean splitter: <= 8, <= 16, beyond).
+LIN = ["d__bac;p__p1;c__c1;o__o1;f__f1;g__g1;s__s1", "d__bac;p__p1;c__c1;o__o1;f__f1;g__g1;s__s2", "d__bac;p__p1;c__c1;o__o1;f__f1;g__g2;s__s3",
+       "d__bac;p__p1;c__c1;o__o1;f__f2;g__g3;s__s4"]
+IDS = [7, 4242, 1660760528, 99999999]
+LIN5 = LIN + ["d__bac;p__p2;c__c2;o__o2;f__f3;g__g4;s__s5"]
+IDS5 = IDS + [1234567890123456]
+
+COUNTERS_BYTES = 120  # sizeof(Counters), blu_kernels.h: eleven 8-byte and eight 4-byte fields
+CHUNK = 1 << 20
+
+# Known answers of InterpolatedIdentity::interpolate_identities (linnaean_ranks.rs:220-383), SURVEY.md section 3.3: rank names,
+# the bacteria cutoffs, the CUTOFFS_16S cutoffs.
+NAN = float("nan")
+KAT = [
+    ("d p c o f g s", [60, 75, 80, 85, 92, 97, 99], [50, 75, 80, 85, 92, 97, 99]),
+    ("d clade p c o f g species-group species-subgroup s", [60, 67.5, 75, 80, 85, 92, 97, 97.667, 98.333, 99],
+     [50, 62.5, 75, 80, 85, 92, 97, 97.667, 98.333, 99]),
+    ("d p c o f g s strain", [60, 75, 80, 85, 92, 97, 99, 100], [50, 75, 80, 85, 92, 97, 99, 100]),
+    ("d clade clade p c o f g s strain", [60, 65, 70, 75, 80, 85, 92, 97, 99, 100], [50, 58.333, 66.667, 75, 80, 85, 92, 97, 99, 100]),
+    ("no-rank d p c o f g s", [99, 60, 75, 80, 85, 92, 97, 99], [50, 50, 75, 80, 85, 92, 97, 99]),
+    ("d p c o suborder f g s", [60, 75, 80, 85, 88.5, 92, 97, 99], [50, 75, 80, 85, 88.5, 92, 97, 99]),
+    ("d p c o f no-rank g s", [60, 75, 80, 85, 92, 94.333, 97, 99], [50, 75, 80, 85, 92, 94.333, 97, 99]),
+    ("d p c o f g s subspecies no-rank", [60, 75, 80, 85, 92, 97, 99, 99.5, 100], [50, 75, 80, 85, 92, 97, 99, 99.5, 100]),
+    ("d k p c o f g s", [60, 67.5, 75, 80, 85, 92, 97, 99], [50, 60, 75, 80, 85, 92, 97, 99]),
+    ("superkingdom p c o f g s", [99, 75, 80, 85, 92, 97, 99], [50, 75, 80, 85, 92, 97, 99]),
+    ("no-rank d k p c o f g s no-rank", [99, 60, 66.667, 75, 80, 85, 92, 97, 99, NAN], [50, 50, 60, 75, 80, 85, 92, 97, 99, NAN]),
+    ("clade", [NAN], [NAN]),
+]
+
+
+def same(a, b):
+    """Equal cutoff vectors, NaN equal to NaN."""
+    return len(a) == len(b) and all((math.isnan(x) and math.isnan(y)) or x == y for x, y in zip(a, b))
+
+
+def engine(taxon, strategy, use_taxid=False, custom=None, lineages=None, **kwargs):
+    """A ConsensusEngine from taxon ("bacteria", "fungi", "eukaryotes", "custom") and strategy ("cautious", "relaxed")
+    names and a cutoff dict; keyword arguments (chunk_bytes, text_refs, devices) go to the constructor, and
+    `lineages` = (ids, lineage strings) is loaded when given."""
+    from blutils_b200 import ConsensusEngine, ConsensusStrategy, CustomTaxon, Taxon
+
+    ct = None
+    if custom is not None:
+        ct = CustomTaxon(domain=custom["domain"], species=custom["species"], kingdom=custom.get("kingdom"), phylum=custom.get("phylum"),
+                         class_=custom.get("class"), order=custom.get("order"), family=custom.get("family"), genus=custom.get("genus"))
+    eng = ConsensusEngine(Taxon[taxon.capitalize()], ConsensusStrategy[strategy.capitalize()], use_taxid, ct, **kwargs)
+    if lineages is not None:
+        eng.load_taxonomy_arrays(*lineages)
+    return eng
+
+
+def to_device(text):
+    """`text` in a zero-padded device buffer (a multiple of 128 bytes, at least 128 bytes of padding)."""
+    import torch
+
+    n = len(text)
+    t = torch.zeros((n + 255) // 128 * 128, dtype=torch.uint8, device="cuda")
+    t[:n] = torch.frombuffer(bytearray(text), dtype=torch.uint8).cuda()
+    torch.cuda.synchronize()
+    return t
+
+
+def current_stream():
+    import torch
+
+    return torch.cuda.current_stream().cuda_stream
+
+
+def device_sets():
+    """Device lists of multi-device contexts: [0] always, more where the box has the GPUs."""
+    import torch
+
+    n = torch.cuda.device_count()
+    sets = [[0]]
+    if n >= 2:
+        sets += [[0, 1], [1, 0]]
+    if n >= 4:
+        sets.append([0, 1, 2, 3])
+    if n >= 8:
+        sets.append(list(range(8)))
+    return sets
+
+
+def hit_row(q, acc, taxid, pident, ln, bits, *, mismatch=0, sstart=1, evalue="0.0"):
+    """One 13-column hit row (outfmt 6 std + bitscore): an alignment of `ln` columns, the subject's from `sstart`."""
+    return f"{q}\t{acc}\t{taxid}\t{pident}\t{ln}\t{mismatch}\t0\t1\t{ln}\t{sstart}\t{ln + sstart - 1}\t{evalue}\t{bits}\n"
+
+
+def hit_table(n_queries, rows_per_query, seed):
+    """Queries over IDS / LIN, `rows_per_query` rows each (0: 1, 2, 3, 40 or 700 at random), 1, 2 or 4 of them top rows."""
+    rng = random.Random(seed)
+    rows = []
+    for q in range(n_queries):
+        n = rows_per_query if rows_per_query > 0 else rng.choice([1, 2, 3, 40, 700])
+        best = set(rng.sample(range(n), min(n, rng.choice([1, 2, 4]))))
+        for h in range(n):
+            rows.append(hit_row(f"query_{q:06d}", f"NR_{(q * 17 + h) % 3000:06d}.1", IDS[(q + h) % 4], f"{88 + h % 12}.{(q + h) % 1000:03d}",
+                                300 + h % 200, "950" if h in best else str(100 + (h * 13 + q) % 800), mismatch=3, sstart=17, evalue="1e-50"))
+    return "".join(rows).encode()
+
+
+def tiny_rows():
+    """120 000 queries of one or two tiny rows over IDS: a fresh context's first capacity estimate holds about a third of
+    the records."""
+    rows = []
+    for q in range(120000):
+        for h in range(1 + (q % 5 == 0)):
+            rows.append(f"q{q}\tA\t{IDS[q % 2]}\t9{h}\t{1 + q % 9}\t0\t0\t1\t1\t1\t1\t0\t{5 + (q + h) % 3}\n")
+    return "".join(rows).encode()
+
+
+def synth_case(n_taxa, n_queries, hits, zipf=False, seed=11):
+    """(taxids, lineage strings, hit table) of a synthetic workload."""
+    from blutils_b200.synth import SynthWorkload
+
+    w = SynthWorkload(n_taxa, seed=seed)
+    ids, off, blob = w.lineages()
+    lin = [bytes(blob[int(off[i]):int(off[i + 1])]).decode() for i in range(len(ids))]
+    text = w.hits(0, n_queries, hits, zipf=zipf)
+    return ids.tolist(), lin, text
+
+
+def scattered_table(rng, n_queries, max_hits, n_taxa, blank_lines=False, final_newline=True):
+    """Rows of every query dealt out over the file in up to three far-apart fragments (file order inside a query kept)."""
+    ids = list(range(1, n_taxa + 1))
+    lin = [f"d__bac;p__p{t % 3};c__c{t % 7};o__o{t % 11};f__f{t % 13};g__g{t % 17};s__s{t}" for t in ids]
+    parts = [[], [], []]
+    for q in range(n_queries):
+        t0 = rng.randrange(n_taxa)
+        hits = rng.randint(1, max_hits)
+        for h in range(hits):
+            t = ids[(t0 + rng.choice([0, 0, 1, 2, 17])) % n_taxa]
+            bits = 900 - 10 * (h // 3) + (1 if rng.random() < 0.05 else 0)  # now and then the best row sits in a later fragment
+            row = hit_row(f"read_{q:06d}/1" if q % 7 else f"M0{q}:long:read:name:{q:09d}:abcdefgh", f"ACC{q}_{h}.{h % 3}", t,
+                          f"{88 + (h * 5 + q) % 12}.{(q + h) % 100:02d}", 150 + h, str(bits))
+            parts[min(2, rng.randrange(4))].append(row)
+    rows = parts[0] + parts[1] + parts[2]
+    if blank_lines:
+        for i in range(5, len(rows), 211):
+            rows[i] = "\n" + rows[i]
+    text = "".join(rows)
+    if not final_newline:
+        text = text[:-1]
+    return ids, lin, text.encode()
+
 
 BACKBONE_RANKS = ["d", "p", "c", "o", "f", "g", "s"]
 ODD_RANKS = ["clade", "no rank", "species group", "species subgroup", "strain", "subspecies", "k", "superkingdom",

@@ -11,11 +11,8 @@ import pytest
 
 import pyoracle as po
 import sim_ffi
-from helpers import ROOT, random_blast, random_taxonomy, write_taxonomy
+from helpers import CUTOFFS_16S, KAT, ROOT, random_blast, random_taxonomy, same, write_taxonomy
 from oracle_ffi import Oracle, OracleDataError
-from test_oracle_interpolation import KAT, YAML16S, same
-
-FULL = YAML16S
 
 
 def test_header_symbols_exported():
@@ -57,13 +54,13 @@ def test_product_has_no_oracle_dependency():
 def test_product_interpolation_kat(ranks, bact, cust):
     names = ranks.split()
     assert same(sim_ffi.interpolate(names, "bacteria"), [float(x) for x in bact])
-    assert same(sim_ffi.interpolate(names, "custom", YAML16S), [float(x) for x in cust])
+    assert same(sim_ffi.interpolate(names, "custom", CUTOFFS_16S), [float(x) for x in cust])
 
 
 def test_custom_cutoff_files(tmp_path):
     y = tmp_path / "c.yaml"
     y.write_text("domain: 50\nkingdom: 60\nphylum: 75\nclass: 80\norder: 85\nfamily: 92\ngenus: 97\nspecies: 99\n")
-    assert sim_ffi.custom_cutoffs(str(y)) == YAML16S == po.load_custom_cutoffs(str(y))
+    assert sim_ffi.custom_cutoffs(str(y)) == CUTOFFS_16S == po.load_custom_cutoffs(str(y))
     y2 = tmp_path / "d.yaml"
     y2.write_text("# partial\n---\ndomain: 40\nspecies: 98   # trailing comment\ngenus: ~\n")
     assert sim_ffi.custom_cutoffs(str(y2)) == {"domain": 40, "kingdom": None, "phylum": None, "class": None, "order": None, "family": None,
@@ -123,7 +120,7 @@ def test_device_core_on_host_vs_oracle(seed):
             for use_taxid in (False, True):
                 custom = None
                 if taxon == "custom":
-                    custom = FULL if seed % 3 else {"domain": 50, "species": 99, "genus": 95}
+                    custom = CUTOFFS_16S if seed % 3 else {"domain": 50, "species": 99, "genus": 95}
                 lin = [(u["numericLineage"] if use_taxid else u["textLineage"]) for u in units]
                 ids = [u["taxid"] for u in units]
                 try:

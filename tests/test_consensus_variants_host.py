@@ -7,7 +7,7 @@ from hypothesis import HealthCheck, given, settings
 from hypothesis import strategies as st
 
 import consensus_variants as V
-from test_properties_hypothesis import _text, _three_ways
+from generators import _text, _three_ways
 
 
 @settings(max_examples=40, derandomize=True, database=None, deadline=None, suppress_health_check=[HealthCheck.too_slow, HealthCheck.data_too_large])

@@ -10,7 +10,7 @@ import subprocess
 
 import pytest
 
-from helpers import random_blast, random_taxonomy, write_taxonomy
+from helpers import CUTOFFS_16S, random_blast, random_taxonomy, write_taxonomy
 
 pytestmark = pytest.mark.gpu
 
@@ -87,8 +87,7 @@ def test_build_consensus_custom_cutoffs_and_errors(tmp_path):
     blast, tax_path, text, tax = _case(tmp_path, 31)
     y = tmp_path / "cut.yaml"
     y.write_text("domain: 50\nkingdom: 60\nphylum: 75\nclass: 80\norder: 85\nfamily: 92\ngenus: 97\nspecies: 99\n")
-    custom = {"domain": 50, "kingdom": 60, "phylum": 75, "class": 80, "order": 85, "family": 92, "genus": 97, "species": 99}
-    want = po.build_consensus_identities(text, tax, "custom", "cautious", custom)
+    want = po.build_consensus_identities(text, tax, "custom", "cautious", CUTOFFS_16S)
     got = _run(["blastn", "build-consensus", blast, "--tax-file", tax_path, "--taxon", "custom", "-c", str(y), "--strategy", "cautious",
                 "--out-format", "jsonl"]).stdout.decode()
     assert got == "null\n" + po.results_to_jsonl(want, UUID.search(got).group(0))

@@ -4,29 +4,22 @@ import ctypes as C
 
 import pytest
 
+from helpers import CUTOFFS_16S, engine
+from oracle_ffi import Oracle
+
 pytestmark = pytest.mark.gpu
 
-YAML16S = {"domain": 50, "kingdom": 60, "phylum": 75, "class": 80, "order": 85, "family": 92, "genus": 97, "species": 99}
 
-
-def _setup(n_taxa, seed, taxon="bacteria", strategy="relaxed", custom=None, chunk_bytes=0, numeric=False):
-    from blutils_b200 import ConsensusEngine, ConsensusStrategy, CustomTaxon, Taxon
+def _baseline_case(n_taxa, seed, taxon="bacteria", strategy="relaxed", custom=None, chunk_bytes=0, numeric=False):
+    """A synthetic workload, an engine that holds its lineage map (loaded through the raw-array entry point), the oracle."""
     from blutils_b200.synth import SynthWorkload
-    from oracle_ffi import Oracle
 
     w = SynthWorkload(n_taxa, seed=seed)
     ids, off, blob = w.lineages(numeric=numeric)
-    ct = None
-    if custom:
-        ct = CustomTaxon(domain=custom["domain"], species=custom["species"], kingdom=custom.get("kingdom"), phylum=custom.get("phylum"),
-                         class_=custom.get("class"), order=custom.get("order"), family=custom.get("family"), genus=custom.get("genus"))
-    eng = ConsensusEngine({"bacteria": Taxon.Bacteria, "custom": Taxon.Custom}[taxon],
-                          {"cautious": ConsensusStrategy.Cautious, "relaxed": ConsensusStrategy.Relaxed}[strategy], numeric, ct,
-                          chunk_bytes=chunk_bytes)
+    eng = engine(taxon, strategy, numeric, custom, chunk_bytes=chunk_bytes)
     eng.load_taxonomy_raw(ids.ctypes.data, off.ctypes.data, blob.ctypes.data, len(ids))
     lin = [bytes(blob[int(off[i]):int(off[i + 1])]).decode() for i in range(len(ids))]
-    orc = Oracle(ids.tolist(), lin, taxon, strategy, custom)
-    return w, eng, orc
+    return w, eng, Oracle(ids.tolist(), lin, taxon, strategy, custom)
 
 
 def _check(eng, orc, text, n_queries):
@@ -41,7 +34,7 @@ def _check(eng, orc, text, n_queries):
 
 def test_c2_custom_16s_cutoffs():
     """C2 shape: 50 hits/query, 30 k taxa, --taxon custom with the 16S YAML values (120 k queries, 458 MB)."""
-    w, eng, orc = _setup(30_000, 20261020, taxon="custom", custom=YAML16S)
+    w, eng, orc = _baseline_case(30_000, 20261020, taxon="custom", custom=CUTOFFS_16S)
     text = w.hits(0, 120_000, 50)
     _check(eng, orc, text, 120_000)
     eng.close()
@@ -49,7 +42,7 @@ def test_c2_custom_16s_cutoffs():
 
 def test_c3_two_million_taxa():
     """C3 shape: 100 hits/query against a 2 M-taxon lineage map (hash table + tables beyond L1, 60 k queries)."""
-    w, eng, orc = _setup(2_000_000, 20261021, strategy="cautious", numeric=True)
+    w, eng, orc = _baseline_case(2_000_000, 20261021, strategy="cautious", numeric=True)
     text = w.hits(0, 60_000, 100)
     out = _check(eng, orc, text, 60_000)
     # device-resident path on the same table
@@ -65,7 +58,7 @@ def test_c3_two_million_taxa():
 
 def test_c4_zipf_skew():
     """C4 shape: Zipf(1.1) hits/query on [1, 5000] (long-tail queries take the block path), ~400 MB."""
-    w, eng, orc = _setup(200_000, 20261022)
+    w, eng, orc = _baseline_case(200_000, 20261022)
     text = w.hits(0, 12_000, 5000, zipf=True)
     out = _check(eng, orc, text, 12_000)
     assert eng.timings()["n_deferred_runs"] >= 0  # (the streaming kernels carry queries of any length; only top groups > 32 rows take the block path)
@@ -77,7 +70,7 @@ def test_c5_streamed_shards():
     on its own, the shard checksums must add up to the checksum of the whole (and to the oracle's)."""
     from blutils_b200 import shard_cuts
 
-    w, eng, orc = _setup(200_000, 20261023, chunk_bytes=64 << 20)
+    w, eng, orc = _baseline_case(200_000, 20261023, chunk_bytes=64 << 20)
     text = w.hits(0, 300_000, 50)
     whole = _check(eng, orc, text, 300_000).checksum()
     cuts = shard_cuts(text, 8)

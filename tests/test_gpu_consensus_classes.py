@@ -1,4 +1,4 @@
-"""The generated cases of tests/test_properties_hypothesis.py, rewritten by tests/consensus_variants.py, through all three
+"""The generated cases of tests/generators.py, rewritten by tests/consensus_variants.py, through all three
 consensus implementations of the GPU: cons_compute<8> (top groups of 1..8 rows), cons_compute<32> (9..32 rows) and the
 long-run kernel's long_consensus / consensus_single (more than 32 rows, or a bit score beyond int32).  Lineage maps with
 non-Linnaean levels, rank names that occur twice at one level (fully tied beans), unequal depths; fungi, eukaryote and custom
@@ -14,17 +14,16 @@ import json
 from collections import Counter
 
 import pytest
-from hypothesis import HealthCheck, given, settings
+from hypothesis import given, settings
 from hypothesis import strategies as st
 
 import consensus_variants as V
+from generators import GPU, _text
+from helpers import engine
 from oracle_ffi import Oracle, OracleDataError
-from test_gpu_parity import _engine
-from test_properties_hypothesis import _text
 
 pytestmark = pytest.mark.gpu
 
-GPU = dict(max_examples=150, derandomize=True, deadline=None, database=None, suppress_health_check=list(HealthCheck))
 PANICS_PER_CLASS = 3  # aborting queries per case and class that are run alone on the GPU
 
 # Floors of the counts over the 150 derandomised cases: about half of what the draws and the C++ oracle give.  They depend on
@@ -38,7 +37,7 @@ TIED_FLOOR = {"warp32": 170, "block": 400}  # compared results with two fully ti
 def fixed_engines():
     """One context per configuration with fixed cutoffs (the six of bacteria, fungi, eukaryotes); every case loads its own
     taxonomy into them."""
-    engines = {(taxon, strategy): _engine(taxon, strategy) for taxon, strategy in V.CONFIGS if taxon != "custom"}
+    engines = {(taxon, strategy): engine(taxon, strategy) for taxon, strategy in V.CONFIGS if taxon != "custom"}
     yield engines
     for e in engines.values():
         e.close()
@@ -86,7 +85,7 @@ def _engines_for(fixed, tax, custom):
     engines, own = [], []
     for taxon, strategy in V.CONFIGS:
         if taxon == "custom":
-            eng = _engine(taxon, strategy, custom=custom)
+            eng = engine(taxon, strategy, custom=custom)
             own.append(eng)
         else:
             eng = fixed[(taxon, strategy)]

@@ -6,52 +6,22 @@ import random
 
 import pytest
 
-from helpers import random_blast, random_taxonomy
+from helpers import IDS, LIN, engine, hit_table, random_blast, random_taxonomy, tiny_rows
+from oracle_ffi import Oracle, OracleDataError
 
 pytestmark = pytest.mark.gpu
-
-LIN = ["d__bac;p__p1;c__c1;o__o1;f__f1;g__g1;s__s1", "d__bac;p__p1;c__c1;o__o1;f__f1;g__g1;s__s2", "d__bac;p__p1;c__c1;o__o1;f__f1;g__g2;s__s3",
-       "d__bac;p__p1;c__c1;o__o1;f__f2;g__g3;s__s4"]
-IDS = [7, 4242, 1660760528, 99999999]
-
-
-def _engine(chunk_bytes=0, strategy="relaxed"):
-    from blutils_b200 import ConsensusEngine, ConsensusStrategy, Taxon
-
-    eng = ConsensusEngine(Taxon.Bacteria, ConsensusStrategy.Relaxed if strategy == "relaxed" else ConsensusStrategy.Cautious, False, None,
-                          chunk_bytes=chunk_bytes)
-    eng.load_taxonomy_arrays(IDS, LIN)
-    return eng
-
-
-def _row(q, acc, taxid, pident, ln, bits):
-    return f"{q}\t{acc}\t{taxid}\t{pident}\t{ln}\t3\t0\t1\t{ln}\t17\t{ln + 16}\t1e-50\t{bits}\n"
-
-
-def _table(n_queries, rows_per_query, seed):
-    rng = random.Random(seed)
-    rows = []
-    for q in range(n_queries):
-        n = rows_per_query if rows_per_query > 0 else rng.choice([1, 2, 3, 40, 700])
-        best = set(rng.sample(range(n), min(n, rng.choice([1, 2, 4]))))
-        for h in range(n):
-            rows.append(_row(f"query_{q:06d}", f"NR_{(q * 17 + h) % 3000:06d}.1", IDS[(q + h) % 4], f"{88 + h % 12}.{(q + h) % 1000:03d}", 300 + h % 200,
-                             "950" if h in best else str(100 + (h * 13 + q) % 800)))
-    return "".join(rows).encode()
 
 
 @pytest.mark.parametrize("chunk,threads", [(1 << 20, None), (1 << 20, "1"), (3 << 20, "5"), (0, None)])
 def test_streamed_file_equals_memory_and_oracle(tmp_path, chunk, threads, monkeypatch):
     """~9 MB table: nine 1 MiB chunks (the staging ring wraps three times), three 3 MiB chunks, and one chunk."""
-    from oracle_ffi import Oracle
-
     if threads:
         monkeypatch.setenv("BLU_READ_THREADS", threads)
-    text = _table(900, 0, seed=3)
+    text = hit_table(900, 0, seed=3)
     path = tmp_path / "blast.out"
     path.write_bytes(text)
     want = Oracle(IDS, LIN, "bacteria", "relaxed").run_raw(text)[0]
-    eng = _engine(chunk)
+    eng = engine("bacteria", "relaxed", chunk_bytes=chunk, lineages=(IDS, LIN))
     from_file = eng.run_file(str(path))
     assert from_file.jsonl() == want
     t = eng.timings()
@@ -64,17 +34,11 @@ def test_streamed_file_equals_memory_and_oracle(tmp_path, chunk, threads, monkey
 def test_streamed_file_restarts_after_a_capacity_retry(tmp_path):
     """Tiny rows, one or two per query: more queries than the first capacity estimate allows, so the run starts over from
     chunk 0 while the reader is already ahead."""
-    from oracle_ffi import Oracle
-
-    rows = []
-    for q in range(120000):
-        for h in range(1 + (q % 5 == 0)):
-            rows.append(f"q{q}\tA\t{IDS[q % 2]}\t9{h}\t{1 + q % 9}\t0\t0\t1\t1\t1\t1\t0\t{5 + (q + h) % 3}\n")
-    text = "".join(rows).encode()
+    text = tiny_rows()
     path = tmp_path / "tiny.out"
     path.write_bytes(text)
     want = Oracle(IDS, LIN, "bacteria", "relaxed").run_raw(text)[0]
-    eng = _engine(1 << 20)
+    eng = engine("bacteria", "relaxed", chunk_bytes=1 << 20, lineages=(IDS, LIN))
     out = eng.run_file(str(path))
     assert len(out) == 120000 and out.jsonl() == want
     eng.close()
@@ -86,17 +50,13 @@ def test_noncontiguous_file_is_regrouped(tmp_path):
     text = random_blast(rng, units, n_queries=40, contiguous=False)
     lin = [u["textLineage"] for u in units]
     ids = [u["taxid"] for u in units]
-    from blutils_b200 import ConsensusEngine, ConsensusStrategy, Taxon
-    from oracle_ffi import Oracle, OracleDataError
-
     try:
         want = Oracle(ids, lin, "fungi", "relaxed").run_raw(text)[0]
     except OracleDataError:
         pytest.skip("generated case hits a reference abort")
     path = tmp_path / "scattered.out"
     path.write_bytes(text)
-    eng = ConsensusEngine(Taxon.Fungi, ConsensusStrategy.Relaxed, False, None)
-    eng.load_taxonomy_arrays(ids, lin)
+    eng = engine("fungi", "relaxed", lineages=(ids, lin))
     out = eng.run_file(str(path))
     assert out.jsonl() == want
     eng.close()
@@ -105,7 +65,7 @@ def test_noncontiguous_file_is_regrouped(tmp_path):
 def test_file_errors(tmp_path):
     from blutils_b200 import ConsensusPanic, MappedErrors
 
-    eng = _engine()
+    eng = engine("bacteria", "relaxed", lineages=(IDS, LIN))
     with pytest.raises(MappedErrors):
         eng.run_file(str(tmp_path / "absent.out"))
     with pytest.raises(MappedErrors):
@@ -115,11 +75,11 @@ def test_file_errors(tmp_path):
     with pytest.raises(ConsensusPanic):
         eng.run_file(str(empty))
     bad = tmp_path / "bad.out"
-    bad.write_bytes(_table(50, 30, seed=1) + b"q\tacc\t7\t99.0\t10\t0\t0\t1\t10\t1\t10\t0.0\n")  # 12 fields in the last row
+    bad.write_bytes(hit_table(50, 30, seed=1) + b"q\tacc\t7\t99.0\t10\t0\t0\t1\t10\t1\t10\t0.0\n")  # 12 fields in the last row
     with pytest.raises(ConsensusPanic):
         eng.run_file(str(bad))
     # the context stays usable after a failed run
     good = tmp_path / "good.out"
-    good.write_bytes(_table(50, 30, seed=1))
+    good.write_bytes(hit_table(50, 30, seed=1))
     assert len(eng.run_file(str(good))) == 50
     eng.close()

@@ -9,37 +9,10 @@ import subprocess
 
 import pytest
 
-from helpers import random_blast, random_taxonomy, write_taxonomy
-from test_gpu_parity import _oracle, _row, _synth_case
+from helpers import ROOT, device_sets, engine, hit_row, random_blast, random_taxonomy, synth_case, write_taxonomy
+from oracle_ffi import Oracle
 
 pytestmark = pytest.mark.gpu
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
-
-def _n_gpus():
-    import torch
-
-    return torch.cuda.device_count()
-
-
-def _multi(devices, strategy="relaxed", chunk_bytes=0, text_refs=False):
-    from blutils_b200 import ConsensusEngine, ConsensusStrategy, Taxon
-
-    return ConsensusEngine(Taxon.Bacteria, {"cautious": ConsensusStrategy.Cautious, "relaxed": ConsensusStrategy.Relaxed}[strategy], False, None,
-                           chunk_bytes=chunk_bytes, devices=devices, text_refs=text_refs)
-
-
-def _device_sets():
-    n = _n_gpus()
-    sets = [[0]]
-    if n >= 2:
-        sets += [[0, 1], [1, 0]]
-    if n >= 4:
-        sets.append([0, 1, 2, 3])
-    if n >= 8:
-        sets.append(list(range(8)))
-    return sets
 
 
 @pytest.mark.parametrize("zipf", [False, True])
@@ -47,14 +20,13 @@ def test_sharded_table_equals_oracle(zipf, tmp_path):
     """host text and file, pooled strings and text references, whole-table checksum == oracle."""
     from oracle_ffi import checksum_jsonl
 
-    ids, lin, text = _synth_case(5000, 300 if zipf else 20000, 5000 if zipf else 50, zipf=zipf, seed=23)
-    want, nq, nr = _oracle(ids, lin, "bacteria", "relaxed").run_raw(text)
+    ids, lin, text = synth_case(5000, 300 if zipf else 20000, 5000 if zipf else 50, zipf=zipf, seed=23)
+    want, nq, nr = Oracle(ids, lin, "bacteria", "relaxed").run_raw(text)
     path = tmp_path / "blast.out"
     path.write_bytes(text)
-    for devs in _device_sets():
+    for devs in device_sets():
         for refs in (False, True):
-            eng = _multi(devs, chunk_bytes=1 << 20, text_refs=refs)
-            eng.load_taxonomy_arrays(ids, lin)
+            eng = engine("bacteria", "relaxed", chunk_bytes=1 << 20, devices=devs, text_refs=refs, lineages=(ids, lin))
             out = eng.run_host(text)
             assert len(out) == nq and out.n_rows == nr, (devs, refs)
             assert out.checksum() == checksum_jsonl(want), (devs, refs)
@@ -82,13 +54,12 @@ def test_scattered_table_across_shards():
     rows = []
     for q in range(400):
         for h in range(rng.randint(1, 6)):
-            rows.append(_row(f"q{q:04d}", f"A{h}.1", rng.choice(ids), "99.0", 100, "500" if h < 2 else "300"))
-    rows.insert(3, _row("q0399", "Z.1", 3, "99.5", 100, "900"))  # a better hit of the LAST query, at the start of the file
+            rows.append(hit_row(f"q{q:04d}", f"A{h}.1", rng.choice(ids), "99.0", 100, "500" if h < 2 else "300"))
+    rows.insert(3, hit_row("q0399", "Z.1", 3, "99.5", 100, "900"))  # a better hit of the LAST query, at the start of the file
     text = "".join(rows).encode()
-    want = _oracle(ids, lin, "bacteria", "cautious").run_raw(text)[0]
-    for devs in _device_sets():
-        eng = _multi(devs, "cautious")
-        eng.load_taxonomy_arrays(ids, lin)
+    want = Oracle(ids, lin, "bacteria", "cautious").run_raw(text)[0]
+    for devs in device_sets():
+        eng = engine("bacteria", "cautious", devices=devs, lineages=(ids, lin))
         out = eng.run_host(text)
         assert out.jsonl() == want, devs
         assert int(eng.timings()["n_regrouped"]) == 2  # regrouped on the first GPU of the context
@@ -101,13 +72,12 @@ def test_errors_and_tiny_tables_multi():
     from blutils_b200 import ConsensusPanic
 
     lin = ["d__bac;p__p1;c__c1"]
-    one = _row("only", "A.1", 1, "99.0", 100, "500").encode()
-    want = _oracle([1], lin, "bacteria", "cautious").run_raw(one)[0]
-    for devs in _device_sets():
-        eng = _multi(devs, "cautious")
-        eng.load_taxonomy_arrays([1], lin)
+    one = hit_row("only", "A.1", 1, "99.0", 100, "500").encode()
+    want = Oracle([1], lin, "bacteria", "cautious").run_raw(one)[0]
+    for devs in device_sets():
+        eng = engine("bacteria", "cautious", devices=devs, lineages=([1], lin))
         assert eng.run_host(one).jsonl() == want
-        bad = "".join(_row(f"q{i}", "A.1", 1 if i != 777 else 42, "99.0", 100, "500") for i in range(1000)).encode()  # taxid 42 is unmapped
+        bad = "".join(hit_row(f"q{i}", "A.1", 1 if i != 777 else 42, "99.0", 100, "500") for i in range(1000)).encode()  # taxid 42 is unmapped
         with pytest.raises(ConsensusPanic):
             eng.run_host(bad)
         eng.close()
@@ -131,7 +101,7 @@ def test_cli_devices(tmp_path):
     blast.write_bytes(text)
     exe = os.path.join(ROOT, "blutils_b200", "blu")
     outs = []
-    for devs in _device_sets():
+    for devs in device_sets():
         o = tmp_path / ("out_" + "_".join(map(str, devs)))
         subprocess.run([exe, "blastn", "build-consensus", str(blast), "--tax-file", tax_path, "--taxon", "bacteria", "--strategy", "relaxed",
                         "--blutils-out-file", str(o), "--out-format", "jsonl", "--devices", ",".join(map(str, devs))], check=True)

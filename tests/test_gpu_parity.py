@@ -6,29 +6,11 @@ import random
 
 import pytest
 
-from helpers import random_blast, random_taxonomy, write_taxonomy
+from helpers import (CUTOFFS_16S, current_stream, engine, hit_row, random_blast, random_taxonomy, synth_case, to_device,
+                     write_taxonomy)
+from oracle_ffi import Oracle
 
 pytestmark = pytest.mark.gpu
-
-FULL = {"domain": 50, "kingdom": 60, "phylum": 75, "class": 80, "order": 85, "family": 92, "genus": 97, "species": 99}
-
-
-def _engine(taxon, strategy, use_taxid=False, custom=None, chunk_bytes=0):
-    from blutils_b200 import ConsensusEngine, ConsensusStrategy, CustomTaxon, Taxon
-
-    ct = None
-    if custom is not None:
-        ct = CustomTaxon(domain=custom["domain"], species=custom["species"], kingdom=custom.get("kingdom"), phylum=custom.get("phylum"),
-                         class_=custom.get("class"), order=custom.get("order"), family=custom.get("family"), genus=custom.get("genus"))
-    return ConsensusEngine({"bacteria": Taxon.Bacteria, "fungi": Taxon.Fungi, "eukaryotes": Taxon.Eukaryotes, "custom": Taxon.Custom}[taxon],
-                           {"cautious": ConsensusStrategy.Cautious, "relaxed": ConsensusStrategy.Relaxed}[strategy], use_taxid, ct,
-                           chunk_bytes=chunk_bytes)
-
-
-def _oracle(ids, lin, taxon, strategy, custom=None):
-    from oracle_ffi import Oracle
-
-    return Oracle(ids, lin, taxon, strategy, custom)
 
 
 @pytest.mark.parametrize("seed", range(24))
@@ -44,15 +26,14 @@ def test_random_small(seed):
             use_taxid = bool((seed + len(strategy)) & 1)
             custom = None
             if taxon == "custom":
-                custom = FULL if seed % 3 else {"domain": 50, "species": 99, "genus": 95}
+                custom = CUTOFFS_16S if seed % 3 else {"domain": 50, "species": 99, "genus": 95}
             lin = [(u["numericLineage"] if use_taxid else u["textLineage"]) for u in units]
             ids = [u["taxid"] for u in units]
             try:
-                want = _oracle(ids, lin, taxon, strategy, custom).run_raw(text)[0]
+                want = Oracle(ids, lin, taxon, strategy, custom).run_raw(text)[0]
             except OracleDataError:
                 want = None
-            eng = _engine(taxon, strategy, use_taxid, custom)
-            eng.load_taxonomy_arrays(ids, lin)
+            eng = engine(taxon, strategy, use_taxid, custom, lineages=(ids, lin))
             if want is None:
                 with pytest.raises(ConsensusPanic):
                     eng.run_host(text)
@@ -61,25 +42,14 @@ def test_random_small(seed):
             eng.close()
 
 
-def _synth_case(n_taxa, n_queries, hits, zipf=False, seed=11):
-    from blutils_b200.synth import SynthWorkload
-
-    w = SynthWorkload(n_taxa, seed=seed)
-    ids, off, blob = w.lineages()
-    lin = [bytes(blob[int(off[i]):int(off[i + 1])]).decode() for i in range(len(ids))]
-    text = w.hits(0, n_queries, hits, zipf=zipf)
-    return ids.tolist(), lin, text
-
-
 @pytest.mark.parametrize("n_queries,hits,zipf", [(300, 50, False), (4000, 50, False), (2000, 100, False), (600, 5000, True),
                                                  (40000, 1, False), (30000, 2, False), (3000, 200, False)])
 def test_synth_vs_oracle(n_queries, hits, zipf):
     """Multi-tile inputs (0.1 - 30 MB): windows, ownership, look-ahead, long-run path (Zipf up to 5000 hits)."""
-    ids, lin, text = _synth_case(5000, n_queries, hits, zipf)
+    ids, lin, text = synth_case(5000, n_queries, hits, zipf)
     for strategy in ("cautious", "relaxed"):
-        want, nq, nr = _oracle(ids, lin, "bacteria", strategy).run_raw(text)
-        eng = _engine("bacteria", strategy)
-        eng.load_taxonomy_arrays(ids, lin)
+        want, nq, nr = Oracle(ids, lin, "bacteria", strategy).run_raw(text)
+        eng = engine("bacteria", strategy, lineages=(ids, lin))
         out = eng.run_host(text)
         assert len(out) == nq and out.n_rows == nr
         assert out.jsonl() == want
@@ -89,39 +59,27 @@ def test_synth_vs_oracle(n_queries, hits, zipf):
 def test_device_resident_equals_host_and_streamed():
     """Same text through: host single chunk, host streamed in 1 MiB chunks (carry-over of the unfinished query),
     and device-resident (torch tensor)."""
-    import torch
-
-    ids, lin, text = _synth_case(5000, 6000, 50, seed=5)
-    want = _oracle(ids, lin, "bacteria", "relaxed").run_raw(text)[0]
-    eng = _engine("bacteria", "relaxed")
-    eng.load_taxonomy_arrays(ids, lin)
+    ids, lin, text = synth_case(5000, 6000, 50, seed=5)
+    want = Oracle(ids, lin, "bacteria", "relaxed").run_raw(text)[0]
+    eng = engine("bacteria", "relaxed", lineages=(ids, lin))
     assert eng.run_host(text).jsonl() == want
-    n = len(text)
-    t = torch.zeros((n + 255) // 128 * 128, dtype=torch.uint8, device="cuda")
-    t[:n] = torch.frombuffer(bytearray(text), dtype=torch.uint8).cuda()
-    torch.cuda.synchronize()
-    out = eng.run_device(t.data_ptr(), n, torch.cuda.current_stream().cuda_stream)
+    t = to_device(text)
+    out = eng.run_device(t.data_ptr(), len(text), current_stream())
     assert out.jsonl() == want
     assert out.checksum() == __import__("oracle_ffi").checksum_jsonl(want)
     eng.close()
     for chunk in (1 << 20, 3 << 20):
-        eng2 = _engine("bacteria", "relaxed", chunk_bytes=chunk)
-        eng2.load_taxonomy_arrays(ids, lin)
+        eng2 = engine("bacteria", "relaxed", chunk_bytes=chunk, lineages=(ids, lin))
         assert eng2.run_host(text).jsonl() == want
         eng2.close()
 
 
 def test_streamed_zipf_long_runs():
-    ids, lin, text = _synth_case(5000, 400, 5000, zipf=True, seed=9)
-    want = _oracle(ids, lin, "bacteria", "cautious").run_raw(text)[0]
-    eng = _engine("bacteria", "cautious", chunk_bytes=2 << 20)
-    eng.load_taxonomy_arrays(ids, lin)
+    ids, lin, text = synth_case(5000, 400, 5000, zipf=True, seed=9)
+    want = Oracle(ids, lin, "bacteria", "cautious").run_raw(text)[0]
+    eng = engine("bacteria", "cautious", chunk_bytes=2 << 20, lineages=(ids, lin))
     assert eng.run_host(text).jsonl() == want
     eng.close()
-
-
-def _row(q, acc, taxid, pident, ln, bits):
-    return f"{q}\t{acc}\t{taxid}\t{pident}\t{ln}\t0\t0\t1\t{ln}\t1\t{ln}\t0.0\t{bits}\n"
 
 
 def test_big_top_group_and_edge_rows():
@@ -131,20 +89,19 @@ def test_big_top_group_and_edge_rows():
     ids = [11, 12, 13, 14]
     rows = []
     for i in range(40):
-        rows.append(_row("qA", f"ACC{i % 7}.1", ids[i % 2], "99.5", 400, "700"))
-    rows.append(_row("qA", "LOW.1", 13, "80.0", 400, "100"))
+        rows.append(hit_row("qA", f"ACC{i % 7}.1", ids[i % 2], "99.5", 400, "700"))
+    rows.append(hit_row("qA", "LOW.1", 13, "80.0", 400, "100"))
     for i in range(700):
-        rows.append(_row("qB", f"B{i % 50:03d}.1", ids[i % 3], f"{97 + (i % 3)}.{i % 10}", 300 + i % 2, "512.0" if i % 2 else "512.9"))
+        rows.append(hit_row("qB", f"B{i % 50:03d}.1", ids[i % 3], f"{97 + (i % 3)}.{i % 10}", 300 + i % 2, "512.0" if i % 2 else "512.9"))
     rows.append("\n\n")
-    rows.append(_row("qC", "C1.1", 14, "99.9", 1500, "84.2"))
-    rows.append(_row("qC", "C2.1", 14, "98.1", 1500, "84.9"))
-    rows.append(_row("qC", "C0.1", 13, "99.0", 1500, "83.99"))
-    rows.append(_row("qD", "D1.1", 14, "100.000", 1500, "1.000e+03").rstrip("\n"))
+    rows.append(hit_row("qC", "C1.1", 14, "99.9", 1500, "84.2"))
+    rows.append(hit_row("qC", "C2.1", 14, "98.1", 1500, "84.9"))
+    rows.append(hit_row("qC", "C0.1", 13, "99.0", 1500, "83.99"))
+    rows.append(hit_row("qD", "D1.1", 14, "100.000", 1500, "1.000e+03").rstrip("\n"))
     text = "".join(rows).encode()
     for strategy in ("cautious", "relaxed"):
-        want = _oracle(ids, lin, "bacteria", strategy).run_raw(text)[0]
-        eng = _engine("bacteria", strategy)
-        eng.load_taxonomy_arrays(ids, lin)
+        want = Oracle(ids, lin, "bacteria", strategy).run_raw(text)[0]
+        eng = engine("bacteria", strategy, lineages=(ids, lin))
         assert eng.run_host(text).jsonl() == want
         eng.close()
 
@@ -158,7 +115,7 @@ def test_reference_abort_cases(bad):
     """Inputs on which the reference panics must yield an error, never a result."""
     from blutils_b200 import ConsensusPanic
 
-    eng = _engine("bacteria", "cautious")
+    eng = engine("bacteria", "cautious")
     eng.load_taxonomy_arrays([1], ["d__a;p__b"])
     with pytest.raises(ConsensusPanic):
         eng.run_host(bad)
@@ -177,11 +134,10 @@ def test_noncontiguous_tables(seed):
     from oracle_ffi import OracleDataError
 
     try:
-        want = _oracle(ids, lin, "fungi", "relaxed").run_raw(text)[0]
+        want = Oracle(ids, lin, "fungi", "relaxed").run_raw(text)[0]
     except OracleDataError:
         pytest.skip("generated case hits a reference abort")
-    eng = _engine("fungi", "relaxed")
-    eng.load_taxonomy_arrays(ids, lin)
+    eng = engine("fungi", "relaxed", lineages=(ids, lin))
     out = eng.run_host(text)
     assert out.jsonl() == want
     assert int(eng.timings()["n_regrouped"]) in (0, 2)
@@ -192,9 +148,8 @@ def test_sharded_equals_whole():
     """SURVEY 8e: query-range shards (blu_shard_cuts) processed independently and concatenated == the whole table."""
     from blutils_b200 import shard_cuts
 
-    ids, lin, text = _synth_case(3000, 3000, 50, seed=21)
-    eng = _engine("bacteria", "cautious")
-    eng.load_taxonomy_arrays(ids, lin)
+    ids, lin, text = synth_case(3000, 3000, 50, seed=21)
+    eng = engine("bacteria", "cautious", lineages=(ids, lin))
     whole = eng.run_host(text).jsonl()
     for n in (2, 3, 8):
         cuts = shard_cuts(text, n)
@@ -244,14 +199,12 @@ def test_file_api_headers_and_writer(tmp_path):
 def test_tile_and_window_edges():
     """Texts cut at every kind of position relative to the 48 KiB tile grid, with and without a trailing newline,
     with empty lines, through both the host path and tiny streaming chunks."""
-    ids, lin, text = _synth_case(2000, 2600, 50, seed=31)
+    ids, lin, text = synth_case(2000, 2600, 50, seed=31)
     rows = text.split(b"\n")
     rows = [r for r in rows if r]
-    orc = _oracle(ids, lin, "bacteria", "relaxed")
-    eng = _engine("bacteria", "relaxed")
-    eng.load_taxonomy_arrays(ids, lin)
-    eng_small = _engine("bacteria", "relaxed", chunk_bytes=96 << 10)
-    eng_small.load_taxonomy_arrays(ids, lin)
+    orc = Oracle(ids, lin, "bacteria", "relaxed")
+    eng = engine("bacteria", "relaxed", lineages=(ids, lin))
+    eng_small = engine("bacteria", "relaxed", chunk_bytes=96 << 10, lineages=(ids, lin))
     # prefix lengths (in rows) that put the end of the text just before / at / after tile and window borders
     sizes = []
     acc = 0
@@ -288,13 +241,12 @@ def test_long_rows():
     for q in range(120):
         name = f"q{q:04d}_" + "x" * (1500 if q % 3 == 0 else 20)
         for h in range(30):
-            rows.append(_row(name, f"ACC{h % 5}.1", ids[(q + h) % 2], "99.5" if h < 3 else "90.1", 400, "700" if h < 3 else "300"))
+            rows.append(hit_row(name, f"ACC{h % 5}.1", ids[(q + h) % 2], "99.5" if h < 3 else "90.1", 400, "700" if h < 3 else "300"))
     text = "".join(rows).encode()
-    want = _oracle(ids, lin, "bacteria", "cautious").run_raw(text)[0]
-    eng = _engine("bacteria", "cautious")
-    eng.load_taxonomy_arrays(ids, lin)
+    want = Oracle(ids, lin, "bacteria", "cautious").run_raw(text)[0]
+    eng = engine("bacteria", "cautious", lineages=(ids, lin))
     assert eng.run_host(text).jsonl() == want
-    big = (_row("q_small", "A.1", 11, "99.0", 10, "50") + _row("q" + "y" * 70000, "A.1", 11, "99.0", 10, "50")).encode()
+    big = (hit_row("q_small", "A.1", 11, "99.0", 10, "50") + hit_row("q" + "y" * 70000, "A.1", 11, "99.0", 10, "50")).encode()
     with pytest.raises(Unsupported):
         eng.run_host(big)
     eng.close()
@@ -302,10 +254,9 @@ def test_long_rows():
 
 def test_streamed_chunk_sizes_zipf():
     """Carry-over logic under stress: chunk sizes from 64 KiB up, long-tail (Zipf) queries of up to ~380 KB."""
-    ids, lin, text = _synth_case(3000, 250, 5000, zipf=True, seed=17)
-    want = _oracle(ids, lin, "bacteria", "relaxed").run_raw(text)[0]
+    ids, lin, text = synth_case(3000, 250, 5000, zipf=True, seed=17)
+    want = Oracle(ids, lin, "bacteria", "relaxed").run_raw(text)[0]
     for chunk in (512 << 10, 1 << 20, (1 << 20) + 4096 + 128):
-        eng = _engine("bacteria", "relaxed", chunk_bytes=chunk)
-        eng.load_taxonomy_arrays(ids, lin)
+        eng = engine("bacteria", "relaxed", chunk_bytes=chunk, lineages=(ids, lin))
         assert eng.run_host(text).jsonl() == want, chunk
         eng.close()

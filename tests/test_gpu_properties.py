@@ -1,4 +1,4 @@
-"""The generated cases of tests/test_properties_hypothesis.py through the CUDA path (C ABI): lineage maps with non-Linnaean levels,
+"""The generated cases of tests/generators.py through the CUDA path (C ABI): lineage maps with non-Linnaean levels,
 unequal lengths, rank names that occur twice and fully tied beans; hit groups that tie on the truncated bit score; custom cutoff
 tables; rows with odd fields.  Derandomised: every run draws the same cases.
 
@@ -6,16 +6,15 @@ These cases have top groups of 1..4 rows nearly always, so they reach the 8-lane
 top groups of 9..1000 rows and bit scores beyond int32 (the 32-lane and the block-parallel consensus) are in
 tests/test_gpu_consensus_classes.py."""
 import pytest
-from hypothesis import HealthCheck, given, settings
+from hypothesis import given, settings
 from hypothesis import strategies as st
 
-import test_properties_hypothesis as P
+import generators as P
+from generators import GPU
+from helpers import engine
 from oracle_ffi import Oracle, OracleDataError
-from test_gpu_parity import _engine
 
 pytestmark = pytest.mark.gpu
-
-GPU = dict(max_examples=150, derandomize=True, deadline=None, database=None, suppress_health_check=list(HealthCheck))
 
 
 def _gpu_equals_oracle(tax, text, taxon, strategy, custom=None, loud_limits=False):
@@ -27,7 +26,7 @@ def _gpu_equals_oracle(tax, text, taxon, strategy, custom=None, loud_limits=Fals
         want = Oracle(ids, lin, taxon, strategy, custom, threads=2).run_raw(text)[0]
     except OracleDataError:
         want = None
-    eng = _engine(taxon, strategy, False, custom)
+    eng = engine(taxon, strategy, False, custom)
     try:
         eng.load_taxonomy_arrays(ids, lin)
         try:

@@ -5,34 +5,20 @@ import random
 
 import pytest
 
-from helpers import random_blast, random_taxonomy
-from test_gpu_parity import FULL, _engine, _oracle, _row, _synth_case
+from helpers import current_stream, engine, hit_row, random_blast, random_taxonomy, scattered_table, synth_case, to_device
+from oracle_ffi import Oracle
 
 pytestmark = pytest.mark.gpu
-
-
-def _to_device(text):
-    import torch
-
-    n = len(text)
-    t = torch.zeros((n + 255) // 128 * 128, dtype=torch.uint8, device="cuda")
-    t[:n] = torch.frombuffer(bytearray(text), dtype=torch.uint8).cuda()
-    torch.cuda.synchronize()
-    return t
-
 
 @pytest.mark.parametrize("n_queries,hits,zipf", [(300, 50, False), (6000, 50, False), (400, 5000, True)])
 def test_device_resident_result(n_queries, hits, zipf):
     """Text in HBM -> records in HBM (no download, strings stay references into the device text); downloaded afterwards
     the result is the one of the host path.  Twice on the same context: the result arrays are recycled."""
-    import torch
-
-    ids, lin, text = _synth_case(5000, n_queries, hits, zipf, seed=13)
-    want, nq, nr = _oracle(ids, lin, "bacteria", "relaxed").run_raw(text)
-    eng = _engine("bacteria", "relaxed")
-    eng.load_taxonomy_arrays(ids, lin)
-    t = _to_device(text)
-    stream = torch.cuda.current_stream().cuda_stream
+    ids, lin, text = synth_case(5000, n_queries, hits, zipf, seed=13)
+    want, nq, nr = Oracle(ids, lin, "bacteria", "relaxed").run_raw(text)
+    eng = engine("bacteria", "relaxed", lineages=(ids, lin))
+    t = to_device(text)
+    stream = current_stream()
     for _ in range(2):
         out = eng.run_device_resident(t.data_ptr(), len(text), stream)
         assert len(out) == nq and out.n_rows == nr
@@ -52,14 +38,11 @@ def test_device_resident_result(n_queries, hits, zipf):
 def test_text_refs_equal_pool(chunk):
     """BLU_OPT_TEXT_REFS: the result's strings are references into the caller's text (nothing is gathered or downloaded
     but records / beans / 8-byte accession references); same result, fewer bytes."""
-    from blutils_b200 import ConsensusEngine, ConsensusStrategy, Taxon
-
-    ids, lin, text = _synth_case(5000, 5000, 50, seed=19)
-    want = _oracle(ids, lin, "bacteria", "cautious").run_raw(text)[0]
+    ids, lin, text = synth_case(5000, 5000, 50, seed=19)
+    want = Oracle(ids, lin, "bacteria", "cautious").run_raw(text)[0]
     d2h = {}
     for refs in (False, True):
-        eng = ConsensusEngine(Taxon.Bacteria, ConsensusStrategy.Cautious, False, None, chunk_bytes=chunk, text_refs=refs)
-        eng.load_taxonomy_arrays(ids, lin)
+        eng = engine("bacteria", "cautious", chunk_bytes=chunk, text_refs=refs, lineages=(ids, lin))
         out = eng.run_host(text)
         assert out.jsonl() == want
         d2h[refs] = int(eng.timings()["d2h_bytes"])
@@ -72,7 +55,7 @@ def _group_rows(q, n, ids, rng, n_acc=50, bits="700"):
     rows = []
     for i in range(n):
         pid = rng.choice(["99.5", "99.50", "98.123", "100.000", "97", "99.999"])
-        rows.append(_row(q, f"AC{rng.randrange(n_acc):04d}.{rng.randint(1, 2)}", rng.choice(ids), pid, rng.choice([400, 401, 1500]), bits))
+        rows.append(hit_row(q, f"AC{rng.randrange(n_acc):04d}.{rng.randint(1, 2)}", rng.choice(ids), pid, rng.choice([400, 401, 1500]), bits))
     return rows
 
 
@@ -91,13 +74,12 @@ def test_top_groups_of_every_size(sizes):
     for k, n in enumerate(sizes):
         pool = ids if k % 3 == 0 else (ids[:2] + ids[5:7] if k % 3 == 1 else ids[:1])
         rows += _group_rows(f"big{k}_{n}", n, pool, rng, n_acc=max(3, n // 7))
-        rows += [_row(f"big{k}_{n}", "LOW.1", ids[2], "80.0", 400, "100")] * 3
+        rows += [hit_row(f"big{k}_{n}", "LOW.1", ids[2], "80.0", 400, "100")] * 3
         rows += _group_rows(f"small{k}", rng.randint(1, 8), ids[:3], rng)
     text = "".join(rows).encode()
     for strategy in ("cautious", "relaxed"):
-        want = _oracle(ids, lin, "bacteria", strategy).run_raw(text)[0]
-        eng = _engine("bacteria", strategy)
-        eng.load_taxonomy_arrays(ids, lin)
+        want = Oracle(ids, lin, "bacteria", strategy).run_raw(text)[0]
+        eng = engine("bacteria", strategy, lineages=(ids, lin))
         assert eng.run_host(text).jsonl() == want, strategy
         eng.close()
 
@@ -106,9 +88,8 @@ def test_top_group_beyond_the_cap_is_loud():
     from blutils_b200 import Unsupported
 
     lin = ["d__bac;p__p1"]
-    rows = [_row("q", f"A{i}.1", 1, "99.0", 100, "500") for i in range(8193)]
-    eng = _engine("bacteria", "cautious")
-    eng.load_taxonomy_arrays([1], lin)
+    rows = [hit_row("q", f"A{i}.1", 1, "99.0", 100, "500") for i in range(8193)]
+    eng = engine("bacteria", "cautious", lineages=([1], lin))
     with pytest.raises(Unsupported):
         eng.run_host("".join(rows).encode())
     eng.close()
@@ -127,11 +108,10 @@ def test_mixed_group_sizes_random():
         text = random_blast(rng, units, n_queries=300, max_hits=45, tie_rate=0.9)
         for strategy in ("cautious", "relaxed"):
             try:
-                want = _oracle(ids, lin, "bacteria", strategy).run_raw(text)[0]
+                want = Oracle(ids, lin, "bacteria", strategy).run_raw(text)[0]
             except OracleDataError:
                 continue
-            eng = _engine("bacteria", strategy)
-            eng.load_taxonomy_arrays(ids, lin)
+            eng = engine("bacteria", strategy, lineages=(ids, lin))
             assert eng.run_host(text).jsonl() == want
             eng.close()
             done += 1
@@ -145,13 +125,12 @@ def test_consensus_errors_on_a_reused_context():
 
     lin = ["d__bac;p__p1;c__c1", "d__arc;p__p9;c__c9", "d__bac;p__p1;c__c2"]
     ids = [1, 2, 3]
-    good = "".join(_row(f"q{i}", "A.1", 1 + 2 * (i % 2), "99.0", 100, "500") for i in range(200)).encode()
-    root = (good.decode() + _row("qr", "A.1", 1, "99.0", 100, "500") + _row("qr", "B.1", 2, "99.0", 100, "500")).encode()
-    empty = (good.decode() + _row("qe", "A.1", 1, "10.0", 100, "500")).encode()
-    many = "".join(_row(f"m{i}", f"A{i}.1", 1, "99.0", 100, "500") for i in range(60000)).encode()  # tiny rows: the arrays must grow
-    eng = _engine("bacteria", "cautious")
-    eng.load_taxonomy_arrays(ids, lin)
-    want = _oracle(ids, lin, "bacteria", "cautious").run_raw(good)[0]
+    good = "".join(hit_row(f"q{i}", "A.1", 1 + 2 * (i % 2), "99.0", 100, "500") for i in range(200)).encode()
+    root = (good.decode() + hit_row("qr", "A.1", 1, "99.0", 100, "500") + hit_row("qr", "B.1", 2, "99.0", 100, "500")).encode()
+    empty = (good.decode() + hit_row("qe", "A.1", 1, "10.0", 100, "500")).encode()
+    many = "".join(hit_row(f"m{i}", f"A{i}.1", 1, "99.0", 100, "500") for i in range(60000)).encode()  # tiny rows: the arrays must grow
+    eng = engine("bacteria", "cautious", lineages=(ids, lin))
+    want = Oracle(ids, lin, "bacteria", "cautious").run_raw(good)[0]
     for bad in (root, empty):
         assert eng.run_host(good).jsonl() == want
         with pytest.raises(ConsensusPanic):
@@ -170,12 +149,11 @@ def test_scattered_query_with_a_failing_fragment():
     failing.  The fragment's error must not abort the run before the table is known to be scattered."""
     lin = ["d__bac;p__p1;c__c1", "d__arc;p__p9;c__c9"]
     ids = [1, 2]
-    rows = [_row("qA", "A.1", 1, "99.0", 100, "100"), _row("qB", "B.1", 1, "98.0", 100, "90"), _row("qA", "A2.1", 999, "97.0", 100, "50"),
-            _row("qC", "C.1", 1, "98.0", 100, "90"), _row("qA", "A3.1", 2, "97.0", 100, "50"), _row("qA", "A4.1", 1, "97.0", 100, "50")]
+    rows = [hit_row("qA", "A.1", 1, "99.0", 100, "100"), hit_row("qB", "B.1", 1, "98.0", 100, "90"), hit_row("qA", "A2.1", 999, "97.0", 100, "50"),
+            hit_row("qC", "C.1", 1, "98.0", 100, "90"), hit_row("qA", "A3.1", 2, "97.0", 100, "50"), hit_row("qA", "A4.1", 1, "97.0", 100, "50")]
     text = "".join(rows).encode()
-    want = _oracle(ids, lin, "bacteria", "cautious").run_raw(text)[0]
-    eng = _engine("bacteria", "cautious")
-    eng.load_taxonomy_arrays(ids, lin)
+    want = Oracle(ids, lin, "bacteria", "cautious").run_raw(text)[0]
+    eng = engine("bacteria", "cautious", lineages=(ids, lin))
     out = eng.run_host(text)
     assert out.jsonl() == want
     assert int(eng.timings()["n_regrouped"]) == 2  # regrouped on the GPU
@@ -196,37 +174,12 @@ def test_windows_full_of_top_rows(group):
         t0 = rng.randrange(n_taxa)
         for h in range(group):
             t = ids[(t0 + (h % 3 if rng.random() < 0.5 else 0)) % n_taxa]
-            rows.append(_row(f"q{q:05d}", f"ACC{q}_{h}.1", t, f"{90 + (h * 7 + q) % 10}.{(q + h) % 100:02d}", 200 + h, "640"))
+            rows.append(hit_row(f"q{q:05d}", f"ACC{q}_{h}.1", t, f"{90 + (h * 7 + q) % 10}.{(q + h) % 100:02d}", 200 + h, "640"))
     text = "".join(rows).encode()
-    want = _oracle(ids, lin, "bacteria", "relaxed").run_raw(text)[0]
-    eng = _engine("bacteria", "relaxed")
-    eng.load_taxonomy_arrays(ids, lin)
+    want = Oracle(ids, lin, "bacteria", "relaxed").run_raw(text)[0]
+    eng = engine("bacteria", "relaxed", lineages=(ids, lin))
     assert eng.run_host(text).jsonl() == want
     eng.close()
-
-
-def _scattered_table(rng, n_queries, max_hits, n_taxa, blank_lines=False, final_newline=True):
-    """Rows of every query dealt out over the file in up to three far-apart fragments (file order inside a query kept)."""
-    ids = list(range(1, n_taxa + 1))
-    lin = [f"d__bac;p__p{t % 3};c__c{t % 7};o__o{t % 11};f__f{t % 13};g__g{t % 17};s__s{t}" for t in ids]
-    parts = [[], [], []]
-    for q in range(n_queries):
-        t0 = rng.randrange(n_taxa)
-        hits = rng.randint(1, max_hits)
-        for h in range(hits):
-            t = ids[(t0 + rng.choice([0, 0, 1, 2, 17])) % n_taxa]
-            bits = 900 - 10 * (h // 3) + (1 if rng.random() < 0.05 else 0)  # now and then the best row sits in a later fragment
-            row = _row(f"read_{q:06d}/1" if q % 7 else f"M0{q}:long:read:name:{q:09d}:abcdefgh", f"ACC{q}_{h}.{h % 3}", t,
-                       f"{88 + (h * 5 + q) % 12}.{(q + h) % 100:02d}", 150 + h, str(bits))
-            parts[min(2, rng.randrange(4))].append(row)
-    rows = parts[0] + parts[1] + parts[2]
-    if blank_lines:
-        for i in range(5, len(rows), 211):
-            rows[i] = "\n" + rows[i]
-    text = "".join(rows)
-    if not final_newline:
-        text = text[:-1]
-    return ids, lin, text.encode()
 
 
 @pytest.mark.parametrize("where", ["gpu", "host"])
@@ -235,32 +188,28 @@ def test_scattered_tables_regrouped(where, shape, monkeypatch):
     """Non-contiguous tables (the reference's HashMap grouping, mod.rs:145,192) through both regrouping paths: on the GPU
     (blu_regroup.cu: row index, id hash table with byte-exact check, stable radix sort, copy) and on the host; host text,
     device text and a file; against the oracle, which groups the way the reference does."""
-    import torch
-
     if where == "host":
         monkeypatch.setenv("BLU_REGROUP_HOST", "1")
     else:
         monkeypatch.delenv("BLU_REGROUP_HOST", raising=False)
     rng = random.Random(len(shape) * 31 + 5)
-    ids, lin, text = _scattered_table(rng, 60_000 if shape == "big" else 700, 9, 60, blank_lines=shape == "blank_lines",
+    ids, lin, text = scattered_table(rng, 60_000 if shape == "big" else 700, 9, 60, blank_lines=shape == "blank_lines",
                                       final_newline=shape != "no_final_newline")
-    want = _oracle(ids, lin, "bacteria", "relaxed").run_raw(text)[0]
-    eng = _engine("bacteria", "relaxed")
-    eng.load_taxonomy_arrays(ids, lin)
+    want = Oracle(ids, lin, "bacteria", "relaxed").run_raw(text)[0]
+    eng = engine("bacteria", "relaxed", lineages=(ids, lin))
     code = 2 if where == "gpu" else 1
     out = eng.run_host(text)
     assert out.jsonl() == want
     assert int(eng.timings()["n_regrouped"]) == code
     out.close()
-    t = _to_device(text)
-    out = eng.run_device(t.data_ptr(), len(text), torch.cuda.current_stream().cuda_stream)
+    t = to_device(text)
+    out = eng.run_device(t.data_ptr(), len(text), current_stream())
     assert out.jsonl() == want
     assert int(eng.timings()["n_regrouped"]) == code
     out.close()
     # a contiguous table afterwards on the same context: nothing is regrouped
-    ids2, lin2, text2 = _synth_case(5000, 300, 20, seed=3)
-    eng2 = _engine("bacteria", "relaxed")
-    eng2.load_taxonomy_arrays(ids2, lin2)
+    ids2, lin2, text2 = synth_case(5000, 300, 20, seed=3)
+    eng2 = engine("bacteria", "relaxed", lineages=(ids2, lin2))
     eng2.run_host(text2).close()
     assert int(eng2.timings()["n_regrouped"]) == 0
     eng2.close()
@@ -269,12 +218,11 @@ def test_scattered_tables_regrouped(where, shape, monkeypatch):
 
 def test_scattered_table_from_a_file(tmp_path):
     rng = random.Random(99)
-    ids, lin, text = _scattered_table(rng, 3000, 6, 40)
-    want = _oracle(ids, lin, "bacteria", "cautious").run_raw(text)[0]
+    ids, lin, text = scattered_table(rng, 3000, 6, 40)
+    want = Oracle(ids, lin, "bacteria", "cautious").run_raw(text)[0]
     path = tmp_path / "scattered.blast.out"
     path.write_bytes(text)
-    eng = _engine("bacteria", "cautious")
-    eng.load_taxonomy_arrays(ids, lin)
+    eng = engine("bacteria", "cautious", lineages=(ids, lin))
     out = eng.run_file(str(path))
     assert out.jsonl() == want
     assert int(eng.timings()["n_regrouped"]) == 2
@@ -289,12 +237,11 @@ def test_scattered_table_device_resident():
     import torch
 
     rng = random.Random(4711)
-    ids, lin, text = _scattered_table(rng, 5000, 8, 50)
-    want = _oracle(ids, lin, "bacteria", "relaxed").run_raw(text)[0]
-    eng = _engine("bacteria", "relaxed")
-    eng.load_taxonomy_arrays(ids, lin)
-    t = _to_device(text)
-    out = eng.run_device_resident(t.data_ptr(), len(text), torch.cuda.current_stream().cuda_stream)
+    ids, lin, text = scattered_table(rng, 5000, 8, 50)
+    want = Oracle(ids, lin, "bacteria", "relaxed").run_raw(text)[0]
+    eng = engine("bacteria", "relaxed", lineages=(ids, lin))
+    t = to_device(text)
+    out = eng.run_device_resident(t.data_ptr(), len(text), current_stream())
     assert int(eng.timings()["n_regrouped"]) == 2
     ptr, n = out.device_text()
     assert ptr and ptr != t.data_ptr() and n >= len(text)  # (every row newline-terminated; nothing else changes)
@@ -303,11 +250,10 @@ def test_scattered_table_device_resident():
     assert out.download().jsonl() == want
     out.close()
     # contiguous table: the references point into the caller's text
-    ids2, lin2, text2 = _synth_case(5000, 300, 20, seed=3)
-    eng2 = _engine("bacteria", "relaxed")
-    eng2.load_taxonomy_arrays(ids2, lin2)
-    t2 = _to_device(text2)
-    out2 = eng2.run_device_resident(t2.data_ptr(), len(text2), torch.cuda.current_stream().cuda_stream)
+    ids2, lin2, text2 = synth_case(5000, 300, 20, seed=3)
+    eng2 = engine("bacteria", "relaxed", lineages=(ids2, lin2))
+    t2 = to_device(text2)
+    out2 = eng2.run_device_resident(t2.data_ptr(), len(text2), current_stream())
     assert out2.device_text() == (t2.data_ptr(), len(text2))
     out2.close()
     eng2.close()
@@ -324,16 +270,15 @@ def test_fully_tied_beans(group):
     rows = []
     for q in range(50):
         for h in range(group):
-            rows.append(_row(f"q{q:03d}", f"A{q}_{h}.1", 1 + (h + q) % 3, "91.5", 300, "700"))
-        rows.append(_row(f"q{q:03d}", f"L{q}.1", 4, "80.0", 300, "100"))
+            rows.append(hit_row(f"q{q:03d}", f"A{q}_{h}.1", 1 + (h + q) % 3, "91.5", 300, "700"))
+        rows.append(hit_row(f"q{q:03d}", f"L{q}.1", 4, "80.0", 300, "100"))
     text = "".join(rows).encode()
     for order in ([1, 2, 3, 4], [3, 2, 1, 4], [2, 4, 3, 1]):
         ids = order
         lin = [lineages[i] for i in order]
         for strategy in ("cautious", "relaxed"):
-            want = _oracle(ids, lin, "bacteria", strategy).run_raw(text)[0]
-            eng = _engine("bacteria", strategy)
-            eng.load_taxonomy_arrays(ids, lin)
+            want = Oracle(ids, lin, "bacteria", strategy).run_raw(text)[0]
+            eng = engine("bacteria", strategy, lineages=(ids, lin))
             assert eng.run_host(text).jsonl() == want, (order, strategy)
             eng.close()
     first = [json.loads(l)["taxon"]["consensusBeans"][0]["rank"] for l in want.decode().splitlines()[:1]]

@@ -10,32 +10,12 @@ import random
 
 import pytest
 
-from helpers import random_blast, random_taxonomy
-from test_gpu_file_stream import IDS, LIN, _row, _table
+from helpers import (CHUNK, COUNTERS_BYTES, CUTOFFS_16S, IDS, LIN, current_stream, engine, hit_row, hit_table, random_blast, random_taxonomy,
+                     tiny_rows, to_device)
 
 pytestmark = pytest.mark.gpu
 
-YAML16S = {"domain": 50, "kingdom": 60, "phylum": 75, "class": 80, "order": 85, "family": 92, "genus": 97, "species": 99}
-STRICT = {k: 96 for k in YAML16S}  # an identity below 96 % misses every cutoff
-COUNTERS_BYTES = 120
-CHUNK = 1 << 20
-
-
-def _ct(d):
-    from blutils_b200 import CustomTaxon
-
-    return CustomTaxon(domain=d["domain"], kingdom=d["kingdom"], phylum=d["phylum"], class_=d["class"], order=d["order"], family=d["family"],
-                       genus=d["genus"], species=d["species"])
-
-
-def _engine(ids, lin, taxon, strategy, custom=None, numeric=False, chunk_bytes=0, text_refs=False):
-    from blutils_b200 import ConsensusEngine, ConsensusStrategy, Taxon
-
-    eng = ConsensusEngine({"bacteria": Taxon.Bacteria, "custom": Taxon.Custom}[taxon],
-                          {"cautious": ConsensusStrategy.Cautious, "relaxed": ConsensusStrategy.Relaxed}[strategy], numeric,
-                          _ct(custom) if custom else None, chunk_bytes=chunk_bytes, text_refs=text_refs)
-    eng.load_taxonomy_arrays(ids, lin)
-    return eng
+STRICT = {k: 96 for k in CUTOFFS_16S}  # an identity below 96 % misses every cutoff
 
 
 class Group:
@@ -46,7 +26,7 @@ class Group:
 
         self.engines, self.oracles = [], []
         for ids, lin, taxon, strategy, custom, numeric in specs:
-            self.engines.append(_engine(ids, lin, taxon, strategy, custom, numeric, chunk_bytes, text_refs))
+            self.engines.append(engine(taxon, strategy, numeric, custom, chunk_bytes=chunk_bytes, text_refs=text_refs, lineages=(ids, lin)))
             self.oracles.append(Oracle(ids, lin, taxon, strategy, custom))
 
     def close(self):
@@ -63,30 +43,14 @@ def _knobs(chunk_bytes=0, seed=20261020):
     for numeric in (False, True):
         ids, off, blob = w.lineages(numeric=numeric)
         lins[numeric] = (ids.tolist(), [bytes(blob[int(off[i]):int(off[i + 1])]).decode() for i in range(len(ids))])
-    specs = [(*lins[numeric], taxon, strategy, YAML16S if taxon == "custom" else None, numeric)
+    specs = [(*lins[numeric], taxon, strategy, CUTOFFS_16S if taxon == "custom" else None, numeric)
              for numeric in (False, True) for taxon in ("bacteria", "custom") for strategy in ("cautious", "relaxed")]
     return w, Group(specs, chunk_bytes)
 
 
-def _small_specs(custom=YAML16S):
+def _small_specs(custom=CUTOFFS_16S):
     return [(IDS, LIN, "bacteria", "cautious", None, False), (IDS, LIN, "bacteria", "relaxed", None, False),
             (IDS, LIN, "custom", "cautious", custom, False), (IDS, LIN, "custom", "relaxed", custom, False)]
-
-
-def _to_device(text):
-    import torch
-
-    n = len(text)
-    t = torch.zeros((n + 255) // 128 * 128, dtype=torch.uint8, device="cuda")
-    t[:n] = torch.frombuffer(bytearray(text), dtype=torch.uint8).cuda()
-    torch.cuda.synchronize()
-    return t
-
-
-def _stream():
-    import torch
-
-    return torch.cuda.current_stream().cuda_stream
 
 
 def _run(kind, engines, text, tmp_path, dev=None):
@@ -99,8 +63,8 @@ def _run(kind, engines, text, tmp_path, dev=None):
         path = tmp_path / "blast.out"
         path.write_bytes(text)
         return run_file_configs(engines, str(path))
-    t = _to_device(text) if dev is None else dev
-    outs = run_device_resident_configs(engines, t.data_ptr(), len(text), _stream())
+    t = to_device(text) if dev is None else dev
+    outs = run_device_resident_configs(engines, t.data_ptr(), len(text), current_stream())
     for o in outs:
         o.download()
     return outs
@@ -113,8 +77,8 @@ def _single(kind, eng, text, tmp_path):
         path = tmp_path / "single.out"
         path.write_bytes(text)
         return eng.run_file(str(path))
-    t = _to_device(text)
-    return eng.run_device_resident(t.data_ptr(), len(text), _stream()).download()
+    t = to_device(text)
+    return eng.run_device_resident(t.data_ptr(), len(text), current_stream()).download()
 
 
 def _check_group(g, outs, text, tmp_path, kind):
@@ -147,8 +111,8 @@ def _size_classes():
         bits = "950" if q % 2 else "3000000000"
         for h in range(g + 3):
             top = h < g
-            rows.append(_row(f"sz_{q:03d}", f"NR_{(q * 7 + h) % 500:06d}.1", IDS[(q + h) % 4] if q % 3 else IDS[h % 2],
-                             f"{90 + h % 10}.{(q + h) % 1000:03d}", 300 + h % 50, bits if top else str(100 + h % 300)))
+            rows.append(hit_row(f"sz_{q:03d}", f"NR_{(q * 7 + h) % 500:06d}.1", IDS[(q + h) % 4] if q % 3 else IDS[h % 2],
+                             f"{90 + h % 10}.{(q + h) % 1000:03d}", 300 + h % 50, bits if top else str(100 + h % 300), mismatch=3, sstart=17, evalue="1e-50"))
     return "".join(rows).encode()
 
 
@@ -162,18 +126,10 @@ def test_every_top_group_size_class(tmp_path, kind):
     g.close()
 
 
-def _tiny_rows():
-    rows = []
-    for q in range(120000):
-        for h in range(1 + (q % 5 == 0)):
-            rows.append(f"q{q}\tA\t{IDS[q % 2]}\t9{h}\t{1 + q % 9}\t0\t0\t1\t1\t1\t1\t0\t{5 + (q + h) % 3}\n")
-    return "".join(rows).encode()
-
-
 @pytest.mark.parametrize("kind", ["host", "file", "resident"])
 def test_capacity_retry_on_fresh_contexts(tmp_path, kind):
     """More queries than a fresh context's first estimate: the whole pass runs again with grown capacities."""
-    text = _tiny_rows()
+    text = tiny_rows()
     g = Group(_small_specs(), chunk_bytes=CHUNK)
     outs = _run(kind, g.engines, text, tmp_path)
     for k, (orc, out) in enumerate(zip(g.oracles, outs)):
@@ -186,7 +142,7 @@ def _scattered():
     units = random_taxonomy(rng, n_leaves=40)
     text = random_blast(rng, units, n_queries=400, max_hits=12, contiguous=False)
     ids = [u["taxid"] for u in units]
-    specs = [(ids, [u["numericLineage" if numeric else "textLineage"] for u in units], taxon, strategy, YAML16S if taxon == "custom" else None,
+    specs = [(ids, [u["numericLineage" if numeric else "textLineage"] for u in units], taxon, strategy, CUTOFFS_16S if taxon == "custom" else None,
               numeric) for numeric in (False, True) for taxon, strategy in (("bacteria", "cautious"), ("custom", "relaxed"))]
     return text, specs
 
@@ -207,8 +163,8 @@ def test_scattered_resident_results_share_the_regrouped_text(tmp_path):
 
     text, specs = _scattered()
     g = Group(specs)
-    t = _to_device(text)
-    outs = run_device_resident_configs(g.engines, t.data_ptr(), len(text), _stream())
+    t = to_device(text)
+    outs = run_device_resident_configs(g.engines, t.data_ptr(), len(text), current_stream())
     texts = {o.device_text() for o in outs}
     assert len(texts) == 1
     ptr, n = texts.pop()
@@ -224,7 +180,7 @@ def test_scattered_resident_results_share_the_regrouped_text(tmp_path):
 def test_text_references_point_into_the_callers_text():
     from blutils_b200 import _ffi, run_host_configs
 
-    text = _table(900, 0, seed=3)
+    text = hit_table(900, 0, seed=3)
     buf = C.create_string_buffer(text, len(text))
     g = Group(_small_specs(), chunk_bytes=CHUNK, text_refs=True)
     outs = run_host_configs(g.engines, C.addressof(buf), len(text))
@@ -244,7 +200,7 @@ def test_text_references_point_into_the_callers_text():
 def test_grammar_error_fails_the_call(tmp_path):
     from blutils_b200 import ConsensusPanic, run_file_configs, run_host_configs
 
-    text = _table(50, 0, seed=5) + b"broken\trow\n" + _table(5, 0, seed=6)
+    text = hit_table(50, 0, seed=5) + b"broken\trow\n" + hit_table(5, 0, seed=6)
     g = Group(_small_specs())
     with pytest.raises(ConsensusPanic) as single:
         g.engines[2].run_host(text)
@@ -265,8 +221,9 @@ def test_consensus_error_of_one_configuration_names_it(tmp_path, kind):
     from blutils_b200 import ConsensusPanic
     from oracle_ffi import OracleDataError
 
-    text = (_row("qa", "NR_1.1", IDS[0], "95.5", 300, "900") +
-            "".join(_row(f"q{q}", f"NR_{q}.{h}", IDS[(q + h) % 4], f"9{7 + h % 3}.5", 300, str(900 - h)) for q in range(30) for h in range(4))).encode()
+    text = (hit_row("qa", "NR_1.1", IDS[0], "95.5", 300, "900", mismatch=3, sstart=17, evalue="1e-50") +
+            "".join(hit_row(f"q{q}", f"NR_{q}.{h}", IDS[(q + h) % 4], f"9{7 + h % 3}.5", 300, str(900 - h), mismatch=3, sstart=17, evalue="1e-50")
+                    for q in range(30) for h in range(4))).encode()
     g = Group([(IDS, LIN, "bacteria", "relaxed", None, False), (IDS, LIN, "custom", "cautious", STRICT, False),
                (IDS, LIN, "custom", "relaxed", STRICT, False)])
     assert g.oracles[0].run_raw(text)[1] == 31
@@ -290,16 +247,15 @@ def eng_error(eng):
 
 
 def test_bad_groups_are_refused():
-    from blutils_b200 import ConsensusEngine, ConsensusStrategy, Taxon, _ffi, run_host_configs
+    from blutils_b200 import _ffi, run_host_configs
 
-    text = _table(20, 0, seed=4)
-    a = _engine(IDS, LIN, "bacteria", "relaxed")
-    b = _engine(IDS, LIN, "bacteria", "cautious")
-    other_chunk = _engine(IDS, LIN, "bacteria", "cautious", chunk_bytes=CHUNK)
-    other_flags = _engine(IDS, LIN, "bacteria", "cautious", text_refs=True)
-    no_tax = ConsensusEngine(Taxon.Bacteria, ConsensusStrategy.Relaxed, False, None)
-    multi = ConsensusEngine(Taxon.Bacteria, ConsensusStrategy.Relaxed, False, None, devices=[0])
-    multi.load_taxonomy_arrays(IDS, LIN)
+    text = hit_table(20, 0, seed=4)
+    a = engine("bacteria", "relaxed", lineages=(IDS, LIN))
+    b = engine("bacteria", "cautious", lineages=(IDS, LIN))
+    other_chunk = engine("bacteria", "cautious", chunk_bytes=CHUNK, lineages=(IDS, LIN))
+    other_flags = engine("bacteria", "cautious", text_refs=True, lineages=(IDS, LIN))
+    no_tax = engine("bacteria", "relaxed")
+    multi = engine("bacteria", "relaxed", devices=[0], lineages=(IDS, LIN))
     cases = [([a, a], "ctxs[1]: the same context as ctxs[0]"), ([a, multi], "ctxs[1]: a multi-device context"),
              ([a, no_tax], "ctxs[1]: no taxonomy loaded"), ([a, other_chunk], "ctxs[1]: chunk_bytes differs"),
              ([a, other_flags], "ctxs[1]: flags differ"), ([a, b] * 4 + [a], "a group holds 1 to 8 contexts")]
@@ -323,7 +279,7 @@ def test_bad_groups_are_refused():
 @pytest.mark.parametrize("kind", ["host", "file"])
 def test_the_pass_is_shared(tmp_path, kind):
     """Host text and files cross PCIe once: the group copies and tiles what one single run does."""
-    text = _table(900, 0, seed=3)
+    text = hit_table(900, 0, seed=3)
     chunks = (len(text) + CHUNK - 1) // CHUNK
     assert chunks > 2
     g = Group(_small_specs(), chunk_bytes=CHUNK)
@@ -345,12 +301,12 @@ def test_the_pass_is_shared(tmp_path, kind):
 
 
 def test_resident_timings():
-    text = _table(900, 0, seed=3)
+    text = hit_table(900, 0, seed=3)
     g = Group(_small_specs())
-    t = _to_device(text)
+    t = to_device(text)
     from blutils_b200 import run_device_resident_configs
 
-    outs = run_device_resident_configs(g.engines, t.data_ptr(), len(text), _stream())
+    outs = run_device_resident_configs(g.engines, t.data_ptr(), len(text), current_stream())
     K = len(outs)
     for eng in g.engines:
         tm = eng.timings()
@@ -365,12 +321,12 @@ def test_sort_and_headers_as_for_single_runs(tmp_path):
 
     w, g = _knobs(seed=11)
     text = w.hits(0, 3000, 20)
-    t = _to_device(text)
-    outs = run_device_resident_configs(g.engines, t.data_ptr(), len(text), _stream())
+    t = to_device(text)
+    outs = run_device_resident_configs(g.engines, t.data_ptr(), len(text), current_stream())
     headers = [f"absent_{i}" for i in range(5)]
     for k, (eng, orc, out) in enumerate(zip(g.engines, g.oracles, outs)):
         out.sort_by_query().download()
-        single = eng.run_device_resident(t.data_ptr(), len(text), _stream()).sort_by_query().download()
+        single = eng.run_device_resident(t.data_ptr(), len(text), current_stream()).sort_by_query().download()
         assert out.query_ids() == single.query_ids() == sorted(single.query_ids()), f"configuration {k}"
         out.add_headers(headers)
         single.add_headers(headers)
@@ -383,7 +339,7 @@ def test_sort_and_headers_as_for_single_runs(tmp_path):
     # a result is sorted with its own context only
     from blutils_b200 import _ffi
 
-    other = run_device_resident_configs(g.engines[:2], t.data_ptr(), len(text), _stream())
+    other = run_device_resident_configs(g.engines[:2], t.data_ptr(), len(text), current_stream())
     assert _ffi.lib().blu_result_sort_by_query(g.engines[0]._h, other[1]._h) == _ffi.BLU_ERR_ARG
     assert _ffi.lib().blu_result_sort_by_query(g.engines[1]._h, other[1]._h) == 0
     for o in other:

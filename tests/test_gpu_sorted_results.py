@@ -7,9 +7,8 @@ import random
 import numpy as np
 import pytest
 
-from test_gpu_multi import _device_sets, _multi
-from test_gpu_parity import _engine, _oracle, _row
-from test_gpu_round2 import _scattered_table, _to_device
+from helpers import current_stream, device_sets, engine, hit_row, scattered_table, synth_case, to_device
+from oracle_ffi import Oracle
 
 pytestmark = pytest.mark.gpu
 
@@ -83,7 +82,7 @@ def _table(query_ids, seed=5):
     rows = []
     for k, q in enumerate(query_ids):
         for h in range(rng.randint(1, 4)):
-            rows.append(_row("\x00", f"ACC{k % 97}_{h}.1", ids[(k + h) % 4], f"{90 + (k + h) % 10}.5", 150, str(800 - 7 * h)).encode().replace(b"\x00", q))
+            rows.append(hit_row("\x00", f"ACC{k % 97}_{h}.1", ids[(k + h) % 4], f"{90 + (k + h) % 10}.5", 150, str(800 - 7 * h)).encode().replace(b"\x00", q))
     return ids, lin, b"".join(rows)
 
 
@@ -94,46 +93,31 @@ def _run_both(eng, run):
 # --- 1. every producing path ------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("text_refs", [False, True])
 def test_run_host_sorted(text_refs, tmp_path):
-    from blutils_b200 import ConsensusEngine, ConsensusStrategy, Taxon
-
-    from test_gpu_parity import _synth_case
-
-    ids, lin, text = _synth_case(5000, 4000, 30, seed=23)
-    eng = ConsensusEngine(Taxon.Bacteria, ConsensusStrategy.Relaxed, False, None, text_refs=text_refs)
-    eng.load_taxonomy_arrays(ids, lin)
+    ids, lin, text = synth_case(5000, 4000, 30, seed=23)
+    eng = engine("bacteria", "relaxed", text_refs=text_refs, lineages=(ids, lin))
     a, b = _run_both(eng, lambda e: e.run_host(text))
     _check(a, b, tmp_path)
-    assert a.jsonl() == _oracle(ids, lin, "bacteria", "relaxed").run_raw(text)[0]
+    assert a.jsonl() == Oracle(ids, lin, "bacteria", "relaxed").run_raw(text)[0]
 
 
 def test_run_file_and_device_sorted(tmp_path):
-    import torch
-
-    from test_gpu_parity import _synth_case
-
-    ids, lin, text = _synth_case(5000, 6000, 20, seed=29)
+    ids, lin, text = synth_case(5000, 6000, 20, seed=29)
     path = tmp_path / "t.blast.out"
     path.write_bytes(text)
-    eng = _engine("bacteria", "cautious")
-    eng.load_taxonomy_arrays(ids, lin)
+    eng = engine("bacteria", "cautious", lineages=(ids, lin))
     a, b = _run_both(eng, lambda e: e.run_file(str(path)))
     _check(a, b, tmp_path)
-    t = _to_device(text)
-    s = torch.cuda.current_stream().cuda_stream
+    t = to_device(text)
+    s = current_stream()
     a, b = _run_both(eng, lambda e: e.run_device(t.data_ptr(), len(text), s))
     _check(a, b, tmp_path)
 
 
 def test_device_resident_sorted_before_download(tmp_path):
-    import torch
-
-    from test_gpu_parity import _synth_case
-
-    ids, lin, text = _synth_case(5000, 20000, 10, seed=31)
-    eng = _engine("bacteria", "relaxed")
-    eng.load_taxonomy_arrays(ids, lin)
-    t = _to_device(text)
-    s = torch.cuda.current_stream().cuda_stream
+    ids, lin, text = synth_case(5000, 20000, 10, seed=31)
+    eng = engine("bacteria", "relaxed", lineages=(ids, lin))
+    t = to_device(text)
+    s = current_stream()
     a = eng.run_device_resident(t.data_ptr(), len(text), s).download()
     b = eng.run_device_resident(t.data_ptr(), len(text), s)
     b.sort_by_query()
@@ -145,18 +129,12 @@ def test_device_resident_sorted_before_download(tmp_path):
 
 
 def test_device_resident_needs_its_own_context():
-    import torch
-
     from blutils_b200 import _ffi
 
-    from test_gpu_parity import _synth_case
-
-    ids, lin, text = _synth_case(500, 300, 5, seed=3)
-    e1, e2 = _engine("bacteria", "relaxed"), _engine("bacteria", "relaxed")
-    for e in (e1, e2):
-        e.load_taxonomy_arrays(ids, lin)
-    t = _to_device(text)
-    out = e1.run_device_resident(t.data_ptr(), len(text), torch.cuda.current_stream().cuda_stream)
+    ids, lin, text = synth_case(500, 300, 5, seed=3)
+    e1, e2 = engine("bacteria", "relaxed", lineages=(ids, lin)), engine("bacteria", "relaxed", lineages=(ids, lin))
+    t = to_device(text)
+    out = e1.run_device_resident(t.data_ptr(), len(text), current_stream())
     assert _ffi.lib().blu_result_sort_by_query(e2._h, out._h) == _ffi.BLU_ERR_ARG
     out.sort_by_query()
     _assert_strictly_increasing(_device_ids(out))
@@ -173,7 +151,7 @@ def _accepted_control_bytes():
             continue
         ids, lin, text = _table([b"ctl" + bytes([c]) + b"x"])
         try:
-            _oracle(ids, lin, "bacteria", "relaxed").run_raw(text)
+            Oracle(ids, lin, "bacteria", "relaxed").run_raw(text)
         except OracleDataError:
             continue
         ok.append(c)
@@ -212,12 +190,9 @@ def test_adversarial_ids(tmp_path):
     qids = sorted(ids_set)
     rng.shuffle(qids)
     ids, lin, text = _table(qids)
-    want = _oracle(ids, lin, "bacteria", "relaxed").run_raw(text)[0]
+    want = Oracle(ids, lin, "bacteria", "relaxed").run_raw(text)[0]
     for refs in (False, True):
-        from blutils_b200 import ConsensusEngine, ConsensusStrategy, Taxon
-
-        eng = ConsensusEngine(Taxon.Bacteria, ConsensusStrategy.Relaxed, False, None, text_refs=refs)
-        eng.load_taxonomy_arrays(ids, lin)
+        eng = engine("bacteria", "relaxed", text_refs=refs, lineages=(ids, lin))
         a, b = _run_both(eng, lambda e: e.run_host(text))
         assert a.jsonl() == want
         assert b.query_ids() == sorted(qids)
@@ -226,8 +201,7 @@ def test_adversarial_ids(tmp_path):
 
 def test_single_query(tmp_path):
     ids, lin, text = _table([b"only-one"])
-    eng = _engine("bacteria", "relaxed")
-    eng.load_taxonomy_arrays(ids, lin)
+    eng = engine("bacteria", "relaxed", lineages=(ids, lin))
     a, b = _run_both(eng, lambda e: e.run_host(text))
     assert b.query_ids() == [b"only-one"]
     _check(a, b, tmp_path)
@@ -238,8 +212,7 @@ def test_reverse_file_order(tmp_path):
     qids = sorted({b"%s%06d" % (p, i) for i in range(34000) for p in (b"SRR0000", b"SRR00001", b"M0001:12:000000000")})[:100_000]
     qids.reverse()
     ids, lin, text = _table(qids)
-    eng = _engine("bacteria", "relaxed")
-    eng.load_taxonomy_arrays(ids, lin)
+    eng = engine("bacteria", "relaxed", lineages=(ids, lin))
     a, b = _run_both(eng, lambda e: e.run_host(text))
     assert b.query_ids() == qids[::-1]
     _check(a, b, tmp_path)
@@ -247,14 +220,11 @@ def test_reverse_file_order(tmp_path):
 
 # --- 3. a scattered table, device-resident --------------------------------------------------------------------------
 def test_scattered_table_device_resident_sorted(tmp_path):
-    import torch
-
     rng = random.Random(4711)
-    ids, lin, text = _scattered_table(rng, 5000, 8, 50)
-    eng = _engine("bacteria", "relaxed")
-    eng.load_taxonomy_arrays(ids, lin)
-    t = _to_device(text)
-    s = torch.cuda.current_stream().cuda_stream
+    ids, lin, text = scattered_table(rng, 5000, 8, 50)
+    eng = engine("bacteria", "relaxed", lineages=(ids, lin))
+    t = to_device(text)
+    s = current_stream()
     a = eng.run_host(text)
     b = eng.run_device_resident(t.data_ptr(), len(text), s)
     assert int(eng.timings()["n_regrouped"]) == 2
@@ -274,8 +244,7 @@ def test_hitless_headers(when, tmp_path):
     random.Random(8).shuffle(qids)
     ids, lin, text = _table(qids)
     headers = ["read_0001", "read_1999", "read_0000", "read_0001", "aaa", "zzz", "read_0500x", "read_0500"]  # between records, dups, a record's id
-    eng = _engine("bacteria", "relaxed")
-    eng.load_taxonomy_arrays(ids, lin)
+    eng = engine("bacteria", "relaxed", lineages=(ids, lin))
     a = eng.run_host(text)
     a.add_headers(headers)
     b = eng.run_host(text)
@@ -293,14 +262,11 @@ def test_hitless_headers(when, tmp_path):
 
 # --- 5. multi-device contexts ----------------------------------------------------------------------------------------
 def test_multi_device_sorted_equals_single(tmp_path):
-    from test_gpu_parity import _synth_case
-
-    ids, lin, text = _synth_case(5000, 30000, 8, seed=37)
+    ids, lin, text = synth_case(5000, 30000, 8, seed=37)
     ref = None
-    for devs in _device_sets():
+    for devs in device_sets():
         for refs in (False, True):
-            eng = _multi(devs, text_refs=refs)
-            eng.load_taxonomy_arrays(ids, lin)
+            eng = engine("bacteria", "relaxed", devices=devs, text_refs=refs, lineages=(ids, lin))
             a, b = _run_both(eng, lambda e: e.run_host(text))
             if ref is None:
                 ref = b.query_ids()
@@ -311,15 +277,10 @@ def test_multi_device_sorted_equals_single(tmp_path):
 
 # --- 6. determinism --------------------------------------------------------------------------------------------------
 def test_two_runs_same_order():
-    import torch
-
-    from test_gpu_parity import _synth_case
-
-    ids, lin, text = _synth_case(5000, 20000, 10, seed=41)
-    eng = _engine("bacteria", "relaxed")
-    eng.load_taxonomy_arrays(ids, lin)
-    t = _to_device(text)
-    s = torch.cuda.current_stream().cuda_stream
+    ids, lin, text = synth_case(5000, 20000, 10, seed=41)
+    eng = engine("bacteria", "relaxed", lineages=(ids, lin))
+    t = to_device(text)
+    s = current_stream()
     seqs = []
     for _ in range(2):
         out = eng.run_device_resident(t.data_ptr(), len(text), s).sort_by_query()

@@ -7,30 +7,14 @@ import random
 
 import pytest
 
+from helpers import IDS5, LIN5, current_stream, engine, hit_row, synth_case, to_device
+from oracle_ffi import Oracle, checksum_jsonl
+
 pytestmark = pytest.mark.gpu
-
-LIN = ["d__bac;p__p1;c__c1;o__o1;f__f1;g__g1;s__s1", "d__bac;p__p1;c__c1;o__o1;f__f1;g__g1;s__s2", "d__bac;p__p1;c__c1;o__o1;f__f1;g__g2;s__s3",
-       "d__bac;p__p1;c__c1;o__o1;f__f2;g__g3;s__s4", "d__bac;p__p2;c__c2;o__o2;f__f3;g__g4;s__s5"]
-IDS = [7, 4242, 1660760528, 99999999, 1234567890123456]  # 1 .. 16 digits (lean splitter: <= 8, <= 16, beyond)
-
-
-def _engine(strategy="relaxed", chunk_bytes=0):
-    from blutils_b200 import ConsensusEngine, ConsensusStrategy, Taxon
-
-    eng = ConsensusEngine(Taxon.Bacteria, {"cautious": ConsensusStrategy.Cautious, "relaxed": ConsensusStrategy.Relaxed}[strategy], False, None,
-                          chunk_bytes=chunk_bytes)
-    eng.load_taxonomy_arrays(IDS, LIN)
-    return eng
 
 
 def _want(text, strategy="relaxed"):
-    from oracle_ffi import Oracle
-
-    return Oracle(IDS, LIN, "bacteria", strategy).run_raw(text)[0]
-
-
-def _row(q, acc, taxid, pident, ln, bits, evalue="0.0"):
-    return f"{q}\t{acc}\t{taxid}\t{pident}\t{ln}\t3\t0\t1\t{ln}\t17\t{ln + 16}\t{evalue}\t{bits}\n"
+    return Oracle(IDS5, LIN5, "bacteria", strategy).run_raw(text)[0]
 
 
 def _check(text, strategies=("relaxed", "cautious"), chunks=(0,)):
@@ -39,7 +23,7 @@ def _check(text, strategies=("relaxed", "cautious"), chunks=(0,)):
     for st in strategies:
         want = _want(text, st)
         for ch in chunks:
-            eng = _engine(st, ch)
+            eng = engine("bacteria", st, chunk_bytes=ch, lineages=(IDS5, LIN5))
             assert eng.run_host(text).jsonl() == want, (st, ch)
             eng.close()
 
@@ -54,7 +38,8 @@ def test_best_score_found_in_a_later_window():
         best = sorted(rng.sample(range(n), rng.choice([1, 2, 5, 9])))
         for h in range(n):
             bits = "900" if h in best else str(100 + (h * 7 + q) % 700)
-            rows.append(_row(f"query_{q:05d}", f"NR_{(q * 31 + h) % 1000:06d}.1", IDS[(q + h) % 4], f"{90 + (h % 10)}.{h % 1000:03d}", 400 + h % 50, bits))
+            rows.append(hit_row(f"query_{q:05d}", f"NR_{(q * 31 + h) % 1000:06d}.1", IDS5[(q + h) % 4], f"{90 + (h % 10)}.{h % 1000:03d}", 400 + h % 50, bits,
+                                mismatch=3, sstart=17))
     _check("".join(rows), chunks=(0, 1 << 20))
 
 
@@ -66,10 +51,10 @@ def test_carried_top_group_overflows_to_the_block_path():
         n = 1300
         tops = set(range(0, n, 33)) if q % 3 == 0 else {5, 700}
         for h in range(n):
-            rows.append(_row(f"q{q:03d}", f"ACC{h % 9}.1", IDS[h % 3], "98.500", 300, "500" if h in tops else str(50 + h % 400)))
+            rows.append(hit_row(f"q{q:03d}", f"ACC{h % 9}.1", IDS5[h % 3], "98.500", 300, "500" if h in tops else str(50 + h % 400), mismatch=3, sstart=17))
     text = "".join(rows)
     want = _want(text.encode())
-    eng = _engine()
+    eng = engine("bacteria", "relaxed", lineages=(IDS5, LIN5))
     assert eng.run_host(text.encode()).jsonl() == want
     assert eng.timings()["n_deferred_runs"] >= 4  # the four 40-row top groups really took the block path
     eng.close()
@@ -82,7 +67,7 @@ def test_windows_full_of_tiny_queries():
     rows = []
     for q in range(60000):
         for h in range(1 + (q % 7 == 0)):
-            rows.append(f"q{q}\tA\t{IDS[q % 2]}\t9{h}\t{1 + q % 9}\t0\t0\t1\t1\t1\t1\t0\t{5 + (q + h) % 3}\n")
+            rows.append(f"q{q}\tA\t{IDS5[q % 2]}\t9{h}\t{1 + q % 9}\t0\t0\t1\t1\t1\t1\t0\t{5 + (q + h) % 3}\n")
     rng.random()
     _check("".join(rows), strategies=("relaxed",), chunks=(0, 1 << 20))
 
@@ -98,7 +83,7 @@ def test_number_shapes_lean_and_fallback():
         for bits in bitss:
             ev = evalues[q % len(evalues)]
             for h in range(3):
-                rows.append(_row(f"q{q:04d}", f"WP_{q}.{h}", IDS[(q + h) % 5], pid, 250 + h, bits, ev))
+                rows.append(hit_row(f"q{q:04d}", f"WP_{q}.{h}", IDS5[(q + h) % 5], pid, 250 + h, bits, mismatch=3, sstart=17, evalue=ev))
             q += 1
     _check("".join(rows))
 
@@ -110,31 +95,19 @@ def test_non_ascii_and_long_identifiers():
         name = ["müller_%d" % q, "q%d_" % q + "x" * 40, "漢字_%d" % q, "r%d_" % q + "y" * 90][q % 4]
         for h in range(20):
             acc = "ACC_é%d.1" % (h % 3) if q % 5 == 0 else "NR_%06d.1" % h
-            rows.append(_row(name, acc, IDS[h % 4], "97.125", 300, "450" if h < 2 else str(100 + h)))
+            rows.append(hit_row(name, acc, IDS5[h % 4], "97.125", 300, "450" if h < 2 else str(100 + h), mismatch=3, sstart=17))
     _check("".join(rows).encode("utf-8"))
 
 
 def test_large_table_is_deterministic():
     """A 200 MB device-resident table run five times: identical checksums (a race between phases / windows would show up
     as a varying result), equal to the oracle's."""
-    import torch
-    from blutils_b200 import ConsensusEngine, ConsensusStrategy, Taxon
-    from blutils_b200.synth import SynthWorkload
-    from oracle_ffi import Oracle, checksum_jsonl
-
-    w = SynthWorkload(20000, seed=77)
-    ids, off, blob = w.lineages()
-    lin = [bytes(blob[int(off[i]):int(off[i + 1])]).decode() for i in range(len(ids))]
-    text = w.hits(0, 52000, 50)
-    want = checksum_jsonl(Oracle(ids.tolist(), lin, "bacteria", "relaxed").run_raw(text)[0])
-    eng = ConsensusEngine(Taxon.Bacteria, ConsensusStrategy.Relaxed, False, None)
-    eng.load_taxonomy_arrays(ids.tolist(), lin)
-    n = len(text)
-    t = torch.zeros((n + 255) // 128 * 128, dtype=torch.uint8, device="cuda")
-    t[:n] = torch.frombuffer(bytearray(text), dtype=torch.uint8).cuda()
-    torch.cuda.synchronize()
+    ids, lin, text = synth_case(20000, 52000, 50, seed=77)
+    want = checksum_jsonl(Oracle(ids, lin, "bacteria", "relaxed").run_raw(text)[0])
+    eng = engine("bacteria", "relaxed", lineages=(ids, lin))
+    t = to_device(text)
     for _ in range(5):
-        out = eng.run_device(t.data_ptr(), n, torch.cuda.current_stream().cuda_stream)
+        out = eng.run_device(t.data_ptr(), len(text), current_stream())
         assert len(out) == 52000 and out.checksum() == want
         out.close()
     eng.close()
@@ -146,11 +119,11 @@ def test_query_spanning_many_segments():
     rows = []
     for q in range(40):
         for h in range(30):
-            rows.append(_row(f"small_a{q:03d}", f"NR_{h:06d}.1", IDS[h % 3], "97.500", 300, "400" if h < 2 else str(100 + h)))
+            rows.append(hit_row(f"small_a{q:03d}", f"NR_{h:06d}.1", IDS5[h % 3], "97.500", 300, "400" if h < 2 else str(100 + h), mismatch=3, sstart=17))
     for h in range(150_000):
         bits = "999" if h in (7, 70_000, 149_999) else str(100 + h % 800)
-        rows.append(_row("the_big_one", f"NR_{h % 5000:06d}.1", IDS[h % 4], f"9{h % 10}.{h % 1000:03d}", 250 + h % 100, bits))
+        rows.append(hit_row("the_big_one", f"NR_{h % 5000:06d}.1", IDS5[h % 4], f"9{h % 10}.{h % 1000:03d}", 250 + h % 100, bits, mismatch=3, sstart=17))
     for q in range(40):
         for h in range(30):
-            rows.append(_row(f"small_b{q:03d}", f"NR_{h:06d}.1", IDS[(h + 1) % 3], "96.250", 300, "380" if h < 3 else str(90 + h)))
+            rows.append(hit_row(f"small_b{q:03d}", f"NR_{h:06d}.1", IDS5[(h + 1) % 3], "96.250", 300, "380" if h < 3 else str(90 + h), mismatch=3, sstart=17))
     _check("".join(rows), strategies=("relaxed",), chunks=(0, 4 << 20))

@@ -5,10 +5,8 @@ import random
 import pytest
 
 import pyoracle as po
-from helpers import random_blast, random_taxonomy
+from helpers import CUTOFFS_16S, random_blast, random_taxonomy
 from oracle_ffi import Oracle, OracleDataError
-
-FULL = {"domain": 50, "kingdom": 60, "phylum": 75, "class": 80, "order": 85, "family": 92, "genus": 97, "species": 99}
 
 
 @pytest.mark.parametrize("seed", range(60))
@@ -23,7 +21,7 @@ def test_crosscheck(seed):
             for use_taxid in (False, True):
                 custom = None
                 if taxon == "custom":
-                    custom = FULL if seed % 3 else {"domain": 50, "species": 99, "genus": 95}
+                    custom = CUTOFFS_16S if seed % 3 else {"domain": 50, "species": 99, "genus": 95}
                 tax = {u["taxid"]: (u["numericLineage"] if use_taxid else u["textLineage"]) for u in units}
                 try:
                     a = po.results_to_jsonl(po.build_consensus_identities(text, tax, taxon, strat, custom))

@@ -1,43 +1,19 @@
 """Known-answer vectors for InterpolatedIdentity::interpolate_identities (linnaean_ranks.rs:220-383),
 SURVEY.md section 3.3, checked on BOTH oracle restatements (Python mirror and C++)."""
-import math
-
 import pytest
 
 import pyoracle as po
+from helpers import CUTOFFS_16S, KAT, same
 from oracle_ffi import interpolate as c_interpolate
-
-NAN = float("nan")
-YAML16S = {"domain": 50, "kingdom": 60, "phylum": 75, "class": 80, "order": 85, "family": 92, "genus": 97, "species": 99}
-KAT = [
-    ("d p c o f g s", [60, 75, 80, 85, 92, 97, 99], [50, 75, 80, 85, 92, 97, 99]),
-    ("d clade p c o f g species-group species-subgroup s", [60, 67.5, 75, 80, 85, 92, 97, 97.667, 98.333, 99],
-     [50, 62.5, 75, 80, 85, 92, 97, 97.667, 98.333, 99]),
-    ("d p c o f g s strain", [60, 75, 80, 85, 92, 97, 99, 100], [50, 75, 80, 85, 92, 97, 99, 100]),
-    ("d clade clade p c o f g s strain", [60, 65, 70, 75, 80, 85, 92, 97, 99, 100], [50, 58.333, 66.667, 75, 80, 85, 92, 97, 99, 100]),
-    ("no-rank d p c o f g s", [99, 60, 75, 80, 85, 92, 97, 99], [50, 50, 75, 80, 85, 92, 97, 99]),
-    ("d p c o suborder f g s", [60, 75, 80, 85, 88.5, 92, 97, 99], [50, 75, 80, 85, 88.5, 92, 97, 99]),
-    ("d p c o f no-rank g s", [60, 75, 80, 85, 92, 94.333, 97, 99], [50, 75, 80, 85, 92, 94.333, 97, 99]),
-    ("d p c o f g s subspecies no-rank", [60, 75, 80, 85, 92, 97, 99, 99.5, 100], [50, 75, 80, 85, 92, 97, 99, 99.5, 100]),
-    ("d k p c o f g s", [60, 67.5, 75, 80, 85, 92, 97, 99], [50, 60, 75, 80, 85, 92, 97, 99]),
-    ("superkingdom p c o f g s", [99, 75, 80, 85, 92, 97, 99], [50, 75, 80, 85, 92, 97, 99]),
-    ("no-rank d k p c o f g s no-rank", [99, 60, 66.667, 75, 80, 85, 92, 97, 99, NAN], [50, 50, 60, 75, 80, 85, 92, 97, 99, NAN]),
-    ("clade", [NAN], [NAN]),
-]
-
-
-def same(a, b):
-    return len(a) == len(b) and all((math.isnan(x) and math.isnan(y)) or x == y for x, y in zip(a, b))
-
 
 @pytest.mark.parametrize("ranks,bact,cust", KAT)
 def test_interpolation_kat(ranks, bact, cust):
     names = ranks.split()
     pr = [po.rank_from_str(x) for x in names]
     assert same(po.interpolate(pr, po.backbone_for("bacteria")), [float(x) for x in bact])
-    assert same(po.interpolate(pr, po.backbone_for("custom", YAML16S)), [float(x) for x in cust])
+    assert same(po.interpolate(pr, po.backbone_for("custom", CUTOFFS_16S)), [float(x) for x in cust])
     assert same(c_interpolate(names, "bacteria"), [float(x) for x in bact])
-    assert same(c_interpolate(names, "custom", YAML16S), [float(x) for x in cust])
+    assert same(c_interpolate(names, "custom", CUTOFFS_16S), [float(x) for x in cust])
 
 
 def test_fungi_equals_eukaryotes():
